@@ -6,6 +6,7 @@ Headline (`value`, `e2e`, `roofline`): BASELINE.json configs[1] — the fused NC
 the reference's run() blocks of 819 200 samples. Metric: Msamples/s of INPUT cf32 consumed.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]        our arm (one process per GPU under torchrun)
+  python bench.py ... --dump-outputs DIR                      also write the output of the last timed step, DIR/audio.npy
   python bench.py --impl reference ...                        the reference's own CPU chain, same metric
 
 One JSON line on stdout (rank 0). `value` = whole-job throughput with the input resident in HBM; `e2e` = the same chain
@@ -336,7 +337,8 @@ def run_cfg2(cx: Ctx):
     assert nrec.value == args.steps, (nrec.value, args.steps)
     ms_max = cx.allmax(ms)
     value = cx.world * n * args.steps / (ms_max * 1e-3) / 1e6
-
+    # the audio of the last timed step, read back before the passes below reuse `audio` and the chain's stream position
+    last_audio = audio[:n_out].cpu().numpy() if args.dump_outputs else None
 
     # ---- parity of THIS run's output (device path) and of the host-buffer path, against the CPU oracle ----
     parity = None
@@ -440,7 +442,21 @@ def run_cfg2(cx: Ctx):
     del x, audio
     torch.cuda.empty_cache()
     return {"value": value, "ms_per_step": ms_max / args.steps, "warm": warm, "launches": int(launches), "e2e": e2e,
-            "clocks": clocks, "roofline": roof, "parity": parity, "sustained": sustained, "n": n}
+            "clocks": clocks, "roofline": roof, "parity": parity, "sustained": sustained, "n": n, "last_audio": last_audio}
+
+
+DUMP_BYTES_MAX = 60_000_000     # what --dump-outputs writes stays below 64 MB, .npy headers included
+
+
+def dump_output(out_dir, name, a):
+    """Write a as out_dir/<name>.npy. Above DUMP_BYTES_MAX a fixed seeded sample of its elements (in stream order) is
+    written instead, with their positions as <name>_index.npy, so that two runs with the same arguments stay comparable."""
+    os.makedirs(out_dir, exist_ok=True)
+    if a.nbytes > DUMP_BYTES_MAX:
+        idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_BYTES_MAX // (a.itemsize + 8), replace=False))
+        a = a[idx]
+        np.save(os.path.join(out_dir, name + "_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---- config 1: 127-tap FIR (1a) and FIR + decimate-by-4 (1b), 2^24 samples ---------------------------------
@@ -886,6 +902,8 @@ def ours(args):
         "gpu_launches_whole_run": launches_total, "clocks_whole_run": clocks_all,
     }
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "audio", main["last_audio"])
     if cx.world > 1:
         cx.dist.destroy_process_group()
 
@@ -906,7 +924,13 @@ def main():
     ap.add_argument("--n4", type=int, default=1 << 26, help="config 4 wideband stream length (BASELINE: 2^26)")
     ap.add_argument("--cfg4-world", type=int, default=0, help="development aid: run rank 0's channel share of a W-GPU partition on one GPU")
     ap.add_argument("--n5", type=int, default=1 << 28, help="config 5 stream length (BASELINE: 2^28)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline chain's audio from its last timed step (rank 0) as DIR/audio.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         reference_arm(args)
     else:

@@ -1,6 +1,6 @@
 """CPU gate 1: the oracle is pinned.
 
-tests/golden/reference_vectors.npz was produced by tools/make_golden.py from the UNMODIFIED reference
+tests/golden/reference_vectors{,_2}.npz were produced by tools/make_golden.py from the UNMODIFIED reference
 headers (compiled against oracle/volk/volk.h). The reference itself ships no tests or golden vectors
 (SURVEY.md §4), so these reference-run outputs are the pin. oracle/port.c (plain C restatement) must
 reproduce them bit for bit; when oracle/_ref is present (authoring container, or prebuilt on the GPU

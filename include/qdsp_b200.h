@@ -193,8 +193,11 @@ int qdsp_vfofm_history_len(qdsp_vfofm* h);
  * stream; kernel_ms() synchronises and returns the last launch's device time */
 int qdsp_vfofm_enable_timing(qdsp_vfofm* h, int on);
 double qdsp_vfofm_kernel_ms(qdsp_vfofm* h);
-/* the same with one event pair per launch (round robin over `pairs`), so a whole timed region can be bracketed without a
- * synchronisation between launches; kernel_ms_mean() synchronises and averages the launches recorded since enable */
+/* per-launch timing of a whole timed region without a synchronisation, or any stream operation, between launches: the
+ * row-per-lane kernel writes %globaltimer stamps (first CTA start, last CTA end) into one of `pairs` slots per launch, for
+ * the first `pairs` launches since enable; kernel_ms_mean() synchronises and returns the mean completion-to-completion time
+ * of those launches (the first one: start to end), which for launches that do not overlap equals an event pair around
+ * each. Calls that take another kernel are not recorded. enable_timing() turns the ring off. */
 int qdsp_vfofm_enable_timing_ring(qdsp_vfofm* h, int pairs);
 double qdsp_vfofm_kernel_ms_mean(qdsp_vfofm* h, int* launches);
 

@@ -553,13 +553,22 @@ struct qdsp_channelizer {
     Scratch replay_scratch;      // mixed stream | resampled IQ | run table | checkpoints
     Partition part_replay;
     DecimPlan* plan_replay = nullptr;
-    // bench hook: events around the dominant kernel
+    // bench hook: events around the dominant kernel (enable_timing), or per-launch timestamps written by the row-per-lane
+    // kernel itself (enable_timing_ring): an event recorded between two launches would keep them from overlapping
     bool timing = false;
-    cudaEvent_t ev_k0 = nullptr, ev_k1 = nullptr;          // the current launch's pair (= ring[ring_pos])
-    std::vector<cudaEvent_t> ring0, ring1;                  // one pair per launch, round robin (bench: whole timed region)
+    cudaEvent_t ev_k0 = nullptr, ev_k1 = nullptr;
+    unsigned long long* ring = nullptr;                     // [2 * ring_pairs]: first CTA start, last CTA end (ns)
+    int ring_pairs = 0;
     long long ring_launches = 0;
+    // the last row-per-lane call (see qdsp_resamp): when the very next library launch is this handle's next call on the same
+    // stream, the two grids may overlap; the kernel orders the carried state and its audio stores itself (k_rowlane.cu)
+    long long last_serial = -1;
+    cudaStream_t last_stream = nullptr;
+    const char* last_out = nullptr;
+    size_t last_out_bytes = 0;
 
     int upload_nco() {
+        last_serial = -1;
         std::vector<NcoDev> v(nch);
         for (int c = 0; c < nch; c++) v[c] = NcoDev{nco[c].phase, nco[c].step};
         if (!nco_dev) QDSP_CUDA_OK(cudaMalloc(&nco_dev, sizeof(NcoDev) * nch));
@@ -613,14 +622,8 @@ struct qdsp_channelizer {
         const float* din = demod.p + (size_t)cur * nch;
         float* dout = demod.p + (size_t)(cur ^ 1) * nch;
         int rc;
-        if (timing) {
-            if (!ring0.empty()) {
-                ev_k0 = ring0[ring_launches % (long long)ring0.size()];
-                ev_k1 = ring1[ring_launches % (long long)ring1.size()];
-                ring_launches++;
-            }
-            QDSP_CUDA_OK(cudaEventRecord(ev_k0, s));
-        }
+        const bool events = timing && !ring;
+        if (events) QDSP_CUDA_OK(cudaEventRecord(ev_k0, s));
         bool hist_folded = false;
         int rpad = -1;
         if (fftplan && variant == 0 && !iq && chanfft_usable(fftplan, part, in_dev)) {
@@ -631,10 +634,23 @@ struct qdsp_channelizer {
             part.max_out > 0 && (rpad = rowlane_uniform_pad(part, T)) >= 0) {
             // row-per-lane kernel; the history advance (resampling.h:129) is folded into its first CTA
             const NcoDev nh{nco[0].phase, nco[0].step};
+            // overlap needs: no block-table upload between the launches (uniform partition), no IQ output (stored
+            // without the wait), and no read of the previous call's audio (the input is staged before the wait)
+            const bool overlap_prev = last_serial == g_launches.load() && last_stream == s && !iq &&
+                                      part.view.table == nullptr &&
+                                      !byte_ranges_overlap((const char*)in_dev, (size_t)count * 8, last_out, last_out_bytes);
+            unsigned long long* tslot = ring && ring_launches < ring_pairs ? ring + 2 * ring_launches : nullptr;
             rc = launch_decim_rowlane(plan, taps.data(), (const float2*)hist.ptr(), (float2*)hist.buf[hist.cur ^ 1], hist.H,
                                       (const float2*)in_dev, part, 1, nco_dev, &nh, abs_pos, phasor_speed, din, dout,
-                                      (float2*)iq, audio, rpad, s);
+                                      (float2*)iq, audio, rpad, s, overlap_prev, tslot);
+            if (ring && rc == 0) ring_launches++;
             hist_folded = rc == 0;
+            if (hist_folded && !iq) {
+                last_serial = g_launches.load();
+                last_stream = s;
+                last_out = (const char*)audio;
+                last_out_bytes = (size_t)part.total_out * 4;
+            }
         } else if (plan && variant != 1 && chan_supported(plan) && (reinterpret_cast<uintptr_t>(in_dev) & 15) == 0 &&
                    part.max_out > 0 && (rpad = rowlane_uniform_pad(part, T)) >= 0) {
             // wide rows: channel-per-lane kernel (32 channels share every staged sample), one launch per column slice
@@ -647,8 +663,9 @@ struct qdsp_channelizer {
             rc = launch_generic_vfofm((const float2*)hist.ptr(), hist.H, (const float2*)in_dev, phases_dev, tpp, part,
                                       nco_dev, abs_pos, nch, phasor_speed, din, dout, audio, (float2*)iq, out_stride,
                                       s);
+        if (!hist_folded || iq) last_serial = -1;
         if (rc != 0) return -1;
-        if (timing) QDSP_CUDA_OK(cudaEventRecord(ev_k1, s));
+        if (events) QDSP_CUDA_OK(cudaEventRecord(ev_k1, s));
         if (part.total_out > 0) cur ^= 1;
         if (hist_folded) hist.cur ^= 1;
         else if (hist.advance(in_dev, count, s) != 0) return -1;
@@ -669,12 +686,9 @@ struct qdsp_channelizer {
             if (ev_done[i]) cudaEventDestroy(ev_done[i]);
         }
         if (copy_stream) cudaStreamDestroy(copy_stream);
-        if (ring0.empty()) {
-            if (ev_k0) cudaEventDestroy(ev_k0);
-            if (ev_k1) cudaEventDestroy(ev_k1);
-        }
-        for (cudaEvent_t e : ring0) cudaEventDestroy(e);
-        for (cudaEvent_t e : ring1) cudaEventDestroy(e);
+        if (ev_k0) cudaEventDestroy(ev_k0);
+        if (ev_k1) cudaEventDestroy(ev_k1);
+        if (ring) cudaFree(ring);
     }
 };
 struct qdsp_vfofm {
@@ -768,6 +782,7 @@ long long qdsp_vfofm_process_host(qdsp_vfofm* h, const void* in_host, float* aud
         QDSP_CUDA_OK(cudaStreamWaitEvent(s, ev_h2d[slot], 0));
         const long long m = c.process(c.stage_in[slot], c.stage_out[slot], nullptr, 0, n, nullptr, 0, block_size, nullptr, s);
         if (m < 0) return -1;
+        c.last_serial = -1;   // copies and event waits go between the chunks' kernels: never overlapped
         if (m > 0)
             QDSP_CUDA_OK(cudaMemcpyAsync(audio_out_host + produced, c.stage_out[slot], (size_t)m * sizeof(float),
                                          cudaMemcpyDeviceToHost, s));
@@ -850,6 +865,7 @@ long long qdsp_vfofm_process_replay(qdsp_vfofm* h, const void* in_dev, float* au
 }
 int qdsp_vfofm_reset(qdsp_vfofm* h) {
     qdsp_channelizer& c = h->c;
+    c.last_serial = -1;
     QDSP_CUDA_OK(cudaDeviceSynchronize());
     if (c.hist.reset(nullptr) != 0) return -1;
     std::vector<float> z(2 * c.nch, 0.0f);
@@ -859,14 +875,17 @@ int qdsp_vfofm_reset(qdsp_vfofm* h) {
     return 0;
 }
 int qdsp_vfofm_set_variant(qdsp_vfofm* h, int variant) {
+    h->c.last_serial = -1;
     h->c.variant = variant;
     return 0;
 }
 int qdsp_vfofm_seek(qdsp_vfofm* h, long long start) {
+    h->c.last_serial = -1;
     h->c.abs_pos = start;
     return 0;
 }
 int qdsp_vfofm_import_tail(qdsp_vfofm* h, const void* tail_dev, int src_device, qdsp_stream_t s) {
+    h->c.last_serial = -1;
     return import_tail_impl(h->c.hist, tail_dev, src_device, as_stream(s));
 }
 int qdsp_vfofm_history_len(qdsp_vfofm* h) { return h->c.hist.H; }
@@ -875,44 +894,42 @@ int qdsp_vfofm_enable_timing(qdsp_vfofm* h, int on) {
         QDSP_CUDA_OK(cudaEventCreate(&h->c.ev_k0));
         QDSP_CUDA_OK(cudaEventCreate(&h->c.ev_k1));
     }
+    if (h->c.ring) cudaFree(h->c.ring);
+    h->c.ring = nullptr;
+    h->c.ring_pairs = 0;
     h->c.timing = on != 0;
     return 0;
 }
+// The kernel stamps its slot with %globaltimer: the first CTA's start and the last CTA's end. Launch k is reported as
+// end(k) - end(k-1), the first one as end - start: completion to completion, which for launches that do not overlap is
+// what an event pair around each launch measures, with nothing recorded on the stream between the launches.
 int qdsp_vfofm_enable_timing_ring(qdsp_vfofm* h, int pairs) {
     if (pairs < 1) return -1;
-    if (h->c.ring0.empty() && h->c.ev_k0) {
-        cudaEventDestroy(h->c.ev_k0);
-        cudaEventDestroy(h->c.ev_k1);
-    }
-    for (cudaEvent_t e : h->c.ring0) cudaEventDestroy(e);
-    for (cudaEvent_t e : h->c.ring1) cudaEventDestroy(e);
-    h->c.ring0.assign(pairs, nullptr);
-    h->c.ring1.assign(pairs, nullptr);
-    for (int i = 0; i < pairs; i++) {
-        QDSP_CUDA_OK(cudaEventCreate(&h->c.ring0[i]));
-        QDSP_CUDA_OK(cudaEventCreate(&h->c.ring1[i]));
-    }
-    h->c.ev_k0 = h->c.ring0[0];
-    h->c.ev_k1 = h->c.ring1[0];
-    h->c.ring_launches = 0;
-    h->c.timing = true;
+    qdsp_channelizer& c = h->c;
+    QDSP_CUDA_OK(cudaDeviceSynchronize());
+    if (c.ring) cudaFree(c.ring);
+    c.ring = nullptr;
+    QDSP_CUDA_OK(cudaMalloc(&c.ring, sizeof(unsigned long long) * 2 * (size_t)pairs));
+    std::vector<unsigned long long> init(2 * (size_t)pairs, 0ull);
+    for (int i = 0; i < pairs; i++) init[2 * (size_t)i] = ~0ull;
+    QDSP_CUDA_OK(cudaMemcpy(c.ring, init.data(), sizeof(unsigned long long) * init.size(), cudaMemcpyHostToDevice));
+    c.ring_pairs = pairs;
+    c.ring_launches = 0;
+    c.timing = true;
     return 0;
 }
 double qdsp_vfofm_kernel_ms_mean(qdsp_vfofm* h, int* launches) {
-    const long long n = h->c.ring_launches < (long long)h->c.ring0.size() ? h->c.ring_launches : (long long)h->c.ring0.size();
+    qdsp_channelizer& c = h->c;
+    const long long n = c.ring_launches < (long long)c.ring_pairs ? c.ring_launches : (long long)c.ring_pairs;
     if (launches) *launches = (int)n;
     if (n <= 0) return -1.0;
-    double sum = 0.0;
-    for (long long i = 0; i < n; i++) {
-        float ms = 0.f;
-        if (cudaEventSynchronize(h->c.ring1[i]) != cudaSuccess) return -1.0;
-        if (cudaEventElapsedTime(&ms, h->c.ring0[i], h->c.ring1[i]) != cudaSuccess) return -1.0;
-        sum += ms;
-    }
-    return sum / (double)n;
+    std::vector<unsigned long long> t(2 * (size_t)n);
+    if (cudaDeviceSynchronize() != cudaSuccess) return -1.0;
+    if (cudaMemcpy(t.data(), c.ring, sizeof(unsigned long long) * t.size(), cudaMemcpyDeviceToHost) != cudaSuccess) return -1.0;
+    return (double)(t[2 * (size_t)n - 1] - t[0]) * 1e-6 / (double)n;
 }
 double qdsp_vfofm_kernel_ms(qdsp_vfofm* h) {
-    if (!h->c.ev_k0) return -1.0;
+    if (!h->c.ev_k0 || h->c.ring) return -1.0;
     if (cudaEventSynchronize(h->c.ev_k1) != cudaSuccess) return -1.0;
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, h->c.ev_k0, h->c.ev_k1) != cudaSuccess) return -1.0;
@@ -947,6 +964,7 @@ long long qdsp_channelizer_process(qdsp_channelizer* h, const void* in_dev, floa
                       as_stream(s));
 }
 int qdsp_channelizer_reset(qdsp_channelizer* h) {
+    h->last_serial = -1;
     QDSP_CUDA_OK(cudaDeviceSynchronize());
     if (h->hist.reset(nullptr) != 0) return -1;
     std::vector<float> z(2 * h->nch, 0.0f);
@@ -956,10 +974,12 @@ int qdsp_channelizer_reset(qdsp_channelizer* h) {
     return 0;
 }
 int qdsp_channelizer_set_variant(qdsp_channelizer* h, int variant) {
+    h->last_serial = -1;
     h->variant = variant;
     return 0;
 }
 int qdsp_channelizer_seek(qdsp_channelizer* h, long long start) {
+    h->last_serial = -1;
     h->abs_pos = start;
     return 0;
 }

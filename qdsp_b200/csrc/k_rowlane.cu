@@ -22,10 +22,17 @@
 
 namespace qdsp {
 
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+
 template <int Q, int D>
 struct RowArgs {
     DecimArgs a;
     float2* hist_next;        // when non-null: CTA (0,0) writes the advanced history tail here
+    unsigned long long* tstamp;   // when non-null (timing ring slot, %globaltimer ns): [0] min CTA start, [1] max CTA end
     int nstep;                // steps (of 32 rows) per full tile
     int pad;                  // tap-table alignment pad (uniform over the batch)
     float g[Q * D];           // g[q*D + c] = h[q*D + c - pad], zero outside [0, T)
@@ -46,9 +53,19 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
     const BlkInfo bi = a.part.get(b);
     const int LT = 32 * ra.nstep - (Q - 1) - LEAD;     // outputs per full tile
     const int k0 = tile * LT;
+    if (ra.tstamp != nullptr && tile == 0 && b == 0 && lane == 0) atomicMin(&ra.tstamp[0], globaltimer_ns());
 
+    // Overlapped consecutive calls (programmatic dependent launch, launch_decim_rowlane's overlap_prev): the next call of
+    // the same handle may start while this grid drains. The state carried from call to call -- `hist` and `demod_in`,
+    // written by the previous grid, and `hist_next`, which the previous grid read as `hist` -- is touched only by the
+    // CTAs that wait for the previous grid at their start: CTA (0,0), and a tile whose rows or leading-angle window reach
+    // before sample 0 or which takes its leading angle from `demod_in`. Every other CTA reads only `in` (the launcher
+    // refuses an input that overlaps the previous call's audio) and holds its audio and `demod_out` until its tile is
+    // computed, then waits and stores: write-after-write on `audio` and on the `demod_out` ping-pong stays ordered
+    // whatever buffers the caller passes. Without the launch attribute both instructions are no-ops.
     // ---- folded history advance: new_hist[j] = virtual[count - H + j] ------------------------------
     if (ra.hist_next != nullptr && tile == 0 && b == 0) {
+        asm volatile("griddepcontrol.wait;" ::: "memory");
         for (int j = lane; j < a.H; j += 32) {
             const long long v = a.n_in - a.H + j;
             ra.hist_next[j] = v >= 0 ? a.in[v] : a.hist[a.H + v];
@@ -75,9 +92,10 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
     // leading angle of the block's very first output
     bool use_override = false;
     float override_ang = 0.f;
+    int pb = b - 1;
+    BlkInfo pbi{};
+    long long ovr_win = 0;     // first sample of the window of the previous block's last output (off-grid hand-over)
     if (DEMOD && tile == 0) {
-        int pb = b - 1;
-        BlkInfo pbi{};
         while (pb >= 0) {
             pbi = a.part.get(pb);
             if (pbi.out_count > 0) break;
@@ -85,10 +103,17 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
         }
         if (pb < 0) {
             use_override = true;
-            override_ang = a.demod_in[0];
         } else if (pb != b - 1 || pbi.in_start + (long long)pbi.out_count * D != bi.in_start) {
             use_override = true;  // previous block's last output is off this block's row grid
-            const float2 y = direct_output_warp<ROT>(a, pbi.in_start + (long long)(pbi.out_count - 1) * D - a.T, nco_ph0, nco_step);
+            ovr_win = pbi.in_start + (long long)(pbi.out_count - 1) * D - a.T;
+        }
+    }
+    if (row0 < 0 || (use_override && (pb < 0 || ovr_win < 0))) asm volatile("griddepcontrol.wait;" ::: "memory");
+    if (use_override) {
+        if (pb < 0) {
+            override_ang = a.demod_in[0];
+        } else {
+            const float2 y = direct_output_warp<ROT>(a, ovr_win, nco_ph0, nco_step);
             override_ang = fast_arctan2_ref(y.y, y.x);
         }
     }
@@ -117,6 +142,7 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
         }
     };
     for (int i = 0; i < NSTG; i++) issue(i);
+    asm volatile("griddepcontrol.launch_dependents;");
 
     // ---- per-lane state -------------------------------------------------------------------------------
     float2 Pr = make_float2(1.f, 0.f);        // row phasor of this lane's current row
@@ -124,6 +150,10 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
     float ang_saved = 0.f;
     const bool tail_lane = lane >= 32 - (Q - 1);
     const long long obase = a.out_stride * 0 + bi.out_start + k0 - LEAD;   // output index of tile-relative output 0
+    // the tile's audio, indexed by tile-relative output (32 per step), stored after the wait for the previous grid
+    float* hold = reinterpret_cast<float*>(smem_raw + NSTG * STAGE_BYTES + NSTG * 8 + 16);
+    bool last_here = false;                   // this lane computes the call's last output: its angle is `demod_out`
+    float last_ang = 0.f;
 
 #pragma unroll 1
     for (int i = 0; i < nsteps; i++) {
@@ -199,13 +229,26 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
             if (use_override && orel == 1) prev = override_ang;
             ang_saved = ang;
             if (live) {
-                a.audio[oidx] = fm_step_ref(ang, prev, a.phasor_speed);
-                if (oidx == a.part.total_out - 1) a.demod_out[0] = ang;
-                if (a.out_iq) a.out_iq[oidx] = y;
+                hold[orel] = fm_step_ref(ang, prev, a.phasor_speed);
+                if (oidx == a.part.total_out - 1) {
+                    last_here = true;
+                    last_ang = ang;
+                }
+                if (a.out_iq) a.out_iq[oidx] = y;    // calls that want IQ are never overlapped (launch_decim_rowlane)
             }
         } else {
             if (live) a.out_iq[oidx] = y;
         }
+    }
+    if (DEMOD) {
+        asm volatile("griddepcontrol.wait;" ::: "memory");
+        __syncwarp();
+        for (int e = LEAD + lane; e < nout + LEAD; e += 32) a.audio[obase + e] = hold[e];
+        if (last_here) a.demod_out[0] = last_ang;
+    }
+    if (ra.tstamp != nullptr) {
+        __syncwarp();
+        if (lane == 0) atomicMax(&ra.tstamp[1], globaltimer_ns());
     }
 }
 
@@ -231,7 +274,7 @@ int rowlane_uniform_pad(const Partition& part, int T) {
 int launch_decim_rowlane(DecimPlan* plan, const float* taps_host, const float2* hist, float2* hist_next, int H,
                          const float2* in, const Partition& part, int mode, const NcoDev* nco_dev, const NcoDev* nco_host,
                          long long abs0, float phasor_speed, const float* demod_in, float* demod_out, float2* out_iq,
-                         float* audio, int pad, cudaStream_t s) {
+                         float* audio, int pad, cudaStream_t s, bool overlap_prev, unsigned long long* tstamp) {
     constexpr int Q = 9, D = 50, NSTG = 2;
     static RowArgs<Q, D> ra;     // large (4 KB): built in place; launches copy it at enqueue time
     static std::mutex mtx;
@@ -257,8 +300,12 @@ int launch_decim_rowlane(DecimPlan* plan, const float* taps_host, const float2* 
     a.audio = audio;
     a.out_stride = 0;
     ra.hist_next = hist_next;
+    ra.tstamp = tstamp;
     static const int nstep_env = getenv("QDSP_ROW_NSTEP") ? atoi(getenv("QDSP_ROW_NSTEP")) : 0;
-    ra.nstep = nstep_env >= 2 ? nstep_env : 8;   // B200 sweep (GS/s): 4: 811, 6: 823, 8: 824, 9: 787, 10: 802, 12: 792, 16: 808, 20: 806, 24: 793, 32: 773
+    // B200 sweeps (GS/s), DESIGN.md 6.0. Isolated launches: 4: 811, 6: 823, 8: 824, 9: 787, 10: 802, 12: 792, 16: 808,
+    // 20: 806, 24: 793, 32: 773. Consecutive calls overlapped, bench.py's 100-call burst: 8: 878, 16: 866; under the power
+    // cap (2 s loop) 16 steps win instead (797 vs 775): less tile re-read, fewer instructions per sample.
+    ra.nstep = nstep_env >= 2 ? nstep_env : 8;
     ra.pad = pad;
     for (int j = 0; j < Q * D; j++) {
         const int t = j - pad;
@@ -275,12 +322,24 @@ int launch_decim_rowlane(DecimPlan* plan, const float* taps_host, const float2* 
     const int LT = 32 * ra.nstep - (Q - 1) - lead;
     dim3 grid((part.max_out + LT - 1) / LT, part.view.nblocks, 1);
     if (grid.x < 1) grid.x = 1;
-    constexpr size_t smem = NSTG * 32 * D * 8 + NSTG * 8 + 16;
+    // TMA ring + mbarriers, then (fused) the tile's held audio: one float per lane per step
+    const size_t smem = NSTG * 32 * D * 8 + NSTG * 8 + 16 + (fused ? (size_t)ra.nstep * 32 * sizeof(float) : 0);
+    static const int pdl_env = getenv("QDSP_PDL") ? atoi(getenv("QDSP_PDL")) : 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = dim3(32);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = (overlap_prev && fused && out_iq == nullptr && pdl_env) ? 1 : 0;
 #define QDSP_ROW_LAUNCH(JL, ROTV, DEMV)                                                                   \
     {                                                                                                     \
         auto kern = decim_rowlane_kernel<Q, D, JL, NSTG, ROTV, DEMV>;                                     \
         QDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        kern<<<grid, 32, smem, s>>>(ra);                                                                  \
+        QDSP_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, ra));                                                 \
     }
     // T <= 401: the last tap row (q = 8) has live taps in its first column pair only
     if (plan->T + 1 <= 402) {

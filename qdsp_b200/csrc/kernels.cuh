@@ -56,7 +56,7 @@ int rowlane_uniform_pad(const Partition& part, int T);
 int launch_decim_rowlane(DecimPlan* plan, const float* taps_host, const float2* hist, float2* hist_next, int H,
                          const float2* in, const Partition& part, int mode, const NcoDev* nco_dev, const NcoDev* nco_host,
                          long long abs0, float phasor_speed, const float* demod_in, float* demod_out, float2* out_iq,
-                         float* audio, int pad, cudaStream_t s);
+                         float* audio, int pad, cudaStream_t s, bool overlap_prev, unsigned long long* tstamp);
 
 // ---- k_chan.cu: channel-per-lane decimating FIR (wide rows, many channels off one input) --------------------
 bool chan_supported(const DecimPlan* plan);
@@ -95,7 +95,7 @@ int launch_fir_decim(FirDecimPlan* plan, const float2* hist, int H, const float2
 // ---- k_firrow.cu: row-per-lane decimating FIR for small decimations (config 1b: D = 4, 127 taps) ------------------
 bool firrow_supported(int T, int D);
 int launch_firrow(const float* taps_host, int T, int D, const float2* hist, float2* hist_next, int H, const float2* in,
-                  long long count, long long n_out, float2* out, cudaStream_t s, bool overlap_prev = false);
+                  long long count, long long n_out, float2* out, cudaStream_t s, bool overlap_prev);
 
 // ---- k_recurrent.cu -----------------------------------------------------------------------------
 int launch_deemp(const float2* in, float2* out, long long count, float alpha, float* state, void* scratch,

@@ -4,6 +4,8 @@
 // these as float2.
 #pragma once
 #include <math.h>
+#include <stdint.h>
+#include <qdsp_b200.h>
 
 #define FL_M_PI 3.1415926535f  // the reference's float "pi" (src/dsp/types.h:4)
 
@@ -45,4 +47,31 @@ namespace dsp {
     };
 
     static_assert(sizeof(complex_t) == 8 && sizeof(stereo_t) == 8, "samples must be 8-byte interleaved pairs");
+
+    // integer IQ as radio front ends deliver it (interleaved re, im): USRP / BladeRF / LimeSDR / SDRplay / Airspy HF+
+    // (int16), HackRF (int8), RTL-SDR (uint8). Read as complex_t by IQToComplex<T> (convertion.h) and directly by
+    // FusedVFOFloatFMDemodT<T> (vfo.h), both converting on the GPU: y = (float(x) + offset) * scale per component.
+    struct complex_s16_t { int16_t re; int16_t im; };
+    struct complex_s8_t { int8_t re; int8_t im; };
+    struct complex_u8_t { uint8_t re; uint8_t im; };
+    static_assert(sizeof(complex_s16_t) == 4 && sizeof(complex_s8_t) == 2 && sizeof(complex_u8_t) == 2, "packed pairs");
+
+    // the C ABI format code of a sample type and its usual conversion (include/qdsp_b200.h)
+    template <class T> struct iq_format;
+    template <> struct iq_format<complex_t> {
+        static constexpr int code = QDSP_CF32;
+        static constexpr float scale = 1.0f, offset = 0.0f;
+    };
+    template <> struct iq_format<complex_s16_t> {
+        static constexpr int code = QDSP_CS16;
+        static constexpr float scale = 1.0f / 32768.0f, offset = 0.0f;
+    };
+    template <> struct iq_format<complex_s8_t> {
+        static constexpr int code = QDSP_CS8;
+        static constexpr float scale = 1.0f / 128.0f, offset = 0.0f;
+    };
+    template <> struct iq_format<complex_u8_t> {
+        static constexpr int code = QDSP_CU8;
+        static constexpr float scale = 1.0f / 128.0f, offset = -127.5f;
+    };
 }

@@ -94,41 +94,50 @@ namespace dsp {
         PolyphaseResampler<complex_t> resamp;
     };
 
-    // VFO -> FloatFMDemod in one kernel launch per run() call.
-    class FusedVFOFloatFMDemod : public generic_block<FusedVFOFloatFMDemod> {
+    // VFO -> FloatFMDemod in one kernel launch per run() call. T is the input sample type: complex_t, or integer IQ
+    // (complex_s16_t, complex_s8_t, complex_u8_t), converted to complex_t on the GPU by one more kernel; the input edge
+    // then copies 4 or 2 bytes per sample. FusedVFOFloatFMDemod is the complex_t chain.
+    template <class T>
+    class FusedVFOFloatFMDemodT : public generic_block<FusedVFOFloatFMDemodT<T>> {
+        using base = generic_block<FusedVFOFloatFMDemodT<T>>;
+
     public:
-        FusedVFOFloatFMDemod() {}
-        FusedVFOFloatFMDemod(stream<complex_t>* in, float offset, float inSampleRate, float outSampleRate, float bandWidth, float deviation) {
+        FusedVFOFloatFMDemodT() {}
+        FusedVFOFloatFMDemodT(stream<T>* in, float offset, float inSampleRate, float outSampleRate, float bandWidth, float deviation) {
             init(in, offset, inSampleRate, outSampleRate, bandWidth, deviation);
         }
-        ~FusedVFOFloatFMDemod() {
-            generic_block<FusedVFOFloatFMDemod>::stop();
+        ~FusedVFOFloatFMDemodT() {
+            base::stop();
             if (h) { qdsp_vfofm_destroy(h); }
         }
-        void init(stream<complex_t>* in, float offset, float inSampleRate, float outSampleRate, float bandWidth, float deviation) {
+        void init(stream<T>* in, float offset, float inSampleRate, float outSampleRate, float bandWidth, float deviation) {
             _in = in;
             if (h) { qdsp_vfofm_destroy(h); }
             h = qdsp_vfofm_create(offset, inSampleRate, outSampleRate, bandWidth, deviation);
-            generic_block<FusedVFOFloatFMDemod>::registerInput(_in);
-            generic_block<FusedVFOFloatFMDemod>::registerOutput(&out);
+            if (h && iq_format<T>::code != QDSP_CF32) { setInputScale(iq_format<T>::scale, iq_format<T>::offset); }
+            base::registerInput(_in);
+            base::registerOutput(&out);
         }
         void setOffset(float offset) { qdsp_vfofm_set_offset(h, offset); }
+        // integer input: y = (float(x) + offset) * scale per component (e.g. 1 / 2048 for BladeRF sc16q11)
+        void setInputScale(float scale, float offset) { qdsp_vfofm_set_input_format(h, iq_format<T>::code, scale, offset); }
         int run() override {
-            const int count = _in->readDevice(cuStream);
+            const int count = _in->readDevice(base::cuStream);
             if (count < 0) { return -1; }
-            out.acquireWriteDev(cuStream);
+            out.acquireWriteDev(base::cuStream);
             const int one = count;
-            const long long n = qdsp_vfofm_process(h, _in->readDev(), out.writeDev(), nullptr, count, &one, 1, 0, nullptr, cuStream);
-            _in->flushDevice(cuStream);
+            const long long n = qdsp_vfofm_process(h, _in->readDev(), out.writeDev(), nullptr, count, &one, 1, 0, nullptr, base::cuStream);
+            _in->flushDevice(base::cuStream);
             if (n < 0) { return -1; }
-            if (!out.swapDevice((int)n, cuStream)) { return -1; }
+            if (!out.swapDevice((int)n, base::cuStream)) { return -1; }
             return count;
         }
 
         stream<float> out;
 
     private:
-        stream<complex_t>* _in = nullptr;
+        stream<T>* _in = nullptr;
         qdsp_vfofm* h = nullptr;
     };
+    using FusedVFOFloatFMDemod = FusedVFOFloatFMDemodT<complex_t>;
 }

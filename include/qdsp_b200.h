@@ -31,6 +31,10 @@ extern "C" {
 #define QDSP_ABI_VERSION 1
 typedef void* qdsp_stream_t;
 enum { QDSP_F32 = 0, QDSP_CF32 = 1 }; /* element type of a stream: float or {float re,im} (== stereo_t) */
+/* integer IQ as radio front ends deliver it: interleaved (re, im) pairs of int16 (USRP, BladeRF sc16q11, LimeSDR,
+ * SDRplay, Airspy HF+), int8 (HackRF) or uint8 (RTL-SDR). Accepted by qdsp_iq_convert_process and, after
+ * *_set_input_format, by the fused VFO -> FM chain and the channelizer; every `dtype` argument rejects them. */
+enum { QDSP_CS16 = 2, QDSP_CS8 = 3, QDSP_CU8 = 4 };
 
 /* ---- runtime plumbing (replaces volk_malloc/volk_free in src/dsp/stream.h:25-31) ------------- */
 int qdsp_abi_version(void);
@@ -65,6 +69,14 @@ int qdsp_stream_wait_event(qdsp_stream_t s, void* ev);
 int qdsp_event_sync(void* ev);
 /* number of kernels this library has launched in this process (bench.py "gpu_launches") */
 long long qdsp_launch_count(void);
+
+/* ---- integer IQ -> cf32 --------------------------------------------------------------------- *
+ * One conversion rule wherever this library reads integer IQ: y = (float(x) + offset) * scale, each step rounded to  *
+ * float32 (for cu8, x is the byte value 0..255). Usual parameters, all exact: cs16 1/32768, 0; cs8 1/128, 0; cu8     *
+ * 1/128, -127.5; sc16q11 is cs16 with 1/2048. `scale` must be finite and non-zero, `offset` finite. in_dev holds      *
+ * `count` pairs, aligned to its pair (4 bytes for cs16, 2 for the 8-bit formats); out_dev gets `count` cf32 samples.  */
+long long qdsp_iq_convert_process(int fmt, float scale, float offset, const void* in_dev, void* out_dev, long long count,
+                                  qdsp_stream_t s);
 
 /* ---- tap design, host side, bit-exact with the reference (src/dsp/window.h) ------------------ */
 int qdsp_blackman_tap_count(float cutoff, float transWidth, float sampleRate);                 /* window.h:36-50 */
@@ -175,6 +187,10 @@ long long qdsp_vfofm_process_host(qdsp_vfofm* h, const void* in_host, float* aud
                                   int block_size, qdsp_stream_t s);
 int qdsp_vfofm_reset(qdsp_vfofm* h);
 int qdsp_vfofm_set_variant(qdsp_vfofm* h, int variant);
+/* element type of in_dev (process) and in_host (process_host) from the next call on: QDSP_CF32 (the default; scale and
+ * offset ignored) or QDSP_CS16 / QDSP_CS8 / QDSP_CU8 with the conversion of qdsp_iq_convert_process. The state carried
+ * from call to call (history tail, import_tail, history_len) stays cf32, so formats may change from call to call. */
+int qdsp_vfofm_set_input_format(qdsp_vfofm* h, int fmt, float scale, float offset);
 /* time-sharding: start this shard at absolute stream sample `start` (NCO phase in closed form),
  * history/demod state imported from the previous shard */
 /* DEBUG replay of the reference's recursive float32 NCO (attribution of its drift, DESIGN.md "NCO"): the translator is
@@ -182,7 +198,8 @@ int qdsp_vfofm_set_variant(qdsp_vfofm* h, int variant);
  * of every 512-sample run of every run() call (processing.h:64; n_ckpt = sum over blocks of ceil(count_b / 512), computed
  * by the caller, e.g. with the oracle's rotator) -- with the reference's float recursion inside a run: the mixed samples are
  * bit-identical to the reference's. Unfused (translator, resampler, demodulator as three kernels); state (history of the
- * MIXED stream, demodulator phase) is separate from the fused path's: do not interleave the two on one handle. */
+ * MIXED stream, demodulator phase) is separate from the fused path's: do not interleave the two on one handle. cf32 input
+ * only: fails after qdsp_vfofm_set_input_format with an integer format. */
 long long qdsp_vfofm_process_replay(qdsp_vfofm* h, const void* in_dev, float* audio_out_dev, void* iq_out_dev,
                                     long long count, const int* blocks, int nblocks, int block_size,
                                     const float* ckpt_host, long long n_ckpt, qdsp_stream_t s);
@@ -212,6 +229,8 @@ long long qdsp_channelizer_process(qdsp_channelizer* h, const void* in_dev, floa
                                    long long out_stride, long long count, const int* blocks, int nblocks,
                                    int block_size, qdsp_stream_t s);
 int qdsp_channelizer_reset(qdsp_channelizer* h);
+/* as qdsp_vfofm_set_input_format */
+int qdsp_channelizer_set_input_format(qdsp_channelizer* h, int fmt, float scale, float offset);
 /* variant 0: the fastest path the geometry allows (a uniform comb of 256 channels fs / 256 apart with decimation 1280 --
  * BASELINE config 4 -- takes the FFT polyphase kernels, k_chanfft.cu); 2: direct form (every channel its own VFO) always;
  * 1: the generic kernels. */

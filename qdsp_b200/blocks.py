@@ -16,6 +16,7 @@ import ctypes as C
 import numpy as np
 
 from . import lib as _lib
+from . import synth as _synth
 from .lib import CF32, F32, QdspError, check
 
 
@@ -66,6 +67,49 @@ class DevBuf:
             self.free()
         except Exception:
             pass
+
+
+def _iq_format(fmt, scale=None, offset=None):
+    """'cs16' / 'cs8' / 'cu8' (or the QDSP_* code), with the usual scale / offset unless given -> (name, code, s, o)."""
+    names = {v: k for k, v in _synth.IQ_CODES.items()}
+    name = names.get(fmt, fmt)
+    if name not in _synth.IQ_FORMATS:
+        raise ValueError(f"unknown integer IQ format {fmt!r}: one of {sorted(_synth.IQ_FORMATS)}")
+    _, s0, o0 = _synth.IQ_FORMATS[name]
+    return name, _synth.IQ_CODES[name], float(s0 if scale is None else scale), float(o0 if offset is None else offset)
+
+
+def _iq_input(x, name):
+    """The caller's input for the handle's input format: complex64 samples (name None) or interleaved integer pairs."""
+    if name is None:
+        x = np.ascontiguousarray(x, np.complex64)
+        return x, len(x)
+    x = np.ascontiguousarray(x).reshape(-1)
+    return _iq_input_checked(x, name)
+
+
+def _iq_input_checked(x, name):
+    """As _iq_input, without a copy: for caller-owned (pinned) buffers, which must already have the right type."""
+    want = np.dtype(np.complex64 if name is None else _synth.IQ_FORMATS[name][0])
+    if x.dtype != want or not x.flags.c_contiguous or (name is not None and x.size % 2):
+        raise TypeError(f"{name or 'cf32'} input is a contiguous {want} array" + (" of (re, im) pairs" if name else ""))
+    return x, (x.size if name is None else x.size // 2)
+
+
+class _InputFormat:
+    """set_input_format() of the handles that read integer IQ (qdsp_*_set_input_format)."""
+
+    _in_fmt = None   # None = cf32, else the format name
+
+    def set_input_format(self, fmt, scale=None, offset=None):
+        """fmt: 'cs16' / 'cs8' / 'cu8' (scale / offset default to the usual ones, synth.IQ_FORMATS), or 'cf32' / CF32."""
+        if fmt in ("cf32", CF32):
+            check(getattr(_L(), self._set_fmt)(self.h, CF32, 1.0, 0.0), self._set_fmt)
+            self._in_fmt = None
+            return
+        name, code, sc, off = _iq_format(fmt, scale, offset)
+        check(getattr(_L(), self._set_fmt)(self.h, code, sc, off), self._set_fmt)
+        self._in_fmt = name
 
 
 def _blocks_arg(n: int, block):
@@ -472,10 +516,12 @@ class VFO:
         return self.resamp.process(self.xlator.process(x), block)
 
 
-class VFOFM(_Block):
-    """Fused VFO -> FloatFMDemod (one kernel; translated and resampled IQ stay on chip)."""
+class VFOFM(_InputFormat, _Block):
+    """Fused VFO -> FloatFMDemod (one kernel; translated and resampled IQ stay on chip). After set_input_format('cs16' |
+    'cs8' | 'cu8'), process / process_host take interleaved integer pairs (converted to cf32 on the GPU)."""
 
     _destroy = "qdsp_vfofm_destroy"
+    _set_fmt = "qdsp_vfofm_set_input_format"
     out_dtype = np.float32
 
     def __init__(self, offset, inSampleRate, outSampleRate, bandWidth, deviation):
@@ -543,14 +589,13 @@ class VFOFM(_Block):
 
     def process_host(self, x: np.ndarray, block: int) -> np.ndarray:
         """The host-buffer entry point (qdsp_vfofm_process_host): pinned host in / out, chunked H2D | kernel | D2H."""
-        x = np.ascontiguousarray(x, np.complex64)
-        n = len(x)
+        x, n = _iq_input(x, self._in_fmt)
         L = _L()
-        hin = L.qdsp_malloc_pinned(max(n, 1) * 8)
+        hin = L.qdsp_malloc_pinned(max(x.nbytes, 1))
         cap = self._out_capacity(n, block)
         hout = L.qdsp_malloc_pinned(max(cap, 1) * 4)
         try:
-            C.memmove(hin, x.ctypes.data, n * 8)
+            C.memmove(hin, x.ctypes.data, x.nbytes)
             m = int(check(L.qdsp_vfofm_process_host(self.h, hin, hout, n, int(block), None), "qdsp_vfofm_process_host"))
             y = np.empty(m, np.float32)
             C.memmove(y.ctypes.data, hout, m * 4)
@@ -570,29 +615,33 @@ class VFOFM(_Block):
         return r
 
     def process(self, x, block=None) -> np.ndarray:
-        if not self.want_iq:
+        if not self.want_iq and self._in_fmt is None:
             return super().process(x, block)
-        x = np.ascontiguousarray(x, np.complex64)
-        n = len(x)
+        x, n = _iq_input(x, self._in_fmt)
         din = DevBuf.from_numpy(x)
         cap = self._out_capacity(n, block)
-        dout, diq = DevBuf(cap * 4), DevBuf(cap * 8)
+        dout, diq = DevBuf(cap * 4), (DevBuf(cap * 8) if self.want_iq else None)
         self.stream = None
-        m = int(check(self._run(din.ptr, dout.ptr, n, block, diq.ptr), "VFOFM"))
-        self.last_iq = diq.to_numpy(np.complex64, m)
+        m = int(check(self._run(din.ptr, dout.ptr, n, block, diq.ptr if diq else None), "VFOFM"))
+        if diq:
+            self.last_iq = diq.to_numpy(np.complex64, m)
         return dout.to_numpy(np.float32, m)
 
     def process_host_into(self, x: np.ndarray, out: np.ndarray, block_size: int, stream=None) -> int:
-        """End-to-end call with caller-owned HOST buffers (pinned for real overlap): chunked H2D/compute/D2H inside."""
-        return int(check(_L().qdsp_vfofm_process_host(self.h, x.ctypes.data, out.ctypes.data, len(x), int(block_size),
+        """End-to-end call with caller-owned HOST buffers (pinned for real overlap): chunked H2D/compute/D2H inside.
+        `x` is complex64, or interleaved integer pairs after set_input_format."""
+        x, n = _iq_input_checked(x, self._in_fmt)
+        return int(check(_L().qdsp_vfofm_process_host(self.h, x.ctypes.data, out.ctypes.data, n, int(block_size),
                                                       stream), "qdsp_vfofm_process_host"))
 
 
-class Channelizer(_Block):
+class Channelizer(_InputFormat, _Block):
     """nch x [VFO -> FloatFMDemod] fed by one Splitter (routing.h:47-57): every channel reads the same
-    device-resident wideband buffer; output is [nch, n_out] float32."""
+    device-resident wideband buffer; output is [nch, n_out] float32. set_input_format as VFOFM (the channelizer's
+    kernels read the input converted to cf32)."""
 
     _destroy = "qdsp_channelizer_destroy"
+    _set_fmt = "qdsp_channelizer_set_input_format"
     out_dtype = np.float32
 
     def __init__(self, offsets, inSampleRate, outSampleRate, bandWidth, deviation):
@@ -622,13 +671,34 @@ class Channelizer(_Block):
                                                        bs, stream), "qdsp_channelizer_process"))
 
     def process(self, x, block=None) -> np.ndarray:
-        x = np.ascontiguousarray(x, np.complex64)
-        n = len(x)
+        x, n = _iq_input(x, self._in_fmt)
         stride = (n * self._interp) // self._decim + 16
         din, dout = DevBuf.from_numpy(x), DevBuf(self.nch * stride * 4)
         m = self.process_device(din.ptr, dout.ptr, n, stride, block)
         y = dout.to_numpy(np.float32, self.nch * stride).reshape(self.nch, stride)[:, :m].copy()
         return y
+
+
+class IQConverter(_Block):
+    """Integer IQ from a radio front end -> complex_t (qdsp_iq_convert_process): y = (float(x) + offset) * scale per
+    component. Feeds any cf32 block (VFO, PSKDemod, ...). process() takes interleaved integer pairs."""
+
+    out_dtype = np.complex64
+
+    def __init__(self, fmt, scale=None, offset=None):
+        super().__init__()
+        self.fmt, self.code, self.scale, self.offset = _iq_format(fmt, scale, offset)
+        self.in_dtype = _synth.IQ_FORMATS[self.fmt][0]
+
+    def _run(self, in_ptr, out_ptr, n, block):
+        return _L().qdsp_iq_convert_process(self.code, self.scale, self.offset, in_ptr, out_ptr, n, self.stream)
+
+    def process(self, x, block=None) -> np.ndarray:
+        x, n = _iq_input(x, self.fmt)
+        din, dout = DevBuf.from_numpy(x), DevBuf(max(n, 1) * 8)
+        self.stream = None
+        m = int(check(self._run(din.ptr, dout.ptr, n, None), "IQConverter"))
+        return dout.to_numpy(np.complex64, m)
 
 
 # ---------------------------------------------------------------------------------------------

@@ -89,7 +89,39 @@ int import_tail_impl(History& hist, const void* tail_dev, int src_device, cudaSt
     return 0;
 }
 
+// the blocks that take a `dtype` read float or cf32 only (integer IQ goes through qdsp_iq_convert_process)
+bool real_or_complex(int dtype, const char* who) {
+    if (dtype == QDSP_F32 || dtype == QDSP_CF32) return true;
+    set_last_error("%s: dtype %d is not QDSP_F32 or QDSP_CF32", who, dtype);
+    return false;
+}
+
+// an integer IQ format and its conversion (include/qdsp_b200.h, qdsp_iq_convert_process)
+bool iq_format_ok(int fmt, float scale, float offset, const char* who) {
+    if (fmt != QDSP_CS16 && fmt != QDSP_CS8 && fmt != QDSP_CU8) {
+        set_last_error("%s: format %d is not QDSP_CS16, QDSP_CS8 or QDSP_CU8", who, fmt);
+        return false;
+    }
+    if (!isfinite(scale) || scale == 0.0f || !isfinite(offset)) {
+        set_last_error("%s: scale must be finite and non-zero, offset finite (got %g, %g)", who, (double)scale, (double)offset);
+        return false;
+    }
+    return true;
+}
+
 }  // namespace
+
+extern "C" long long qdsp_iq_convert_process(int fmt, float scale, float offset, const void* in_dev, void* out_dev,
+                                             long long count, qdsp_stream_t s) {
+    if (!iq_format_ok(fmt, scale, offset, "iq_convert_process")) return -1;
+    if (count < 0 || (count > 0 && (!in_dev || !out_dev)) ||
+        (reinterpret_cast<uintptr_t>(in_dev) % iq_pair_bytes(fmt)) != 0 || (reinterpret_cast<uintptr_t>(out_dev) & 7) != 0) {
+        set_last_error("iq_convert_process: bad arguments (input aligned to its pair, output to 8 bytes)");
+        return -1;
+    }
+    if (launch_iq_convert(fmt, IqConv{scale, offset}, in_dev, (float2*)out_dev, count, as_stream(s)) != 0) return -1;
+    return count;
+}
 
 // =================================================================================================
 // FIR
@@ -566,6 +598,19 @@ struct qdsp_channelizer {
     cudaStream_t last_stream = nullptr;
     const char* last_out = nullptr;
     size_t last_out_bytes = 0;
+    // element type of the input (set_input_format): integer input is converted to cf32 in `conv` (grown to the largest
+    // call, so the hot path stays allocation-free) and the kernels read that
+    int in_fmt = QDSP_CF32;
+    IqConv in_conv{1.0f, 0.0f};
+    Scratch conv;
+
+    int set_input_format(int fmt, float scale, float offset, const char* who) {
+        if (fmt != QDSP_CF32 && !iq_format_ok(fmt, scale, offset, who)) return -1;
+        last_serial = -1;
+        in_fmt = fmt;
+        in_conv = fmt == QDSP_CF32 ? IqConv{1.0f, 0.0f} : IqConv{scale, offset};
+        return 0;
+    }
 
     int upload_nco() {
         last_serial = -1;
@@ -623,6 +668,16 @@ struct qdsp_channelizer {
         float* dout = demod.p + (size_t)(cur ^ 1) * nch;
         int rc;
         const bool events = timing && !ring;
+        if (in_fmt != QDSP_CF32) {
+            // integer input: convert, then the cf32 path unchanged
+            if ((reinterpret_cast<uintptr_t>(in_dev) % iq_pair_bytes(in_fmt)) != 0) {
+                set_last_error("process: integer input must be aligned to its pair");
+                return -1;
+            }
+            if (conv.reserve((size_t)count * 8) != 0) return -1;
+            if (launch_iq_convert(in_fmt, in_conv, in_dev, (float2*)conv.p, count, s) != 0) return -1;
+            in_dev = conv.p;
+        }
         if (events) QDSP_CUDA_OK(cudaEventRecord(ev_k0, s));
         bool hist_folded = false;
         int rpad = -1;
@@ -759,7 +814,7 @@ long long qdsp_vfofm_process_host(qdsp_vfofm* h, const void* in_host, float* aud
             if (c.stage_out[i]) cudaFree(c.stage_out[i]);
             c.stage_in[i] = nullptr;
             c.stage_out[i] = nullptr;
-            QDSP_CUDA_OK(cudaMalloc(&c.stage_in[i], chunk * sizeof(float2)));
+            QDSP_CUDA_OK(cudaMalloc(&c.stage_in[i], chunk * sizeof(float2)));   // the widest format
             QDSP_CUDA_OK(cudaMalloc((void**)&c.stage_out[i], (chunk * c.interp / c.decim + 64) * sizeof(float)));
             if (!c.ev_done[i]) QDSP_CUDA_OK(cudaEventCreateWithFlags(&c.ev_done[i], cudaEventDisableTiming));
         }
@@ -769,6 +824,7 @@ long long qdsp_vfofm_process_host(qdsp_vfofm* h, const void* in_host, float* aud
     cudaEvent_t ev_h2d[2];
     for (int i = 0; i < 2; i++) QDSP_CUDA_OK(cudaEventCreateWithFlags(&ev_h2d[i], cudaEventDisableTiming));
     const char* src = (const char*)in_host;
+    const size_t E = (size_t)iq_pair_bytes(c.in_fmt);   // staged as given: 8, 4 or 2 bytes per sample cross the bus
     long long done = 0, produced = 0;
     int slot = 0;
     bool used[2] = {false, false};
@@ -776,8 +832,8 @@ long long qdsp_vfofm_process_host(qdsp_vfofm* h, const void* in_host, float* aud
         const long long n = count - done < (long long)chunk ? count - done : (long long)chunk;
         // the slot's previous kernel + D2H must have drained before its input buffer is overwritten
         if (used[slot]) QDSP_CUDA_OK(cudaStreamWaitEvent(c.copy_stream, c.ev_done[slot], 0));
-        QDSP_CUDA_OK(cudaMemcpyAsync(c.stage_in[slot], src + (size_t)done * sizeof(float2), (size_t)n * sizeof(float2),
-                                     cudaMemcpyHostToDevice, c.copy_stream));
+        QDSP_CUDA_OK(cudaMemcpyAsync(c.stage_in[slot], src + (size_t)done * E, (size_t)n * E, cudaMemcpyHostToDevice,
+                                     c.copy_stream));
         QDSP_CUDA_OK(cudaEventRecord(ev_h2d[slot], c.copy_stream));
         QDSP_CUDA_OK(cudaStreamWaitEvent(s, ev_h2d[slot], 0));
         const long long m = c.process(c.stage_in[slot], c.stage_out[slot], nullptr, 0, n, nullptr, 0, block_size, nullptr, s);
@@ -803,6 +859,10 @@ long long qdsp_vfofm_process_replay(qdsp_vfofm* h, const void* in_dev, float* au
     cudaStream_t s = as_stream(s_);
     if (c.nch != 1 || !ckpt_host) {
         set_last_error("vfofm_process_replay: bad arguments");
+        return -1;
+    }
+    if (c.in_fmt != QDSP_CF32) {
+        set_last_error("vfofm_process_replay: cf32 input only (set_input_format)");
         return -1;
     }
     if (c.part_replay.build(count, blocks, nblocks, block_size, c.interp, c.decim, s) != 0) return -1;
@@ -873,6 +933,9 @@ int qdsp_vfofm_reset(qdsp_vfofm* h) {
     c.abs_pos = 0;
     c.cur = 0;
     return 0;
+}
+int qdsp_vfofm_set_input_format(qdsp_vfofm* h, int fmt, float scale, float offset) {
+    return h->c.set_input_format(fmt, scale, offset, "vfofm_set_input_format");
 }
 int qdsp_vfofm_set_variant(qdsp_vfofm* h, int variant) {
     h->c.last_serial = -1;
@@ -972,6 +1035,9 @@ int qdsp_channelizer_reset(qdsp_channelizer* h) {
     h->abs_pos = 0;
     h->cur = 0;
     return 0;
+}
+int qdsp_channelizer_set_input_format(qdsp_channelizer* h, int fmt, float scale, float offset) {
+    return h->set_input_format(fmt, scale, offset, "channelizer_set_input_format");
 }
 int qdsp_channelizer_set_variant(qdsp_channelizer* h, int variant) {
     h->last_serial = -1;
@@ -1141,6 +1207,7 @@ int qdsp_cagc_get_state(qdsp_cagc* h, float* gain) { return h->st.get(gain, 1); 
 int qdsp_cagc_set_state(qdsp_cagc* h, float gain) { return h->st.set(&gain, 1); }
 
 qdsp_ffagc* qdsp_ffagc_create(int dtype) {
+    if (!real_or_complex(dtype, "ffagc_create")) return nullptr;
     qdsp_ffagc* h = new (std::nothrow) qdsp_ffagc();
     if (!h) return nullptr;
     h->dtype = dtype;
@@ -1373,7 +1440,7 @@ extern "C" {
 
 long long qdsp_math_process(int op, int dtype, const void* a_dev, const void* b_dev, void* out_dev, long long count,
                             qdsp_stream_t s) {
-    if (count < 0) return -1;
+    if (count < 0 || !real_or_complex(dtype, "math_process")) return -1;
     // math.h:32-37, 79-84, 126-131: complex/stereo add and subtract are float add/subtract over 2*count floats;
     // only Multiply<complex_t> is a complex product
     const long long nf = dtype == QDSP_CF32 ? 2 * count : count;
@@ -1415,7 +1482,7 @@ long long qdsp_layout_process(int op, const void* in0_dev, const void* in1_dev, 
 float qdsp_volume_level(float volume) { return powf(volume, 2); }   // Volume::setVolume, processing.h:373-374
 long long qdsp_volume_process(int dtype, float level, int muted, const void* in_dev, void* out_dev, long long count,
                               qdsp_stream_t s) {
-    if (count < 0) return -1;
+    if (count < 0 || !real_or_complex(dtype, "volume_process")) return -1;
     const long long nf = dtype == QDSP_CF32 ? 2 * count : count;
     if (muted) {   // processing.h:392-399
         if (count > 0 && cudaMemsetAsync(out_dev, 0, (size_t)nf * 4, as_stream(s)) != cudaSuccess) {
@@ -1564,6 +1631,7 @@ extern "C" {
 
 qdsp_mm* qdsp_mm_create(int dtype, float omega, float gainOmega, float muGain, float omegaRelLimit,
                         const float* interp_taps) {
+    if (!real_or_complex(dtype, "mm_create")) return nullptr;
     if (!interp_taps) {
         set_last_error("qdsp_mm_create: the 129 x 8 interpolator table is required");
         return nullptr;

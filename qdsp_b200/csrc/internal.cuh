@@ -112,6 +112,14 @@ template <typename T> struct VStream {
     }
 };
 
+// ---- integer IQ input (QDSP_CS16 / QDSP_CS8 / QDSP_CU8, include/qdsp_b200.h): bytes per (re, im) pair --------------
+inline int iq_pair_bytes(int fmt) {
+    return fmt == QDSP_CF32 ? 8 : fmt == QDSP_CS16 ? 4 : (fmt == QDSP_CS8 || fmt == QDSP_CU8) ? 2 : 0;
+}
+struct IqConv {
+    float scale, offset;
+};
+
 // ---- NCO bookkeeping (host) ----------------------------------------------------------------------
 // phase(n) = phase0 * exp(j*n*theta), theta = arg(phaseDelta) of the reference's float32 phasor
 // increment, kept as 64-bit fixed-point turns so any sample index is reachable in O(1).

@@ -340,4 +340,77 @@ int launch_sine(float2* out, long long count, uint64_t phase0, uint64_t step, fl
     return 0;
 }
 
+// ---- integer IQ -> cf32 (qdsp_iq_convert_process) ----------------------------------------------------------------------
+// The one conversion rule of the library: y = (float(x) + offset) * scale, each step rounded to float32 (numpy:
+// (x.astype(np.float32) + np.float32(offset)) * np.float32(scale)). float(x) is formed exactly on the ALU and FMA pipes
+// instead of I2F: the component, made unsigned (x + 2^15 / x + 2^7 for the signed formats), is placed in the low mantissa
+// bits of 2^23 by one PRMT, and 2^23 plus the bias is subtracted (exact below 2^24).
+template <int FMT>
+__device__ __forceinline__ float2 iq_finish(uint32_t m0, uint32_t m1, IqConv c) {
+    const float M = FMT == QDSP_CS16 ? 8421376.0f : FMT == QDSP_CS8 ? 8388736.0f : 8388608.0f;   // 2^23 + bias
+    const float2 x = __fadd2_rn(make_float2(__uint_as_float(m0), __uint_as_float(m1)), make_float2(-M, -M));
+    return __fmul2_rn(__fadd2_rn(x, make_float2(c.offset, c.offset)), make_float2(c.scale, c.scale));
+}
+// one cs16 sample from its 32-bit word
+__device__ __forceinline__ float2 iq_cs16(uint32_t w, IqConv c) {
+    const uint32_t u = w ^ 0x80008000u;
+    return iq_finish<QDSP_CS16>(__byte_perm(u, 0x4B000000u, 0x7410), __byte_perm(u, 0x4B000000u, 0x7432), c);
+}
+// two 8-bit samples from their 32-bit word (the low half only is meaningful for a single sample)
+template <int FMT>
+__device__ __forceinline__ float4 iq_b8x2(uint32_t w, IqConv c) {
+    const uint32_t u = FMT == QDSP_CS8 ? (w ^ 0x80808080u) : w;
+    const float2 s0 = iq_finish<FMT>(__byte_perm(u, 0x4B000000u, 0x7440), __byte_perm(u, 0x4B000000u, 0x7441), c);
+    const float2 s1 = iq_finish<FMT>(__byte_perm(u, 0x4B000000u, 0x7442), __byte_perm(u, 0x4B000000u, 0x7443), c);
+    return make_float4(s0.x, s0.y, s1.x, s1.y);
+}
+template <int FMT>
+__device__ __forceinline__ float2 iq_one(const void* in, long long i, IqConv c) {
+    if (FMT == QDSP_CS16) return iq_cs16(reinterpret_cast<const uint32_t*>(in)[i], c);
+    const float4 v = iq_b8x2<FMT>(reinterpret_cast<const uint16_t*>(in)[i], c);
+    return make_float2(v.x, v.y);
+}
+// Two samples per thread: one 8-byte (cs16) or 4-byte (8-bit) load and one 16-byte store, so a warp's loads and stores
+// each cover one contiguous range. That needs the pair of samples aligned in the input and 16-byte aligned in the
+// output from sample `head` (0 or 1) on; the head, the odd tail, and everything when the two alignments disagree, go
+// one sample per thread (still contiguous across the warp).
+template <int FMT>
+__global__ void __launch_bounds__(256) iq_convert_kernel(const void* __restrict__ in, float2* __restrict__ out, long long count,
+                                                         long long head, long long npairs, IqConv c) {
+    constexpr int E = FMT == QDSP_CS16 ? 4 : 2;   // input bytes per sample
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    const long long tid = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    const char* in2 = reinterpret_cast<const char*>(in) + head * E;
+    float4* out2 = reinterpret_cast<float4*>(out + head);
+    for (long long p = tid; p < npairs; p += stride) {
+        float4 v;
+        if (FMT == QDSP_CS16) {
+            const uint2 w = __ldcs(reinterpret_cast<const uint2*>(in2) + p);
+            const float2 s0 = iq_cs16(w.x, c), s1 = iq_cs16(w.y, c);
+            v = make_float4(s0.x, s0.y, s1.x, s1.y);
+        } else {
+            v = iq_b8x2<FMT>(__ldcs(reinterpret_cast<const unsigned int*>(in2) + p), c);
+        }
+        out2[p] = v;
+    }
+    const long long tail0 = head + 2 * npairs;
+    for (long long i = tid; i < head + (count - tail0); i += stride) {
+        const long long j = i < head ? i : tail0 + (i - head);
+        out[j] = iq_one<FMT>(in, j, c);
+    }
+}
+int launch_iq_convert(int fmt, IqConv c, const void* in, float2* out, long long count, cudaStream_t s) {
+    if (count <= 0) return 0;
+    const int E = iq_pair_bytes(fmt);
+    const long long head = (reinterpret_cast<uintptr_t>(in) % (2 * E)) ? 1 : 0;
+    long long npairs = count > head ? (count - head) / 2 : 0;
+    if (!aligned16(out + head)) npairs = 0;
+    const int g = pw_grid(npairs > 0 ? npairs : count, 256, 8);
+    if (fmt == QDSP_CS16) iq_convert_kernel<QDSP_CS16><<<g, 256, 0, s>>>(in, out, count, head, npairs, c);
+    else if (fmt == QDSP_CS8) iq_convert_kernel<QDSP_CS8><<<g, 256, 0, s>>>(in, out, count, head, npairs, c);
+    else iq_convert_kernel<QDSP_CU8><<<g, 256, 0, s>>>(in, out, count, head, npairs, c);
+    QDSP_LAUNCH_OK();
+    return 0;
+}
+
 }  // namespace qdsp

@@ -129,6 +129,8 @@ int launch_sine(float2* out, long long count, uint64_t phase0, uint64_t step, fl
                 cudaStream_t s);
 int launch_ssb(const float2* in, float* out, long long count, uint64_t phase0, uint64_t step, float2 inc1, float2 inc2,
                float2 inc3, cudaStream_t s);
+// integer IQ (fmt QDSP_CS16 / QDSP_CS8 / QDSP_CU8, `in` aligned to its pair) -> cf32 (`out` 8-byte aligned)
+int launch_iq_convert(int fmt, IqConv c, const void* in, float2* out, long long count, cudaStream_t s);
 
 // ---- k_clock.cu: MMClockRecovery (sequential-exact, one warp per stream) --------------------------
 int launch_mm(int cplx, const void* in, const Partition& part, const float* taps_dev, float omega, float gainOmega,

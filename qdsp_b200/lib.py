@@ -16,6 +16,7 @@ LIB_PATH = os.path.join(HERE, "libqdsp_b200.so")
 HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "qdsp_b200.h")
 
 F32, CF32 = 0, 1
+CS16, CS8, CU8 = 2, 3, 4    # integer IQ: interleaved (re, im) int16 / int8 / uint8 pairs
 
 _f, _d, _i, _u, _ll, _ull = C.c_float, C.c_double, C.c_int, C.c_uint, C.c_longlong, C.c_ulonglong
 _vp, _sz = C.c_void_p, C.c_size_t
@@ -50,6 +51,7 @@ SIGNATURES = {
     "qdsp_event_record": (_i, [_vp, _vp]),
     "qdsp_stream_wait_event": (_i, [_vp, _vp]),
     "qdsp_event_sync": (_i, [_vp]),
+    "qdsp_iq_convert_process": (_ll, [_i, _f, _f, _vp, _vp, _ll, _vp]),
     "qdsp_blackman_tap_count": (_i, [_f, _f, _f]),
     "qdsp_blackman_taps": (None, [_f, _f, _f, _fp, _i, _f]),
     "qdsp_blackman_bandpass_taps": (None, [_f, _f, _f, _f, _fp, _i, _f]),
@@ -109,6 +111,7 @@ SIGNATURES = {
     "qdsp_vfofm_process_replay": (_ll, [_vp, _vp, _vp, _vp, _ll, _ip, _i, _i, _fp, _ll, _vp]),
     "qdsp_vfofm_reset": (_i, [_vp]),
     "qdsp_vfofm_set_variant": (_i, [_vp, _i]),
+    "qdsp_vfofm_set_input_format": (_i, [_vp, _i, _f, _f]),
     "qdsp_vfofm_seek": (_i, [_vp, _ll]),
     "qdsp_vfofm_import_tail": (_i, [_vp, _vp, _i, _vp]),
     "qdsp_vfofm_history_len": (_i, [_vp]),
@@ -122,6 +125,7 @@ SIGNATURES = {
     "qdsp_channelizer_process": (_ll, [_vp, _vp, _vp, _ll, _ll, _ip, _i, _i, _vp]),
     "qdsp_channelizer_reset": (_i, [_vp]),
     "qdsp_channelizer_set_variant": (_i, [_vp, _i]),
+    "qdsp_channelizer_set_input_format": (_i, [_vp, _i, _f, _f]),
     "qdsp_channelizer_seek": (_i, [_vp, _ll]),
     "qdsp_deemp_create": (_vp, [_f, _f]),
     "qdsp_deemp_destroy": (None, [_vp]),

@@ -114,3 +114,30 @@ def stereo_mpx_fm_cf32(start: int, count: int, fs: int = 240_000, dev: float = 7
             integ += sgn * 0.45 * 0.5 * s2 * np.sin(2.0 * np.pi * _frac(n, fb, fs)) / (2.0 * np.pi * fb)
     ph = 2.0 * np.pi * dev * integ
     return (amp * np.exp(1j * ph)).astype(np.complex64)
+
+
+# ---- integer IQ (include/qdsp_b200.h, QDSP_CS16 / QDSP_CS8 / QDSP_CU8) ----------------------------------------------
+# format -> (numpy dtype of a component, the usual (scale, offset)); the conversion is y = (float(x) + offset) * scale
+IQ_FORMATS = {
+    "cs16": (np.int16, 1.0 / 32768, 0.0),
+    "cs8": (np.int8, 1.0 / 128, 0.0),
+    "cu8": (np.uint8, 1.0 / 128, -127.5),
+}
+IQ_CODES = {"cs16": 2, "cs8": 3, "cu8": 4}
+
+
+def iq_to_cf32(raw: np.ndarray, scale: float, offset: float) -> np.ndarray:
+    """The library's conversion rule on the host: interleaved integer pairs -> complex64, each step rounded to float32."""
+    y = (np.asarray(raw).reshape(-1).astype(np.float32) + np.float32(offset)) * np.float32(scale)
+    return y.view(np.complex64)
+
+
+def quantize_iq(x: np.ndarray, fmt: str, scale: float | None = None, offset: float | None = None) -> np.ndarray:
+    """cf32 -> interleaved integer pairs of `fmt` (round to nearest, saturate): the inverse of iq_to_cf32 up to the
+    quantisation step. Test inputs as a radio front end would deliver them."""
+    dt, s0, o0 = IQ_FORMATS[fmt]
+    scale = s0 if scale is None else scale
+    offset = o0 if offset is None else offset
+    info = np.iinfo(dt)
+    f = np.asarray(x, np.complex64).view(np.float32).astype(np.float64)
+    return np.clip(np.rint(f / scale - offset), info.min, info.max).astype(dt)

@@ -364,13 +364,6 @@ int qdsp_mm_set_omega_rel_limit(qdsp_mm* h, float omegaRelLimit);              /
 long long qdsp_mm_max_out(qdsp_mm* h, long long count);
 long long qdsp_mm_process(qdsp_mm* h, const void* in_dev, void* out_dev, long long count, const int* blocks, int nblocks,
                           int block_size, int* out_counts, qdsp_stream_t s);
-/* speculate and verify for one long stream: chunks of `chunk` samples are walked in parallel, each from the default
- * loop state `warmup` samples before its boundary, and accepted only where their loop state at the boundary is
- * bit-equal to what the verified predecessor hands over (otherwise re-walked from the true state): same symbols,
- * counts and state as the sequential walk by construction. chunk = 0 (default) = sequential walk. After a process
- * call, qdsp_mm_last_rewalked() tells how many chunks had to be re-walked. */
-int qdsp_mm_set_speculation(qdsp_mm* h, int chunk, int warmup);
-int qdsp_mm_last_rewalked(qdsp_mm* h);
 /* state[44]: mu, dynOmega, lastOutput, p_0T p_1T p_2T, c_0T c_1T c_2T, nextOffset, delay[0..6] (re, im pairs) */
 int qdsp_mm_get_state(qdsp_mm* h, float state[44]);
 int qdsp_mm_set_state(qdsp_mm* h, const float state[44]);

@@ -1158,13 +1158,6 @@ class MMClockRecovery:
     def setOmegaRelLimit(self, v):  # noqa: N802
         check(_L().qdsp_mm_set_omega_rel_limit(self.h, float(v)))
 
-    def set_speculation(self, chunk: int, warmup: int):
-        """Parallel speculate-and-verify walk (exact by construction); chunk = 0 -> sequential walk."""
-        check(_L().qdsp_mm_set_speculation(self.h, int(chunk), int(warmup)))
-
-    def last_rewalked(self) -> int:
-        return int(_L().qdsp_mm_last_rewalked(self.h))
-
     def get_state(self) -> np.ndarray:
         st = np.zeros(44, np.float32)
         check(_L().qdsp_mm_get_state(self.h, _fptr(st)))

@@ -1081,7 +1081,7 @@ struct qdsp_costas {
     // measured on B200 (2^26 QPSK samples, tools/_costas_sweep.py): (4096, 4096) 38 GS/s, (2048, 2048) 49 GS/s with the same
     // 4e-6 error against the sequential loop; 1536 warm-up samples: 53 GS/s but 2e-5; 1024: 1e-3 (not merged)
     int chunk = 2048, warmup = 2048;
-    bool chunk_user = false;   // set_chunking() / environment: keep; otherwise long calls use 4096-sample chunks
+    bool chunk_user = false;   // set_chunking(): keep; otherwise long calls use 4096-sample chunks
     DevState st;   // [4] state + [1] residual
     Scratch scratch;
 };
@@ -1265,11 +1265,6 @@ qdsp_costas* qdsp_costas_create(int order, float loopBandwidth) {
         h->warmup = ((int)w + 15) / 16 * 16;
         h->chunk = h->warmup > 2048 ? h->warmup : 2048;
     }
-    if (const char* e = getenv("QDSP_COSTAS_CHUNK")) {      // A/B switches
-        h->chunk = atoi(e) >= 16 ? atoi(e) / 16 * 16 : h->chunk;
-        h->chunk_user = true;
-    }
-    if (const char* e = getenv("QDSP_COSTAS_WARMUP")) h->warmup = atoi(e) >= 0 ? atoi(e) / 16 * 16 : h->warmup;
     const float init[5] = {0.0f, 0.0f, 1.0f, 0.0f, 0.0f};
     if (h->st.init(5, init) != 0) {
         delete h;
@@ -1618,10 +1613,7 @@ struct qdsp_mm {
     DevState st;             // 44 floats, layout of oracle/port.c port_mm
     float* taps_dev = nullptr;
     Partition part;
-    Scratch scratch;         // one long long + one int + [nblocks] ints
-    Scratch spec_scratch;    // speculate-and-verify: per-chunk states, counts, offsets, values, source indices
-    int spec_chunk = 0, spec_warm = 0;   // 0 = sequential-exact single walk
-    int last_rewalked = 0;
+    Scratch scratch;         // the total output count (long long) at byte 0, [nblocks] per-block counts at byte 16
     ~qdsp_mm() {
         if (taps_dev) cudaFree(taps_dev);
     }
@@ -1677,22 +1669,6 @@ int qdsp_mm_set_omega_rel_limit(qdsp_mm* h, float omegaRelLimit) {   // :106-112
     h->omegaMax = h->omega + (h->omega * h->rel);
     return 0;
 }
-int qdsp_mm_set_speculation(qdsp_mm* h, int chunk, int warmup) {
-#ifndef QDSP_MM_SPECULATION
-    if (chunk != 0) {
-        set_last_error("qdsp_mm_set_speculation: experimental variant not compiled in (-DQDSP_MM_SPECULATION)");
-        return -1;
-    }
-#endif
-    if (chunk != 0 && (warmup < 0 || chunk < warmup + 8)) {
-        set_last_error("qdsp_mm_set_speculation: need chunk >= warmup + 8");
-        return -1;
-    }
-    h->spec_chunk = chunk;
-    h->spec_warm = warmup;
-    return 0;
-}
-int qdsp_mm_last_rewalked(qdsp_mm* h) { return h->last_rewalked; }
 int qdsp_mm_get_state(qdsp_mm* h, float state[44]) { return h->st.get(state, 44); }
 int qdsp_mm_set_state(qdsp_mm* h, const float state[44]) { return h->st.set(state, 44); }
 long long qdsp_mm_max_out(qdsp_mm* h, long long count) {
@@ -1709,28 +1685,11 @@ long long qdsp_mm_process(qdsp_mm* h, const void* in_dev, void* out_dev, long lo
     if (nb == 0) return 0;
     if (h->scratch.reserve(sizeof(int) * (size_t)nb + 32) != 0) return -1;
     long long* total_dev = (long long*)h->scratch.p;
-    int* rewalked_dev = (int*)((char*)h->scratch.p + 8);
     int* oc_dev = (int*)((char*)h->scratch.p + 16);
-    h->last_rewalked = 0;
-    // speculate and verify: chunks walked in parallel from the default loop state, accepted only where they provably
-    // coincide with the sequential walk (k_clock.cu). Needs omega >= 1 (the reference's 2*omega*count output cap can
-    // then never fire) and at least two chunks.
-    const bool spec = h->spec_chunk > 0 && h->omegaMin >= 1.0f && count >= 2ll * h->spec_chunk;
-    if (spec) {
-        int cap = (int)((double)h->spec_chunk / (double)h->omegaMin) + 4;
-        cap += cap & 1;
-        if (h->spec_scratch.reserve(mm_spec_scratch_bytes(count, h->spec_chunk, cap)) != 0) return -1;
-        if (launch_mm_spec(h->dtype == QDSP_CF32, in_dev, h->part, h->taps_dev, h->gainOmega, h->muGain, h->omegaMin,
-                           h->omegaMax, h->st.p, out_dev, oc_dev, total_dev, rewalked_dev, h->spec_chunk, h->spec_warm, cap,
-                           h->spec_scratch.p, s) != 0)
-            return -1;
-        QDSP_CUDA_OK(cudaMemcpyAsync(&h->last_rewalked, rewalked_dev, sizeof(int), cudaMemcpyDeviceToHost, s));
-    } else if (launch_mm(h->dtype == QDSP_CF32, in_dev, h->part, h->taps_dev, h->omega, h->gainOmega, h->muGain, h->omegaMin,
-                         h->omegaMax, h->st.p, out_dev, oc_dev, total_dev, s) != 0) {
+    if (launch_mm(h->dtype == QDSP_CF32, in_dev, h->part, h->taps_dev, h->omega, h->gainOmega, h->muGain, h->omegaMin,
+                  h->omegaMax, h->st.p, out_dev, oc_dev, total_dev, s) != 0)
         return -1;
-    }
     // the output count is data dependent: this call waits for the kernel
-    (void)0;
     long long total = 0;
     QDSP_CUDA_OK(cudaMemcpyAsync(&total, total_dev, sizeof(total), cudaMemcpyDeviceToHost, s));
     if (out_counts) QDSP_CUDA_OK(cudaMemcpyAsync(out_counts, oc_dev, sizeof(int) * (size_t)nb, cudaMemcpyDeviceToHost, s));

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdlib.h>
 #include <atomic>
 #include <vector>
 #include "common.cuh"
@@ -23,6 +24,25 @@ inline void count_launch(int n = 1) { g_launches.fetch_add(n, std::memory_order_
     } while (0)
 
 inline cudaStream_t as_stream(qdsp_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// Launches kern(*arg) (one kernel-parameter struct). overlap: programmatic dependent launch -- the grid may start while
+// the previous grid of the stream drains, the kernel orders what it shares with it by griddepcontrol.wait (a no-op
+// without the attribute). QDSP_PDL=0 never overlaps: the serialized reference of the overlapped-call tests.
+inline cudaError_t launch_ex(const void* kern, dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool overlap, void* arg) {
+    static const bool pdl = getenv("QDSP_PDL") ? atoi(getenv("QDSP_PDL")) != 0 : true;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = (overlap && pdl) ? 1 : 0;
+    void* args[1] = {arg};
+    return cudaLaunchKernelExC(&cfg, kern, args);
+}
 
 // ---- block partition of a batch of run() calls ------------------------------------------------
 // The reference restarts the resampler schedule (and the AGC decay) at every run() call, so the

@@ -245,16 +245,16 @@ template <int DS, int DC, bool ROT>
 __global__ void __launch_bounds__(32) chan_kernel(const __grid_constant__ ChanArgs ca) {
     chan_dispatch<DS, DC, ROT, 0>((int)blockIdx.z, ca);
 }
-template <int DS, int DC, bool ROT, int NRT>
+// NR = 2: one set of shared-memory tap loads feeds two rows
+template <int DS, int DC, bool ROT>
 __global__ void __launch_bounds__(32) chan_smemtaps_kernel(const __grid_constant__ ChanArgs ca) {
-    chan_body<DS, DC, ROT, -1, NRT>(ca);
+    chan_body<DS, DC, ROT, -1, 2>(ca);
 }
 
 // ---- host side -------------------------------------------------------------------------------------
 bool chan_supported(const DecimPlan* plan) {
-    static const bool on = getenv("QDSP_CHAN") ? atoi(getenv("QDSP_CHAN")) != 0 : true;
     // wide rows of a geometry instantiated below, 8 full tap rows + at most the two stray taps of row 8
-    return on && (plan->DS == 1280 || plan->DS == 128) && plan->T + 1 <= 8 * plan->DS + 2 && plan->T > 4 * plan->DS;
+    return (plan->DS == 1280 || plan->DS == 128) && plan->T + 1 <= 8 * plan->DS + 2 && plan->T > 4 * plan->DS;
 }
 
 // The constant bank holds ONE plan's taps at a time. Uploads are enqueued on the launching stream (stream-ordered with
@@ -308,9 +308,8 @@ static int launch_chan_t(DecimPlan* plan, const float* taps_host, const float2* 
     ca.g8[1] = h(8ll * DS + 1 - pad);
     ca.taps_dev = g_chan_taps_dev;
     // outputs per segment (CTA): enough single-warp CTAs to fill the machine several times over; the halo is 8 rows
-    static const int seg_env = getenv("QDSP_CHAN_SEG") ? atoi(getenv("QDSP_CHAN_SEG")) : 0;
     // B200, 2^26 samples (GS/s wideband): 32 ch (1 group): 80: 27.0, 128: 31.0, 160: 29.3, 320: 29.5; 256 ch: 128: 4.41, 160: 4.44, 320: 3.69
-    ca.seg_rows = seg_env > 0 ? seg_env : (ca.groups < 4 ? 128 : 160);
+    ca.seg_rows = ca.groups < 4 ? 128 : 160;
     dim3 grid((part.max_out + ca.seg_rows - 1) / ca.seg_rows, part.view.nblocks * ca.groups, ca.nslices);
     if (grid.y > 65535) {
         set_last_error("chan: too many run() blocks x channel groups (%u)", grid.y);
@@ -318,16 +317,10 @@ static int launch_chan_t(DecimPlan* plan, const float* taps_host, const float2* 
     }
     // few channel groups: the slice bodies with immediate taps would be resident side by side (instruction-cache thrash);
     // use the one-body variant with taps in shared memory
-    static const int smt_env = getenv("QDSP_CHAN_SMEMTAPS") ? atoi(getenv("QDSP_CHAN_SMEMTAPS")) : -1;
-    const bool smemtaps = smt_env >= 0 ? smt_env != 0 : ca.groups < 4;
+    const bool smemtaps = ca.groups < 4;
     constexpr size_t smem = 4 * 4 * DC * 8 + 64 + 8 * DC * 4 + 64;
-    static const int nr_env = getenv("QDSP_CHAN_NR") ? atoi(getenv("QDSP_CHAN_NR")) : 2;
-    if (rot && smemtaps && nr_env == 2) {
-        auto kern = chan_smemtaps_kernel<DS, DC, true, 2>;
-        QDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<grid, 32, smem, s>>>(ca);
-    } else if (rot && smemtaps) {
-        auto kern = chan_smemtaps_kernel<DS, DC, true, 1>;
+    if (rot && smemtaps) {
+        auto kern = chan_smemtaps_kernel<DS, DC, true>;
         QDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<grid, 32, smem, s>>>(ca);
     } else if (rot) {

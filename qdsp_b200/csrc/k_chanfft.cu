@@ -384,16 +384,14 @@ __global__ void __launch_bounds__(kCfM, 2) chanfft_fft_kernel(const ChanFftBArgs
 
 // ---- host side -------------------------------------------------------------------------------------
 ChanFftPlan* chanfft_plan_create(const float* taps, int T, int interp, int decim, int nch, const uint64_t* nco_steps) {
-    static const bool on = getenv("QDSP_CHAN_FFT") ? atoi(getenv("QDSP_CHAN_FFT")) != 0 : true;
-    static const bool force_rot = getenv("QDSP_CHANFFT_ROT") ? atoi(getenv("QDSP_CHANFFT_ROT")) != 0 : false;
-    if (!on || interp != 1 || nch != kCfM || decim != kCfDR * kCfM || T + 1 > kCfJ * kCfM) return nullptr;
+    if (interp != 1 || nch != kCfM || decim != kCfDR * kCfM || T + 1 > kCfJ * kCfM) return nullptr;
     const double to_rad = 6.283185307179586476925286766559 / 18446744073709551616.0;
     // is channel 0 on the half-bin grid of the M-point FFT (theta_0 = 2 pi hb / (2 M) within rounding)? then no pre-rotation
     // is needed: e^{j theta_0 (A + r + M j)} = [row phase] x [bin shift hb / 2] x [column twist e^{j pi r / M} if hb is odd] x
     // [(-1)^j if hb is odd: folded into the taps]. Otherwise rotate the stream by channel 0's NCO first (hb = 0).
     const uint64_t hb_near = (nco_steps[0] + (1ull << 54)) >> 55;
     const long long res0 = (long long)(nco_steps[0] - (hb_near << 55));
-    const bool rotate = force_rot || fabs((double)res0 * to_rad) > 2e-6;
+    const bool rotate = fabs((double)res0 * to_rad) > 2e-6;
     const uint64_t base = rotate ? nco_steps[0] : (hb_near << 55);
     const int twob = rotate ? 0 : (int)(hb_near & (2 * kCfM - 1));
     // channel k must sit on the bin grid: theta_k = base - 2 pi k / M + delta_k with a tiny delta_k
@@ -504,8 +502,7 @@ int launch_chanfft(ChanFftPlan* plan, const float2* hist, int H, const float2* i
     a.part = part.view;
     a.T = plan->T;
     a.pad = plan->T & 1;                 // blocks start on multiples of D (even): the window start parity is T's
-    static const int seg_env = getenv("QDSP_CHANFFT_SEG") ? atoi(getenv("QDSP_CHANFFT_SEG")) : 0;
-    a.seg_rows = seg_env > 0 ? seg_env : chanfft_pick_seg(part);
+    a.seg_rows = chanfft_pick_seg(part);
     a.abs0 = abs0;
     a.beta_step = beta_step;
     a.beta_ph0 = beta_ph0;

@@ -40,15 +40,15 @@ __host__ __device__ inline int decim_ppad_sup(int P) {
 // packed f32x2 helpers for the two-column phasor recurrence
 __device__ __forceinline__ float2 neg2(float2 v) { return make_float2(-v.x, -v.y); }
 
-template <int Q, int DT, int NSEGT, bool ROT, bool DEMOD, bool SUPRED, int MAXT, int MINB>
+template <int Q, bool ROT, bool DEMOD, bool SUPRED, int MAXT, int MINB>
 __global__ void __launch_bounds__(MAXT, MINB) decim_kernel(const DecimArgs a) {
     constexpr int R = 3;            // rows per stage per segment
     constexpr int NS = Q / R;       // stages per super-iteration == ring depth: slot index is static
     constexpr int LEAD = DEMOD ? 1 : 0;
     static_assert(Q % R == 0 && NS >= 2, "Q must be a multiple of 3, at least 6");
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int D = DT ? DT : a.D;                 // compile-time in the specialised instantiations:
-    const int NSEG = NSEGT ? NSEGT : a.NSEG;     // all shared-memory offsets fold into immediates
+    const int D = a.D;
+    const int NSEG = a.NSEG;
     const int P = D / 2, L = a.L;
     const int t = threadIdx.x;
     const int tile_x = a.plane_fast ? blockIdx.y : blockIdx.x;
@@ -86,7 +86,7 @@ __global__ void __launch_bounds__(MAXT, MINB) decim_kernel(const DecimArgs a) {
     uint64_t* mbar = reinterpret_cast<uint64_t*>(ybuf + NSEG * LL);                          // [NS]
     float* s_misc = reinterpret_cast<float*>(mbar + NS);                                     // [0]=override angle
     // wide rows (more than 64 column pairs): the partial reduce runs in two levels, P -> 64 -> 1
-    const bool two_level = (DT == 0) && P > 64;
+    const bool two_level = P > 64;
     float2* P2 = reinterpret_cast<float2*>(s_misc + 4);                                      // [2][NSEG*R][64]
 
     // ---- thread roles ------------------------------------------------------------------------
@@ -282,22 +282,10 @@ __global__ void __launch_bounds__(MAXT, MINB) decim_kernel(const DecimArgs a) {
         float2 sacc = make_float2(0.f, 0.f);
         if (ovalid) {
             const float2* pb = reinterpret_cast<const float2*>(pbr + par * pbuf_half);
-            if (DT) {
-                constexpr int NPP = ((DT ? DT : 2) / 2 + 7) / 8;
-#pragma unroll
-                for (int i8 = 0; i8 < NPP; i8++) {
-                    if (u + 8 * i8 < P) {
-                        const float2 v = pb[8 * i8];
-                        sacc.x += v.x;
-                        sacc.y += v.y;
-                    }
-                }
-            } else {
-                for (int pp = u; pp < P; pp += 8) {
-                    const float2 v = pb[pp - u];
-                    sacc.x += v.x;
-                    sacc.y += v.y;
-                }
+            for (int pp = u; pp < P; pp += 8) {
+                const float2 v = pb[pp - u];
+                sacc.x += v.x;
+                sacc.y += v.y;
             }
         }
         finish_output(it, sacc);
@@ -311,14 +299,7 @@ __global__ void __launch_bounds__(MAXT, MINB) decim_kernel(const DecimArgs a) {
         const int s2 = o2 / Q, i2 = o2 - s2 * Q;
         if (v2) {
             const float2* pb = reinterpret_cast<const float2*>(reinterpret_cast<const unsigned char*>(Pbuf) + (sup & 1) * pbuf_half) + o2 * Ppad;
-            if (DT) {
-                constexpr int NP2 = ((DT ? DT : 2) / 2 + 1) / 2;
-#pragma unroll
-                for (int i = 0; i < NP2; i++)
-                    if (u2 + 2 * i < P) sacc = __fadd2_rn(sacc, pb[u2 + 2 * i]);
-            } else {
-                for (int pp = u2; pp < P; pp += 2) sacc = __fadd2_rn(sacc, pb[pp]);
-            }
+            for (int pp = u2; pp < P; pp += 2) sacc = __fadd2_rn(sacc, pb[pp]);
         }
         sacc.x += __shfl_xor_sync(0xffffffffu, sacc.x, 1);
         sacc.y += __shfl_xor_sync(0xffffffffu, sacc.y, 1);
@@ -453,10 +434,10 @@ __global__ void __launch_bounds__(MAXT, MINB) decim_kernel(const DecimArgs a) {
 // 3 CTAs/SM 585. Without the finishing pass the kernel runs at 725 (the data-movement ceiling of this layout is
 // 715-745), i.e. what is left is the aux warp's latency chain and one stage of prefetch depth.
 // Compile-time geometry only (D, NSEG); 160-thread CTAs, 4 per SM.
-template <int Q, int D, int NSEG, int NSLOTT = 2>
+template <int Q, int D, int NSEG>
 struct SupGeom {
     static constexpr int P = D / 2;
-    static constexpr int NSLOT = NSLOTT;
+    static constexpr int NSLOT = 2;
     static constexpr int chunk_elems = Q * D;
     static constexpr uint32_t chunk_bytes = (uint32_t)chunk_elems * 8u;
     static constexpr int seg_pad = ((((D * 8) % 128) - (int)(chunk_bytes % 128u)) % 128 + 128) % 128 / 8;
@@ -475,10 +456,10 @@ struct SupGeom {
 
 __device__ __forceinline__ void cta_sync() { asm volatile("bar.sync 0;" ::: "memory"); }
 
-template <int Q, int DT, int NSEGT, bool ROT, bool DEMOD, int NSLOTT = 2, int DBG = 0>
-__global__ void __launch_bounds__(NSLOTT == 3 ? 192 : 160, NSLOTT == 3 ? 3 : 4) decim_sup_kernel(const DecimArgs a) {
-    using G = SupGeom<Q, DT, NSEGT, NSLOTT>;
-    constexpr int D = DT, NSEG = NSEGT, P = G::P;
+template <int Q, int D, int NSEG, bool ROT, bool DEMOD>
+__global__ void __launch_bounds__(160, 4) decim_sup_kernel(const DecimArgs a) {
+    using G = SupGeom<Q, D, NSEG>;
+    constexpr int P = G::P;
     constexpr int LEAD = DEMOD ? 1 : 0;
     constexpr int NSLOT = G::NSLOT;
     static_assert(NSEG * P <= 128 && NSEG <= 32, "CTA geometry");
@@ -541,9 +522,8 @@ __global__ void __launch_bounds__(NSLOTT == 3 ? 192 : 160, NSLOTT == 3 ? 3 : 4) 
     }
     cta_sync();
 
-    constexpr bool TWO_AUX = NSLOTT == 3;
     if (warp >= 4) {
-        const int ap = warp - 4;   // TWO_AUX: warp 4 = producer + pass 0, warp 5 = pass 1
+        const int ap = warp - 4;   // aux warp: 0 = producer + finisher (160-thread CTAs have no other)
         // ================= producer + finisher warp =====================================================
         const long long tile_first = bi.in_start + (long long)(k0 - LEAD) * DSg - a.T - pad + col_off;
         const long long tile_last = tile_first + (long long)(nactive - 1) * L * DSg + (long long)(nsup - 1) * chunk_span + chunk_tail;
@@ -601,7 +581,6 @@ __global__ void __launch_bounds__(NSLOTT == 3 ? 192 : 160, NSLOTT == 3 ? 3 : 4) 
         auto finish = [&](int sup, int par) {
 #pragma unroll
             for (int p = 0; p < G::NPASS; p++) {
-                if (TWO_AUX && p != ap) continue;
                 const int fs = p * G::SA + fls;
                 const bool fvalid = fls < G::SA && fs < NSEG;
                 const float4* pb = reinterpret_cast<const float4*>(
@@ -652,7 +631,7 @@ __global__ void __launch_bounds__(NSLOTT == 3 ? 192 : 160, NSLOTT == 3 ? 3 : 4) 
         for (int sup = 0; sup < nsup; sup++) {
             cta_sync();                  // compute warps are done with slot `slot`; partials of `sup` visible
             if (ap == 0) issue(sup + NSLOT, slot);
-            if (DBG != 2) finish(sup, sup & 1);
+            finish(sup, sup & 1);
             slot = slot == NSLOT - 1 ? 0 : slot + 1;
         }
         return;
@@ -704,7 +683,7 @@ __global__ void __launch_bounds__(NSLOTT == 3 ? 192 : 160, NSLOTT == 3 ? 3 : 4) 
             PI = make_float2(p0.y, p1.y);
         }
         mbar_wait(&mbar[slot], parity);
-        if (seg_active && DBG != 1) {
+        if (seg_active) {
             const unsigned char* xs_ = xme + slot * G::stage_bytes;
             unsigned char* ps_ = pme + (sup & 1) * G::pbuf_half;
 #pragma unroll
@@ -770,8 +749,7 @@ DecimPlan* decim_plan_create(const float* taps, int T, int D) {
     p->nslices = 1;
     // wide rows (config 4: D = 1280) are cut into 128-column slices: each slice is a narrow-row stream of its own
     // (128-thread CTAs, 2-lane partial reduce) whose partial outputs finish_kernel sums
-    static const bool slice_env = getenv("QDSP_DECIM_SLICE") ? atoi(getenv("QDSP_DECIM_SLICE")) != 0 : true;
-    if (slice_env && D > 128 && D % 128 == 0) p->nslices = D / 128;
+    if (D > 128 && D % 128 == 0) p->nslices = D / 128;
     const int Dc = D / p->nslices;
     p->D = Dc;
     p->P = Dc / 2;
@@ -784,16 +762,14 @@ DecimPlan* decim_plan_create(const float* taps, int T, int D) {
     // CTA barrier then only couples 4 warps while four other CTAs keep the SM busy
     int nseg = 128 / p->P >= 1 ? 128 / p->P : 320 / p->P;
     if (nseg > 13) nseg = 13;
-    if (const char* e = getenv("QDSP_DECIM_NSEG")) nseg = atoi(e) < nseg ? atoi(e) : nseg;
     if (nseg < 1) nseg = 1;
     p->NSEG = nseg;
     int nt = nseg * p->P > nseg * 24 ? nseg * p->P : nseg * 24;   // 24 >= Q: also enough epilogue threads
     p->NT = ((nt + 31) / 32) * 32;
     if (p->NT < 64) p->NT = 64;
-    // super-iterations per CTA, measured on B200 (QDSP_DECIM_NSUP sweep): config 2: 15: 639, 19: 644, 20: 665, 22: 659,
+    // super-iterations per CTA, measured on B200: config 2: 15: 639, 19: 644, 20: 665, 22: 659,
     // 24: 665, 26: 640, 29: 636, 44: 646 GS/s; config 4 (wideband): 12: 17.7, 16: 18.4, 20: 19.4, 29: 17.4, 36: 17.9 GS/s
     p->NSUP = 20;
-    if (const char* e = getenv("QDSP_DECIM_NSUP")) p->NSUP = atoi(e) > 1 ? atoi(e) : 20;
     std::vector<float2> tab((size_t)p->nslices * 2 * p->Q * p->P, make_float2(0.f, 0.f));
     for (int sl = 0; sl < p->nslices; sl++)
         for (int pad = 0; pad < 2; pad++)
@@ -868,12 +844,12 @@ int launch_decim_finish(const float2* ypart, long long ypart_stride, int nslices
     return 0;
 }
 
-template <int Q, int DT, int NSEGT, bool ROT, bool DEMOD, bool SUPRED>
+template <int Q, bool ROT, bool DEMOD, bool SUPRED>
 static int launch_decim_t(const DecimArgs& a, dim3 grid, int NT, size_t smem, cudaStream_t s) {
     // launch bounds pick the CTAs/SM that 96 registers per thread allow (640 threads per SM)
 #define QDSP_DECIM_LAUNCH(MAXT, MINB)                                                                          \
     {                                                                                                          \
-        auto kern = decim_kernel<Q, DT, NSEGT, ROT, DEMOD, SUPRED, MAXT, MINB>;                                        \
+        auto kern = decim_kernel<Q, ROT, DEMOD, SUPRED, MAXT, MINB>;                                                  \
         QDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));     \
         kern<<<grid, NT, smem, s>>>(a);                                                                        \
     }
@@ -886,18 +862,14 @@ static int launch_decim_t(const DecimArgs& a, dim3 grid, int NT, size_t smem, cu
     return 0;
 }
 
-template <int Q, int DT, int NSEGT, bool ROT, bool DEMOD, int NSLOTT = 2, int DBG = 0>
+template <int Q, int D, int NSEG, bool ROT, bool DEMOD>
 static int launch_decim_sup_t(const DecimArgs& a, dim3 grid, cudaStream_t s) {
-    auto kern = decim_sup_kernel<Q, DT, NSEGT, ROT, DEMOD, NSLOTT, DBG>;
-    constexpr size_t smem = SupGeom<Q, DT, NSEGT, NSLOTT>::smem_bytes;
+    auto kern = decim_sup_kernel<Q, D, NSEG, ROT, DEMOD>;
+    constexpr size_t smem = SupGeom<Q, D, NSEG>::smem_bytes;
     QDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, NSLOTT == 3 ? 192 : 160, smem, s>>>(a);
+    kern<<<grid, 160, smem, s>>>(a);
     QDSP_LAUNCH_OK();
     return 0;
-}
-static bool decim_v2_enabled() {
-    static const bool on = getenv("QDSP_DECIM_V2") ? atoi(getenv("QDSP_DECIM_V2")) != 0 : true;
-    return on;
 }
 
 int launch_decim(DecimPlan* plan, const float2* hist, int H, const float2* in, const Partition& part, int mode,
@@ -940,8 +912,7 @@ int launch_decim(DecimPlan* plan, const float2* hist, int H, const float2* in, c
     // several planes (channels x column slices) read the same input: make the plane the fastest grid dimension so that
     // the CTAs resident together are the planes of the same few input tiles -- the tile is fetched from DRAM once and the
     // other planes hit L2 (config 4, 32 channels: 3.98 GB -> see DESIGN.md of DRAM reads per 134 MB of input)
-    static const bool pf_env = getenv("QDSP_DECIM_PLANE_FAST") ? atoi(getenv("QDSP_DECIM_PLANE_FAST")) != 0 : true;
-    a.plane_fast = pf_env && nch * plan->nslices > 1 && grid.x <= 65535 && grid.y <= 65535;
+    a.plane_fast = nch * plan->nslices > 1 && grid.x <= 65535 && grid.y <= 65535;
     if (a.plane_fast) grid = dim3(nch * plan->nslices, grid.x, grid.y);
     const size_t stage_bytes = (size_t)a.NSEG * (a.R * a.D + decim_seg_pad(a.D)) * sizeof(float2);
     const size_t smem_stage = (size_t)a.NSTAGE * stage_bytes + (size_t)2 * a.NSEG * a.R * (a.P | 1) * sizeof(float2) +
@@ -968,21 +939,18 @@ int launch_decim(DecimPlan* plan, const float2* hist, int H, const float2* in, c
         a.out_iq = plan->ypart;
         a.audio = nullptr;
         a.out_stride = (long long)ystride;
-        static const bool supred_s = getenv("QDSP_DECIM_SUPRED") ? atoi(getenv("QDSP_DECIM_SUPRED")) != 0 : true;
-        const bool sup = supred_s && plan->NT >= 2 * plan->NSEG * plan->Q;
+        const bool sup = plan->NT >= 2 * plan->NSEG * plan->Q;
         const size_t sm = sup ? smem_sup : smem_stage;
         int rc;
-        if (plan->Q == 9 && plan->D == 128 && plan->NSEG == 2 && sup && plan->NT == 128 && decim_v2_enabled())
+        // 128-column slices: P = 64, NSEG = 2, NT = 128, so Q = 9 always takes the super-iteration kernel (config 4)
+        if (plan->Q == 9 && plan->D == 128 && plan->NSEG == 2 && sup && plan->NT == 128)
             rc = fused ? launch_decim_sup_t<9, 128, 2, true, false>(a, grid, s) : launch_decim_sup_t<9, 128, 2, false, false>(a, grid, s);
-        else if (plan->Q == 9 && plan->D == 128 && plan->NSEG == 2 && sup)   // config 4: compile-time slice geometry
-            rc = fused ? launch_decim_t<9, 128, 2, true, false, true>(a, grid, plan->NT, sm, s)
-                       : launch_decim_t<9, 128, 2, false, false, true>(a, grid, plan->NT, sm, s);
         else if (plan->Q == 9)
-            rc = fused ? (sup ? launch_decim_t<9, 0, 0, true, false, true>(a, grid, plan->NT, sm, s) : launch_decim_t<9, 0, 0, true, false, false>(a, grid, plan->NT, sm, s))
-                       : (sup ? launch_decim_t<9, 0, 0, false, false, true>(a, grid, plan->NT, sm, s) : launch_decim_t<9, 0, 0, false, false, false>(a, grid, plan->NT, sm, s));
+            rc = fused ? (sup ? launch_decim_t<9, true, false, true>(a, grid, plan->NT, sm, s) : launch_decim_t<9, true, false, false>(a, grid, plan->NT, sm, s))
+                       : (sup ? launch_decim_t<9, false, false, true>(a, grid, plan->NT, sm, s) : launch_decim_t<9, false, false, false>(a, grid, plan->NT, sm, s));
         else
-            rc = fused ? (sup ? launch_decim_t<6, 0, 0, true, false, true>(a, grid, plan->NT, sm, s) : launch_decim_t<6, 0, 0, true, false, false>(a, grid, plan->NT, sm, s))
-                       : (sup ? launch_decim_t<6, 0, 0, false, false, true>(a, grid, plan->NT, sm, s) : launch_decim_t<6, 0, 0, false, false, false>(a, grid, plan->NT, sm, s));
+            rc = fused ? (sup ? launch_decim_t<6, true, false, true>(a, grid, plan->NT, sm, s) : launch_decim_t<6, true, false, false>(a, grid, plan->NT, sm, s))
+                       : (sup ? launch_decim_t<6, false, false, true>(a, grid, plan->NT, sm, s) : launch_decim_t<6, false, false, false>(a, grid, plan->NT, sm, s));
         if (rc != 0) return rc;
         long long gx = (part.total_out + 255) / 256;
         if (gx > 1024) gx = 1024;
@@ -993,27 +961,17 @@ int launch_decim(DecimPlan* plan, const float2* hist, int H, const float2* in, c
         QDSP_LAUNCH_OK();
         return 0;
     }
-    static const bool supred_env = getenv("QDSP_DECIM_SUPRED") ? atoi(getenv("QDSP_DECIM_SUPRED")) != 0 : true;
-    const bool supred = supred_env && plan->P <= 64 && plan->NT >= 2 * plan->NSEG * plan->Q;
+    const bool supred = plan->P <= 64 && plan->NT >= 2 * plan->NSEG * plan->Q;
     const size_t smem = supred ? smem_sup : smem_stage;
-#ifdef QDSP_DECIM_DEBUG_VARIANTS   // profiling aids: 1 = no FIR math (data movement only), 2 = no finishing pass
-    if (const char* e = getenv("QDSP_DECIM_DBG")) {
-        if (atoi(e) == 1 && fused) return launch_decim_sup_t<9, 50, 5, true, true, 2, 1>(a, grid, s);
-        if (atoi(e) == 2 && fused) return launch_decim_sup_t<9, 50, 5, true, true, 2, 2>(a, grid, s);
-        if (atoi(e) == 3 && fused) return launch_decim_sup_t<9, 50, 5, true, true, 3, 0>(a, grid, s);
-    }
-#endif
-    if (plan->Q == 9 && plan->D == 50 && plan->NSEG == 5 && supred && plan->NT == 128 && decim_v2_enabled())
+    // D = 50: P = 25, NSEG = 5, NT = 128, so Q = 9 always takes the super-iteration kernel (config 2)
+    if (plan->Q == 9 && plan->D == 50 && plan->NSEG == 5 && supred && plan->NT == 128)
         return fused ? launch_decim_sup_t<9, 50, 5, true, true>(a, grid, s) : launch_decim_sup_t<9, 50, 5, false, false>(a, grid, s);
-    if (plan->Q == 9 && plan->D == 50 && plan->NSEG == 5)
-        return fused ? (supred ? launch_decim_t<9, 50, 5, true, true, true>(a, grid, plan->NT, smem, s) : launch_decim_t<9, 50, 5, true, true, false>(a, grid, plan->NT, smem, s))
-                     : (supred ? launch_decim_t<9, 50, 5, false, false, true>(a, grid, plan->NT, smem, s) : launch_decim_t<9, 50, 5, false, false, false>(a, grid, plan->NT, smem, s));
     if (plan->Q == 9)
-        return fused ? (supred ? launch_decim_t<9, 0, 0, true, true, true>(a, grid, plan->NT, smem, s) : launch_decim_t<9, 0, 0, true, true, false>(a, grid, plan->NT, smem, s))
-                     : (supred ? launch_decim_t<9, 0, 0, false, false, true>(a, grid, plan->NT, smem, s) : launch_decim_t<9, 0, 0, false, false, false>(a, grid, plan->NT, smem, s));
+        return fused ? (supred ? launch_decim_t<9, true, true, true>(a, grid, plan->NT, smem, s) : launch_decim_t<9, true, true, false>(a, grid, plan->NT, smem, s))
+                     : (supred ? launch_decim_t<9, false, false, true>(a, grid, plan->NT, smem, s) : launch_decim_t<9, false, false, false>(a, grid, plan->NT, smem, s));
     if (plan->Q == 6)
-        return fused ? (supred ? launch_decim_t<6, 0, 0, true, true, true>(a, grid, plan->NT, smem, s) : launch_decim_t<6, 0, 0, true, true, false>(a, grid, plan->NT, smem, s))
-                     : (supred ? launch_decim_t<6, 0, 0, false, false, true>(a, grid, plan->NT, smem, s) : launch_decim_t<6, 0, 0, false, false, false>(a, grid, plan->NT, smem, s));
+        return fused ? (supred ? launch_decim_t<6, true, true, true>(a, grid, plan->NT, smem, s) : launch_decim_t<6, true, true, false>(a, grid, plan->NT, smem, s))
+                     : (supred ? launch_decim_t<6, false, false, true>(a, grid, plan->NT, smem, s) : launch_decim_t<6, false, false, false>(a, grid, plan->NT, smem, s));
     set_last_error("decim: unsupported Q=%d", plan->Q);
     return -1;
 }

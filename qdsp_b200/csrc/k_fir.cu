@@ -422,8 +422,7 @@ int launch_fir_decim(FirDecimPlan* plan, const float2* hist, int H, const float2
     VStream<float2> xs{hist, in, H};
     // short sub-filters (config 1b: 32 taps per sub-stream): 128-thread CTAs with 1152-output tiles, 4-5 per SM, overlap one
     // CTA's staging with the others' math better than 2 x 256 threads; long ones keep the big tile (less halo per output)
-    static const int nw_env = getenv("QDSP_FIR_DECIM_NW") ? atoi(getenv("QDSP_FIR_DECIM_NW")) : 0;
-    const int NW = nw_env == 4 || nw_env == 8 ? nw_env : (plan->U <= 36 ? 4 : 8);
+    const int NW = plan->U <= 36 ? 4 : 8;
     const int nout = (NW / 2) * 64 * kFirR;
     const size_t smem = (size_t)plan->D * (nout / 2 + plan->U + 8) * 16 + (size_t)plan->D * 2 * plan->U * 8;
     const long long tiles = (n_out + nout - 1) / nout;
@@ -433,9 +432,7 @@ int launch_fir_decim(FirDecimPlan* plan, const float2* hist, int H, const float2
         fir_decim_kernel<DT, NWT><<<(unsigned)tiles, NWT * 32, smem, s>>>(xs, count, n_out, plan->taps_dev, plan->T, plan->D, \
                                                                           plan->U, out);                           \
     }
-    static const bool scalar_staging = getenv("QDSP_FIR_DECIM_SCALAR") != nullptr;   // A/B switch
-    if (scalar_staging) QDSP_FIR_DECIM_LAUNCH(0, 8)
-    else if (plan->D == 2 && NW == 4) QDSP_FIR_DECIM_LAUNCH(2, 4)
+    if (plan->D == 2 && NW == 4) QDSP_FIR_DECIM_LAUNCH(2, 4)
     else if (plan->D == 2) QDSP_FIR_DECIM_LAUNCH(2, 8)
     else if (plan->D == 4 && NW == 4) QDSP_FIR_DECIM_LAUNCH(4, 4)
     else if (plan->D == 4) QDSP_FIR_DECIM_LAUNCH(4, 8)
@@ -624,21 +621,6 @@ __global__ void __launch_bounds__(256, 3) fir_longcplx_kernel(const __grid_const
 // hist_next / overlap_prev / advanced: when the constant-bank kernels take the call and `hist_next` is given, the kernel's
 // first CTA writes the advanced history tail there (*advanced = true: the caller flips its double buffer instead of
 // launching the advance kernel); overlap_prev lets the grid start while the previous call of the same handle drains
-static cudaError_t fir_launch_ex(const void* kern, dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool overlap, void* arg) {
-    static const int pdl_env = getenv("QDSP_PDL") ? atoi(getenv("QDSP_PDL")) : 1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = (overlap && pdl_env) ? 1 : 0;
-    void* args[1] = {arg};
-    return cudaLaunchKernelExC(&cfg, kern, args);
-}
 int launch_fir_dense(FirPlan* plan, const float2* hist, int H, const float2* in, long long count, int lead,
                      float2* out, cudaStream_t s, float2* hist_next, bool overlap_prev, bool* advanced) {
     if (advanced) *advanced = false;
@@ -649,9 +631,8 @@ int launch_fir_dense(FirPlan* plan, const float2* hist, int H, const float2* in,
     }
     // constant-bank kernel: instantiated for 63 / 127 / 255 taps; a filter of T taps runs as the next instantiated length TT
     // with TT - T leading zero taps (y[n] = sum_j g[j] x[n - (TT-1) + j], g[j] = h[j - (TT - T)]) when that costs < 1/3 more work
-    static const int cplx_env = getenv("QDSP_FIR_CPLX") ? atoi(getenv("QDSP_FIR_CPLX")) : 1;
     const int TT = plan->T <= 63 ? 63 : (plan->T <= 127 ? 127 : 255);
-    if (cplx_env && plan->T <= 255 && 4 * plan->T > 3 * TT && (reinterpret_cast<uintptr_t>(in) & 15) == 0) {
+    if (plan->T <= 255 && 4 * plan->T > 3 * TT && (reinterpret_cast<uintptr_t>(in) & 15) == 0) {
         constexpr int K = 4;
         static FirCplxArgs fa;
         static std::mutex mtx;
@@ -667,13 +648,12 @@ int launch_fir_dense(FirPlan* plan, const float2* hist, int H, const float2* in,
         const long long tiles = (count + K * 288 - 1) / (K * 288);
         const void* kern = TT == 63 ? (const void*)fir_cplx_kernel<63, K>
                                     : (TT == 127 ? (const void*)fir_cplx_kernel<127, K> : (const void*)fir_cplx_kernel<255, K>);
-        QDSP_CUDA_OK(fir_launch_ex(kern, dim3((unsigned)tiles), dim3(32), 0, s, overlap_prev, &fa));
+        QDSP_CUDA_OK(launch_ex(kern, dim3((unsigned)tiles), dim3(32), 0, s, overlap_prev, &fa));
         QDSP_LAUNCH_OK();
         if (advanced && hist_next) *advanced = true;
         return 0;
     }
-    static const int longcplx_env = getenv("QDSP_FIR_LONGCPLX") ? atoi(getenv("QDSP_FIR_LONGCPLX")) : 1;
-    if (longcplx_env && cplx_env && plan->T > 255 && plan->T <= 4095 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 &&
+    if (plan->T > 255 && plan->T <= 4095 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 &&
         !plan->taps_long.empty()) {
         static FirLongArgs la;
         static std::mutex mtx;
@@ -692,7 +672,7 @@ int launch_fir_dense(FirPlan* plan, const float2* hist, int H, const float2* in,
         // per device (the attribute belongs to the current context), so set on every call: it is a cheap driver lookup
         QDSP_CUDA_OK(cudaFuncSetAttribute(fir_longcplx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(((size_t)2304 + kFlMaxTp + 8) * 8)));
         const long long tiles = (count + 2304 - 1) / 2304;
-        QDSP_CUDA_OK(fir_launch_ex((const void*)fir_longcplx_kernel, dim3((unsigned)tiles), dim3(256), smem, s, overlap_prev, &la));
+        QDSP_CUDA_OK(launch_ex((const void*)fir_longcplx_kernel, dim3((unsigned)tiles), dim3(256), smem, s, overlap_prev, &la));
         QDSP_LAUNCH_OK();
         if (advanced && hist_next) *advanced = true;
         return 0;
@@ -700,8 +680,7 @@ int launch_fir_dense(FirPlan* plan, const float2* hist, int H, const float2* in,
     VStream<float2> xs{hist, in, H};
     // short filters (config 1a: 127 taps): 128-thread CTAs with 1152-output tiles, 5 per SM; long ones keep the 2304-output
     // tile (the window's T-1 halo is staged once per tile)
-    static const int nw_env = getenv("QDSP_FIR_NW") ? atoi(getenv("QDSP_FIR_NW")) : 0;
-    const int NW = nw_env == 4 || nw_env == 8 ? nw_env : (plan->U <= 144 ? 4 : 8);
+    const int NW = plan->U <= 144 ? 4 : 8;
     const int nout = (NW / 2) * 64 * kFirR;
     const size_t smem = ((size_t)nout / 2 + plan->U + 8) * 16 + (size_t)2 * plan->U * 8;
     const long long tiles = (count + nout - 1) / nout;

@@ -254,8 +254,7 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
 
 // ---- host side -------------------------------------------------------------------------------------
 bool rowlane_supported(const DecimPlan* plan) {
-    static const bool on = getenv("QDSP_DECIM_ROWLANE") ? atoi(getenv("QDSP_DECIM_ROWLANE")) != 0 : true;
-    return on && plan->nslices == 1 && plan->DS == 50 && plan->Q == 9 && plan->T + 1 > 8 * 50;
+    return plan->nslices == 1 && plan->DS == 50 && plan->Q == 9 && plan->T + 1 > 8 * 50;
 }
 
 // the tap-table alignment pad must be the same for every run() block of the batch: -1 if it is not
@@ -301,11 +300,10 @@ int launch_decim_rowlane(DecimPlan* plan, const float* taps_host, const float2* 
     a.out_stride = 0;
     ra.hist_next = hist_next;
     ra.tstamp = tstamp;
-    static const int nstep_env = getenv("QDSP_ROW_NSTEP") ? atoi(getenv("QDSP_ROW_NSTEP")) : 0;
     // B200 sweeps (GS/s), DESIGN.md 6.0. Isolated launches: 4: 811, 6: 823, 8: 824, 9: 787, 10: 802, 12: 792, 16: 808,
     // 20: 806, 24: 793, 32: 773. Consecutive calls overlapped, bench.py's 100-call burst: 8: 878, 16: 866; under the power
     // cap (2 s loop) 16 steps win instead (797 vs 775): less tile re-read, fewer instructions per sample.
-    ra.nstep = nstep_env >= 2 ? nstep_env : 8;
+    ra.nstep = 8;
     ra.pad = pad;
     for (int j = 0; j < Q * D; j++) {
         const int t = j - pad;
@@ -324,22 +322,12 @@ int launch_decim_rowlane(DecimPlan* plan, const float* taps_host, const float2* 
     if (grid.x < 1) grid.x = 1;
     // TMA ring + mbarriers, then (fused) the tile's held audio: one float per lane per step
     const size_t smem = NSTG * 32 * D * 8 + NSTG * 8 + 16 + (fused ? (size_t)ra.nstep * 32 * sizeof(float) : 0);
-    static const int pdl_env = getenv("QDSP_PDL") ? atoi(getenv("QDSP_PDL")) : 1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(32);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = (overlap_prev && fused && out_iq == nullptr && pdl_env) ? 1 : 0;
+    const bool overlap = overlap_prev && fused && out_iq == nullptr;
 #define QDSP_ROW_LAUNCH(JL, ROTV, DEMV)                                                                   \
     {                                                                                                     \
         auto kern = decim_rowlane_kernel<Q, D, JL, NSTG, ROTV, DEMV>;                                     \
         QDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        QDSP_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, ra));                                                 \
+        QDSP_CUDA_OK(launch_ex((const void*)kern, grid, dim3(32), smem, s, overlap, &ra));                \
     }
     // T <= 401: the last tap row (q = 8) has live taps in its first column pair only
     if (plan->T + 1 <= 402) {

@@ -136,9 +136,5 @@ int launch_iq_convert(int fmt, IqConv c, const void* in, float2* out, long long 
 int launch_mm(int cplx, const void* in, const Partition& part, const float* taps_dev, float omega, float gainOmega,
               float muGain, float omegaMin, float omegaMax, float* state, void* out, int* out_counts_dev,
               long long* total_dev, cudaStream_t s);
-size_t mm_spec_scratch_bytes(long long count, int chunk, int cap);
-int launch_mm_spec(int cplx, const void* in, const Partition& part, const float* taps_dev, float gainOmega, float muGain,
-                   float omegaMin, float omegaMax, float* state, void* out, int* out_counts_dev, long long* total_dev,
-                   int* rewalked_dev, int chunk, int warm, int cap, void* scratch, cudaStream_t s);
 
 }  // namespace qdsp

@@ -187,8 +187,6 @@ SIGNATURES = {
     "qdsp_mm_set_omega_rel_limit": (_i, [_vp, _f]),
     "qdsp_mm_max_out": (_ll, [_vp, _ll]),
     "qdsp_mm_process": (_ll, [_vp, _vp, _vp, _ll, _ip, _i, _i, _ip, _vp]),
-    "qdsp_mm_set_speculation": (_i, [_vp, _i, _i]),
-    "qdsp_mm_last_rewalked": (_i, [_vp]),
     "qdsp_mm_get_state": (_i, [_vp, _fp]),
     "qdsp_mm_set_state": (_i, [_vp, _fp]),
     "qdsp_sinesource_create": (_vp, [_f, _f]),

@@ -575,44 +575,6 @@ def test_psk_demod_chain(name, golden):
     assert np.median(np.abs(y[1000:])) > 0.5
 
 
-@pytest.mark.parametrize("dtype", ["cf32", "f32"])
-def test_clock_recovery_speculate_and_verify(dtype):
-    from qdsp_b200 import blocks as _B, lib as _qlib
-    from tests.runners import interp_taps as _taps
-    _probe = _B.MMClockRecovery(4.0, (0.01 * 0.01) / 4, 0.01, 0.005, _taps())
-    if _qlib.load().qdsp_mm_set_speculation(_probe.h, 4096, 1024) != 0:
-        pytest.skip("experimental MM speculate-and-verify variant not compiled in (-DQDSP_MM_SPECULATION)")
-    # chunks walked in parallel from the default loop state, accepted only where bit-equal at the boundary: symbols,
-    # per-block counts and the carried state must equal the sequential walk's whatever the speculation did -- with a
-    # warm-up long enough to merge (few or no re-walks) and with a hopeless one (every chunk re-walked)
-    from qdsp_b200 import blocks as B, synth
-    from tests.runners import interp_taps
-
-    n = 1 << 18
-    x = synth.qpsk_cf32(91, 0, n, sps=4, freq_off=0.0, sigma=0.05)
-    if dtype == "f32":
-        x = np.ascontiguousarray(x.real)
-    t = interp_taps()
-    args = (4.0, (0.01 * 0.01) / 4, 0.01, 0.005, t, x.dtype)
-    blocks = [100000, 7, 62137, n - 162144]
-    seq = B.MMClockRecovery(*args)
-    y0 = seq.process(x, blocks)
-    oc0, st0 = seq.last_out_counts.copy(), seq.get_state()
-    P = loader.port()
-    yo, oco = P.mm(x, 4.0, (0.01 * 0.01) / 4, 0.01, 0.005, t, blocks)
-    assert np.array_equal(y0.view(np.uint32), yo.view(np.uint32)) and np.array_equal(oc0, oco)
-    for chunk, warm, expect_clean in ((16384, 8192, True), (4096, 64, False)):
-        sp = B.MMClockRecovery(*args)
-        sp.set_speculation(chunk, warm)
-        y = sp.process(x, blocks)
-        assert np.array_equal(y.view(np.uint32), y0.view(np.uint32)), (chunk, warm)
-        assert np.array_equal(sp.last_out_counts, oc0)
-        assert np.array_equal(sp.get_state()[:30].view(np.uint32), st0[:30].view(np.uint32))
-        print(f"MM speculation chunk={chunk} warmup={warm}: {sp.last_rewalked()} of {n // chunk - 1} chunks re-walked")
-        if not expect_clean:
-            assert sp.last_rewalked() > 0
-
-
 def test_agc_unaligned_blocks():
     # run() blocks that start off the 16-byte grid take the scalar head / tail of the 128-bit max and scale passes
     from qdsp_b200 import blocks as B, synth
@@ -627,8 +589,8 @@ def test_agc_unaligned_blocks():
 
 
 def test_channelizer_ragged_partition_plane_fast_grid():
-    # several channels + an explicit (ragged) run() partition: the plane-fastest grid order must decode tile / block /
-    # channel the same way as the default order (QDSP_DECIM_PLANE_FAST=0 is the A/B switch of the launcher)
+    # several channels + an explicit (ragged) run() partition: the plane-fastest grid order (taken whenever several planes
+    # read the same input and the grid fits) must decode tile / block / channel the same way as the one-plane order
     from qdsp_b200 import blocks as B
 
     c = CASES["channelizer"]
@@ -867,34 +829,6 @@ def test_costas_chunked_default_warmup_ragged_streaming(order, gen):
     assert np.abs(y - yo).max() <= 1e-4, np.abs(y - yo).max()
 
 
-def test_costas_warp_staged_kernel_opt_in():
-    # QDSP_COSTAS_WARP=1 (read once per process, hence the subprocess): the warp-private cp.async walk against the
-    # sequential oracle on a ragged three-call stream, all three detectors
-    import os
-    import subprocess
-    import sys
-
-    code = r"""
-import numpy as np
-from oracle import loader
-from qdsp_b200 import blocks as B, synth
-n = 700_001
-for order, gen in [(4, synth.qpsk_cf32), (2, synth.bpsk_cf32), (8, synth.qpsk_cf32)]:
-    x = gen(35, 0, n)
-    yo, _ = loader.port().costas(order, 0.004, x)
-    pl = B.CostasLoop(order, 0.004)
-    cuts = [0, 300_003, 300_003 + 2048 * 37 + 5, n]
-    y = np.concatenate([pl.process(x[a:b]) for a, b in zip(cuts[:-1], cuts[1:])])
-    assert pl.last_residual() < 1e-4, pl.last_residual()
-    assert np.abs(y - yo).max() <= 1e-4, (order, np.abs(y - yo).max())
-print("ok")
-"""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, QDSP_COSTAS_WARP="1", PYTHONPATH=root)
-    r = subprocess.run([sys.executable, "-c", code], cwd=root, env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stdout + r.stderr
-
-
 @pytest.mark.parametrize("ntaps", [50, 63, 100, 101, 126, 127, 200, 255])
 def test_fir_constant_bank_kernel_tap_counts(ntaps):
     # fir_cplx_kernel (taps in the constant bank, instantiated for 63 / 127 / 255 taps): other lengths, even ones included,
@@ -986,44 +920,32 @@ def test_fir_back_to_back_calls_overlapped_launches(ntaps):
         b.free()
 
 
-def test_resampler_sliding_window_kernel_opt_in():
-    # QDSP_FIRROW_SLIDE=1 (read once per process, hence the subprocess): the constant-bank sliding-window decimate-by-4
-    # kernel -- faster than the row-per-lane default for calls of >= 2^26 samples -- on a ragged stream (history carried,
-    # a call shorter than the filter, a ragged last block) and on back-to-back overlapped calls, against the oracle
-    import os
-    import subprocess
-    import sys
+def test_resampler_sliding_window_kernel_long_calls():
+    # calls of >= 2^25 samples take the constant-bank sliding-window decimate-by-4 kernel (fir_slide4_kernel) instead of the
+    # row-per-lane one: two consecutive calls with the history carried (the first off the decimation grid, the second cut
+    # into run() blocks with a ragged last one), then back-to-back overlapped calls on distinct device buffers, against
+    # the oracle
+    from qdsp_b200 import blocks as B, synth
 
-    code = r"""
-import numpy as np
-from oracle import loader
-from qdsp_b200 import blocks as B, synth
-P = loader.port()
-win = B.BlackmanWindow(300e3, 4 * 2.4e6 / 127, 2.4e6)
-taps = P.blackman_taps(300e3, 4 * 2.4e6 / 127, 2.4e6)
-def rel(a, b):
-    return float(np.linalg.norm(a - b) / np.linalg.norm(b))
-n = 1_500_000
-x = synth.uniform_cf32(17, 0, n)
-cuts = [0, 400_000, 400_040, 900_000, n]
-blocks = [b - a for a, b in zip(cuts[:-1], cuts[1:])]
-yo, _ = P.resamp_cf32(taps, 1, 4, x, blocks)
-r = B.PolyphaseResampler(win, 2.4e6, 0.6e6)
-y = np.concatenate([r.process(x[a:b], b - a) for a, b in zip(cuts[:-1], cuts[1:])])
-assert y.shape == yo.shape and rel(y, yo) <= 1e-5, rel(y, yo)
-ncall, m = 8, 1 << 18
-x2 = synth.uniform_cf32(19, 0, ncall * m)
-yo2, _ = P.resamp_cf32(taps, 1, 4, x2, m)
-ins = [B.DevBuf.from_numpy(x2[i * m:(i + 1) * m]) for i in range(ncall)]
-outs = [B.DevBuf(m // 4 * 8) for _ in range(ncall)]
-r2 = B.PolyphaseResampler(win, 2.4e6, 0.6e6)
-for i in range(ncall):
-    assert r2.process_device(ins[i].ptr, outs[i].ptr, m, m) == m // 4
-y2 = np.concatenate([o.to_numpy(np.complex64, m // 4) for o in outs])
-assert rel(y2, yo2) <= 1e-5, rel(y2, yo2)
-print("ok")
-"""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, QDSP_FIRROW_SLIDE="1", PYTHONPATH=root)
-    r = subprocess.run([sys.executable, "-c", code], cwd=root, env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stdout + r.stderr
+    P = loader.port()
+    win = B.BlackmanWindow(300e3, 4 * 2.4e6 / 127, 2.4e6)
+    taps = P.blackman_taps(300e3, 4 * 2.4e6 / 127, 2.4e6)
+    n1, n2, blk = (1 << 25) + 3, (1 << 25) + 4002, 1 << 22
+    x = synth.uniform_cf32(17, 0, n1 + n2)
+    yo, _ = P.resamp_cf32(taps, 1, 4, x, [n1] + [blk] * (n2 // blk) + [n2 % blk])
+    r = B.PolyphaseResampler(win, 2.4e6, 0.6e6)
+    y = np.concatenate([r.process(x[:n1], n1), r.process(x[n1:], blk)])
+    assert y.shape == yo.shape and rel_l2(y, yo) <= 1e-5, rel_l2(y, yo)
+    del x, y, yo
+    ncall, m = 3, 1 << 25
+    x2 = synth.uniform_cf32(19, 0, ncall * m)
+    yo2, _ = P.resamp_cf32(taps, 1, 4, x2, m)
+    ins = [B.DevBuf.from_numpy(x2[i * m:(i + 1) * m]) for i in range(ncall)]
+    outs = [B.DevBuf(m // 4 * 8) for _ in range(ncall)]
+    r2 = B.PolyphaseResampler(win, 2.4e6, 0.6e6)
+    for i in range(ncall):
+        assert r2.process_device(ins[i].ptr, outs[i].ptr, m, m) == m // 4
+    y2 = np.concatenate([o.to_numpy(np.complex64, m // 4) for o in outs])
+    assert rel_l2(y2, yo2) <= 1e-5, rel_l2(y2, yo2)
+    for b in ins + outs:
+        b.free()

@@ -139,17 +139,6 @@ def main():
             ms = timed(lambda: mm.process_device(xp, yp, nm, 1000000, stream=sp), 3, warmup=1)
             print(json.dumps({"config": f"pw MMClockRecovery<complex_t> omega=4, {nm} samples (one stream, sequential-exact)", "ms": ms,
                               "Msamples_s": nm / ms / 1e3, "Msymbols_s": nm / 4 / ms / 1e3}), flush=True)
-            # speculate and verify on real QPSK (the loop has to lock for the chunks to merge), 2^24 samples
-            from qdsp_b200 import synth
-            nq = 1 << 24
-            xq = torch.from_numpy(synth.qpsk_cf32(91, 0, nq, sps=4, freq_off=0.0, sigma=0.05)).cuda()
-            for chunk, warm in (((32768, 8192),) if os.environ.get("QDSP_BENCH_MM_SPEC") else ()):   # needs -DQDSP_MM_SPECULATION
-                mm2 = B.MMClockRecovery(4.0, (0.01 * 0.01) / 4, 0.01, 0.005, taps)
-                mm2.set_speculation(chunk, warm)
-                ms = timed(lambda: mm2.process_device(xq.data_ptr(), yp, nq, 1000000, stream=sp), 3, warmup=1)
-                print(json.dumps({"config": f"pw MMClockRecovery<complex_t> speculate-and-verify chunk={chunk} warmup={warm}, {nq} QPSK samples",
-                                  "ms": ms, "Msamples_s": nq / ms / 1e3, "Msymbols_s": nq / 4 / ms / 1e3,
-                                  "rewalked_chunks": mm2.last_rewalked(), "chunks": nq // chunk}), flush=True)
         except Exception as e:  # noqa: BLE001
             print(json.dumps({"config": "pw MMClockRecovery", "error": str(e)}), flush=True)
         for name, bytes_per, fn in rows:

@@ -2,10 +2,10 @@
 CUDA event pair around the whole loop, with the per-launch timing ring (qdsp_vfofm_enable_timing_ring, what bench.py turns
 on for its headline region) off and on, and overlapped launches allowed (QDSP_PDL=1) or not (QDSP_PDL=0).
 
-    python tools/vfofm_calls.py [--trees . OTHER_TREE] [--pdl 1 0] [--nstep 8] [--steps 200] [--loops 4] [--reps 2]
+    python tools/vfofm_calls.py [--trees . OTHER_TREE] [--pdl 1 0] [--steps 200] [--loops 4] [--reps 2]
 
-Each (tree, QDSP_PDL, QDSP_ROW_NSTEP) runs in a subprocess of its own (the library reads both variables once); the
-combinations are alternated `--reps` times, and inside a subprocess ring-off and ring-on loops alternate `--loops` times.
+Each (tree, QDSP_PDL) runs in a subprocess of its own (the library reads the variable once); the combinations are
+alternated `--reps` times, and inside a subprocess ring-off and ring-on loops alternate `--loops` times.
 Every call reads the same input and writes the same audio buffer, as bench.py's timed steps do. One JSON line per loop,
 then one summary line per arm (median GS/s). `audio_crc` is the CRC-32 of the last call's audio bytes: equal values mean
 bit-identical audio across arms and trees."""
@@ -62,7 +62,7 @@ def child(a):
             e1.record()
             torch.cuda.synchronize()
             ms = e0.elapsed_time(e1)
-            rec = {"tree": a.tree, "pdl": os.environ.get("QDSP_PDL", "1"), "nstep": os.environ.get("QDSP_ROW_NSTEP", "default"),
+            rec = {"tree": a.tree, "pdl": os.environ.get("QDSP_PDL", "1"),
                    "ring": ring, "loop": loop, "steps": a.steps, "ms": round(ms, 4),
                    "us_per_call": round(ms * 1e3 / a.steps, 2), "GS_per_s": round(n * a.steps / ms / 1e6, 1)}
             if ring:
@@ -72,7 +72,7 @@ def child(a):
             print(json.dumps(rec), flush=True)
     L.qdsp_vfofm_enable_timing(chain.h, 0)
     crc = zlib.crc32(audio[:n_out].cpu().numpy().tobytes())
-    print(json.dumps({"tree": a.tree, "pdl": os.environ.get("QDSP_PDL", "1"), "nstep": os.environ.get("QDSP_ROW_NSTEP", "default"),
+    print(json.dumps({"tree": a.tree, "pdl": os.environ.get("QDSP_PDL", "1"),
                       "calls": a.warmup + 2 * a.loops * a.steps, "audio_crc": f"{crc:08x}"}), flush=True)
 
 
@@ -80,7 +80,6 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--trees", nargs="+", default=["."], help="repository trees whose built library to time (alternated)")
     ap.add_argument("--pdl", nargs="+", default=["1", "0"], help="QDSP_PDL values")
-    ap.add_argument("--nstep", nargs="+", default=[None], help="QDSP_ROW_NSTEP values (default: the library's)")
     ap.add_argument("--steps", type=int, default=200, help="calls per timed loop")
     ap.add_argument("--loops", type=int, default=4, help="ring-off / ring-on loop pairs per subprocess")
     ap.add_argument("--reps", type=int, default=2, help="subprocesses per arm, alternated")
@@ -96,25 +95,20 @@ def main():
     for _ in range(a.reps):
         for tree in a.trees:
             for pdl in a.pdl:
-                for nstep in a.nstep:
-                    env = dict(os.environ, QDSP_PDL=str(pdl))
-                    if nstep is not None:
-                        env["QDSP_ROW_NSTEP"] = str(nstep)
-                    else:
-                        env.pop("QDSP_ROW_NSTEP", None)
-                    cmd = [sys.executable, os.path.abspath(__file__), "--child", "--tree", tree, "--steps", str(a.steps),
-                           "--loops", str(a.loops), "--warmup", str(a.warmup), "--samples", str(a.samples)]
-                    out = subprocess.run(cmd, env=env, cwd=REPO, check=True, capture_output=True, text=True).stdout
-                    for line in out.splitlines():
-                        print(line, flush=True)
-                        rows.append(json.loads(line))
+                env = dict(os.environ, QDSP_PDL=str(pdl))
+                cmd = [sys.executable, os.path.abspath(__file__), "--child", "--tree", tree, "--steps", str(a.steps),
+                       "--loops", str(a.loops), "--warmup", str(a.warmup), "--samples", str(a.samples)]
+                out = subprocess.run(cmd, env=env, cwd=REPO, check=True, capture_output=True, text=True).stdout
+                for line in out.splitlines():
+                    print(line, flush=True)
+                    rows.append(json.loads(line))
     arms = {}
     for r in rows:
         if "ring" in r:
-            arms.setdefault((r["tree"], r["pdl"], r["nstep"], r["ring"]), []).append(r)
-    for (tree, pdl, nstep, ring), rs in arms.items():
+            arms.setdefault((r["tree"], r["pdl"], r["ring"]), []).append(r)
+    for (tree, pdl, ring), rs in arms.items():
         g = [r["GS_per_s"] for r in rs]
-        s = {"summary": True, "tree": tree, "pdl": pdl, "nstep": nstep, "ring": ring, "loops": len(g),
+        s = {"summary": True, "tree": tree, "pdl": pdl, "ring": ring, "loops": len(g),
              "GS_per_s_median": statistics.median(g), "GS_per_s_min": min(g), "GS_per_s_max": max(g)}
         if ring:
             s["ring_us_mean_median"] = statistics.median(r["ring_us_mean"] for r in rs)

@@ -240,6 +240,21 @@ int qdsp_channelizer_set_variant(qdsp_channelizer* h, int variant);
  * the outputs those produce (bench.py config 4 at N > 1). Extension: the reference's state is implicit in its run() order. */
 int qdsp_channelizer_seek(qdsp_channelizer* h, long long start);
 
+/* ---- power spectrum: Welch-averaged FFT rows of a cf32 stream (an addition: the reference computes no spectrum) ---- *
+ * Frame f covers stream samples [f hop, f hop + N) (sample 0 = the first after create or reset; samples in a gap between *
+ * frames are never read); P_f[k] = |sum_n w[n] x[f hop + n] e^{-2 pi i k n / N}|^2. Row r is the mean of P over frames   *
+ * r A .. r A + A - 1, FFT-shifted (out[j] = mean P[(j + N / 2) mod N]: bin 0 of a row is -fs / 2), linear power, float32. *
+ * A row is a pure function of the stream: any split into calls gives the same bits. N a power of two in [64, 16384],     *
+ * window N floats (NULL = rectangular), hop >= 1, average >= 1; create returns NULL on anything else. process writes the  *
+ * rows it completes contiguously (N floats each) and returns their number, -1 for a negative count or in_dev not 8-byte  *
+ * aligned; samples of rows not yet complete stay in the handle. out_rows: rows the next call of `count` samples returns.*/
+typedef struct qdsp_spectrum qdsp_spectrum;
+qdsp_spectrum* qdsp_spectrum_create(int fftSize, const float* window, int hop, int average);
+void qdsp_spectrum_destroy(qdsp_spectrum* h);
+long long qdsp_spectrum_out_rows(qdsp_spectrum* h, long long count);
+long long qdsp_spectrum_process(qdsp_spectrum* h, const void* in_dev, float* rows_out_dev, long long count, qdsp_stream_t s);
+int qdsp_spectrum_reset(qdsp_spectrum* h);
+
 /* ---- recurrent blocks (chunked block-parallel scans) ----------------------------------------- */
 /* BFMDeemp::run, src/dsp/filter.h:129-158 (stereo_t in/out, state lastOutL/R) */
 typedef struct qdsp_deemp qdsp_deemp;

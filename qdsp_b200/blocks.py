@@ -701,6 +701,48 @@ class IQConverter(_Block):
         return dout.to_numpy(np.complex64, m)
 
 
+class Spectrum(_Block):
+    """Welch power spectrum of a complex64 stream (qdsp_spectrum_*; an addition, the reference has none). Row r is the
+    mean of |FFT(window * frame)|^2 over frames r*average .. r*average + average - 1, frame f = samples
+    [f*hop, f*hop + fftSize), FFT-shifted (column 0 is -fs/2), linear float32 power. hop defaults to fftSize, window to
+    rectangular. Rows are a pure function of the stream: samples of rows not yet complete stay in the handle."""
+
+    _destroy = "qdsp_spectrum_destroy"
+    out_dtype = np.float32
+
+    def __init__(self, fftSize, window=None, hop=None, average=1):
+        super().__init__()
+        _lib.require_device()
+        self.fftSize = int(fftSize)
+        self.hop = self.fftSize if hop is None else int(hop)
+        self.average = int(average)
+        w = None
+        if window is not None:
+            w = np.ascontiguousarray(window, np.float32)
+            if w.shape != (self.fftSize,):
+                raise ValueError(f"window must hold fftSize = {self.fftSize} values")
+        self.h = check(_L().qdsp_spectrum_create(self.fftSize, None if w is None else _fptr(w), self.hop, self.average),
+                       "qdsp_spectrum_create")
+
+    def out_rows(self, n) -> int:
+        """Rows the next call of n samples completes (host arithmetic)."""
+        return int(check(_L().qdsp_spectrum_out_rows(self.h, int(n)), "qdsp_spectrum_out_rows"))
+
+    def process_device(self, in_ptr, out_ptr, n, stream=None) -> int:
+        """in_ptr: n complex64 samples (8-byte aligned); out_ptr: room for out_rows(n) rows of fftSize floats."""
+        return int(check(_L().qdsp_spectrum_process(self.h, in_ptr, out_ptr, int(n), stream), "qdsp_spectrum_process"))
+
+    def process(self, x) -> np.ndarray:
+        x = np.ascontiguousarray(x, np.complex64)
+        rows = self.out_rows(len(x))
+        din, dout = DevBuf.from_numpy(x), DevBuf(max(rows, 1) * self.fftSize * 4)
+        m = self.process_device(din.ptr, dout.ptr, len(x))
+        return dout.to_numpy(np.float32, m * self.fftSize).reshape(m, self.fftSize)
+
+    def reset(self):
+        check(_L().qdsp_spectrum_reset(self.h), "qdsp_spectrum_reset")
+
+
 # ---------------------------------------------------------------------------------------------
 # recurrent blocks (reference filter.h BFMDeemp, processing.h AGCs, pll.h CostasLoop)
 # ---------------------------------------------------------------------------------------------

@@ -1053,6 +1053,61 @@ int qdsp_channelizer_seek(qdsp_channelizer* h, long long start) {
 }  // extern "C"
 
 // =================================================================================================
+// power spectrum (an addition: the reference has none)
+// =================================================================================================
+struct qdsp_spectrum {
+    SpectrumPlan* plan = nullptr;
+};
+
+extern "C" {
+
+qdsp_spectrum* qdsp_spectrum_create(int fftSize, const float* window, int hop, int average) {
+    if (fftSize < 64 || fftSize > 16384 || (fftSize & (fftSize - 1)) != 0 || hop < 1 || average < 1) {
+        set_last_error("spectrum_create: fftSize must be a power of two in [64, 16384], hop >= 1, average >= 1 (got %d, %d, %d)",
+                       fftSize, hop, average);
+        return nullptr;
+    }
+    if (window)
+        for (int i = 0; i < fftSize; i++)
+            if (!isfinite(window[i])) {
+                set_last_error("spectrum_create: window[%d] is not finite", i);
+                return nullptr;
+            }
+    qdsp_spectrum* h = new (std::nothrow) qdsp_spectrum();
+    if (!h) return nullptr;
+    h->plan = spectrum_plan_create(fftSize, window, hop, average);
+    if (!h->plan) {
+        delete h;
+        return nullptr;
+    }
+    return h;
+}
+void qdsp_spectrum_destroy(qdsp_spectrum* h) {
+    if (!h) return;
+    spectrum_plan_destroy(h->plan);
+    delete h;
+}
+long long qdsp_spectrum_out_rows(qdsp_spectrum* h, long long count) { return spectrum_out_rows(h->plan, count); }
+long long qdsp_spectrum_process(qdsp_spectrum* h, const void* in_dev, float* rows_out_dev, long long count, qdsp_stream_t s) {
+    if (count < 0 || (reinterpret_cast<uintptr_t>(in_dev) & 7) != 0) {
+        set_last_error("spectrum_process: negative count or input not aligned to 8 bytes");
+        return -1;
+    }
+    if (count == 0) return 0;
+    if (!in_dev || (!rows_out_dev && spectrum_out_rows(h->plan, count) > 0)) {
+        set_last_error("spectrum_process: NULL input or output");
+        return -1;
+    }
+    return launch_spectrum(h->plan, (const float2*)in_dev, rows_out_dev, count, as_stream(s));
+}
+int qdsp_spectrum_reset(qdsp_spectrum* h) {
+    spectrum_plan_reset(h->plan);
+    return 0;
+}
+
+}  // extern "C"
+
+// =================================================================================================
 // recurrent blocks
 // =================================================================================================
 struct qdsp_deemp {

@@ -27,6 +27,7 @@
 #include <new>
 #include <vector>
 #include "decim_common.cuh"
+#include "fft_common.cuh"
 
 namespace qdsp {
 
@@ -242,36 +243,6 @@ struct ChanFftBArgs {
     float inv_speed;                // 1 / phasorSpeed (demodulator.h:91)
 };
 
-// a * e^{-j 2 pi P / 16}, P a compile-time constant after unrolling
-__device__ __forceinline__ float2 mul_w16(float2 a, int P) {
-    constexpr float C1 = 0.9238795325112867f, S1 = 0.3826834323650898f, H = 0.7071067811865476f;
-    switch (P) {
-        case 0: return a;
-        case 1: return make_float2(fmaf(a.x, C1, a.y * S1), fmaf(a.y, C1, -a.x * S1));
-        case 2: return make_float2(H * (a.x + a.y), H * (a.y - a.x));
-        case 3: return make_float2(fmaf(a.x, S1, a.y * C1), fmaf(a.y, S1, -a.x * C1));
-        case 4: return make_float2(a.y, -a.x);
-        case 5: return make_float2(fmaf(a.y, C1, -a.x * S1), -fmaf(a.y, S1, a.x * C1));
-        case 6: return make_float2(H * (a.y - a.x), -H * (a.x + a.y));
-        default: return make_float2(fmaf(a.y, S1, -a.x * C1), -fmaf(a.y, C1, a.x * S1));
-    }
-}
-__host__ __device__ constexpr int bitrev4(int i) { return ((i & 1) << 3) | ((i & 2) << 1) | ((i & 4) >> 1) | ((i & 8) >> 3); }
-// 16-point forward DFT in registers (radix-2 decimation in frequency); X[k] is left in a[bitrev4(k)]
-__device__ __forceinline__ void fft16(float2 (&a)[16]) {
-#pragma unroll
-    for (int half = 8; half >= 1; half >>= 1) {
-#pragma unroll
-        for (int i = 0; i < 16; i++) {
-            if ((i & half) == 0) {
-                const int j = i + half;
-                const float2 t = make_float2(a[i].x - a[j].x, a[i].y - a[j].y);
-                a[i] = make_float2(a[i].x + a[j].x, a[i].y + a[j].y);
-                a[j] = mul_w16(t, (i & (half - 1)) * (8 / half));
-            }
-        }
-    }
-}
 // The reference's fast_arctan2 (demodulator.h:11-30) with the quotient from the reciprocal unit (<= 2 ulp: 2e-7 rad) and a
 // multiply by 1 / phasorSpeed in the FM step: this path's outputs are not bit-images of the reference's anyway (the FFT
 // reorders every sum), its budget is the 1e-4 audio tolerance.

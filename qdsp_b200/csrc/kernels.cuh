@@ -77,6 +77,15 @@ int launch_chanfft(ChanFftPlan* plan, const float2* hist, int H, const float2* i
                    uint64_t beta_ph0, long long abs0, float phasor_speed, const float* demod_in, float* demod_out, float* audio,
                    long long out_stride, cudaStream_t s);
 
+// ---- k_spectrum.cu: Welch power spectrum (windowed N-point FFT frames, |X|^2 averaged per row, FFT-shifted) --------------
+struct SpectrumPlan;
+SpectrumPlan* spectrum_plan_create(int N, const float* window, int hop, int average);   // parameters checked by the caller
+void spectrum_plan_destroy(SpectrumPlan* p);
+void spectrum_plan_reset(SpectrumPlan* p);
+long long spectrum_out_rows(const SpectrumPlan* p, long long count);
+// `in` 8-byte aligned; returns the rows written to rows_out ([rows][N]) or -1
+long long launch_spectrum(SpectrumPlan* p, const float2* in, float* rows_out, long long count, cudaStream_t s);
+
 // ---- k_fir.cu: register-blocked dense FIR (cf32, D = 1) -----------------------------------------
 struct FirPlan;
 FirPlan* fir_plan_create(const float* taps, int T);

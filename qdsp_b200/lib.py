@@ -127,6 +127,11 @@ SIGNATURES = {
     "qdsp_channelizer_set_variant": (_i, [_vp, _i]),
     "qdsp_channelizer_set_input_format": (_i, [_vp, _i, _f, _f]),
     "qdsp_channelizer_seek": (_i, [_vp, _ll]),
+    "qdsp_spectrum_create": (_vp, [_i, _fp, _i, _i]),
+    "qdsp_spectrum_destroy": (None, [_vp]),
+    "qdsp_spectrum_out_rows": (_ll, [_vp, _ll]),
+    "qdsp_spectrum_process": (_ll, [_vp, _vp, _vp, _ll, _vp]),
+    "qdsp_spectrum_reset": (_i, [_vp]),
     "qdsp_deemp_create": (_vp, [_f, _f]),
     "qdsp_deemp_destroy": (None, [_vp]),
     "qdsp_deemp_process": (_ll, [_vp, _vp, _vp, _ll, _vp]),

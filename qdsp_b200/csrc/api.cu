@@ -109,6 +109,32 @@ bool iq_format_ok(int fmt, float scale, float offset, const char* who) {
     return true;
 }
 
+bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
+    const char *pa = (const char*)a, *pb = (const char*)b;
+    return pa < pb + nb && pb < pa + na;
+}
+
+// Overlapped consecutive calls (DESIGN.md §6.0f): a handle whose kernel folds the history advance into itself keeps the
+// record of its last such call here. When the very next library launch is that handle's next call on the same stream,
+// the handle's own rule on the buffers decides whether the two grids may overlap (programmatic dependent launch).
+struct CallChain {
+    long long serial = -1;      // g_launches right after the recorded launch; -1: nothing to follow
+    cudaStream_t stream = nullptr;
+    const void *in = nullptr, *out = nullptr;
+    size_t in_bytes = 0, out_bytes = 0;
+
+    void clear() { serial = -1; }
+    bool follows(cudaStream_t s) const { return serial == g_launches.load() && stream == s; }
+    void record(cudaStream_t s, const void* in_, size_t in_bytes_, const void* out_, size_t out_bytes_) {
+        serial = g_launches.load();
+        stream = s;
+        in = in_;
+        in_bytes = in_bytes_;
+        out = out_;
+        out_bytes = out_bytes_;
+    }
+};
+
 }  // namespace
 
 extern "C" long long qdsp_iq_convert_process(int fmt, float scale, float offset, const void* in_dev, void* out_dev,
@@ -135,13 +161,8 @@ struct qdsp_fir {
     FirPlan* plan = nullptr;
     int variant = 0;
     std::vector<float> taps;
-    // the last single-kernel call (constant-bank kernels with the history advance folded in), see qdsp_resamp
-    long long last_serial = -1;
-    cudaStream_t last_stream = nullptr;
-    const char *last_in = nullptr, *last_out = nullptr;
-    size_t last_bytes = 0;
+    CallChain chain;            // the last call on the constant-bank kernels (history advance folded in)
 };
-static bool fir_ranges_overlap(const char* a, size_t na, const char* b, size_t nb) { return a < b + nb && b < a + na; }
 
 extern "C" {
 
@@ -167,7 +188,7 @@ void qdsp_fir_destroy(qdsp_fir* h) {
     delete h;
 }
 int qdsp_fir_set_taps(qdsp_fir* h, const float* taps, int tapCount) {
-    h->last_serial = -1;
+    h->chain.clear();
     h->taps.assign(taps, taps + tapCount);
     if (upload_floats(&h->taps_dev, h->taps) != 0) return -1;
     if (tapCount != h->T) {
@@ -185,26 +206,21 @@ long long qdsp_fir_process(qdsp_fir* h, const void* in_dev, void* out_dev, long 
     if (count == 0) return 0;
     const bool dense = h->plan && h->variant != 1;
     if (dense) {
-        const char *ib = (const char*)in_dev, *ob = (const char*)out_dev;
         const size_t bytes = (size_t)count * 8;
-        const bool overlap_prev = h->last_serial == g_launches.load() && h->last_stream == s &&
-                                  !fir_ranges_overlap(ib, bytes, h->last_out, h->last_bytes) &&
-                                  !fir_ranges_overlap(ob, bytes, h->last_in, h->last_bytes) &&
-                                  !fir_ranges_overlap(ob, bytes, h->last_out, h->last_bytes);
+        const CallChain& prev = h->chain;
+        const bool overlap_prev = prev.follows(s) && !ranges_overlap(in_dev, bytes, prev.out, prev.out_bytes) &&
+                                  !ranges_overlap(out_dev, bytes, prev.in, prev.in_bytes) &&
+                                  !ranges_overlap(out_dev, bytes, prev.out, prev.out_bytes);
         bool advanced = false;
         if (launch_fir_dense(h->plan, (const float2*)h->hist.ptr(), h->hist.H, (const float2*)in_dev, count, 1,
                              (float2*)out_dev, s, (float2*)h->hist.buf[h->hist.cur ^ 1], overlap_prev, &advanced) != 0)
             return -1;
         if (advanced) {              // the kernel's first CTA advanced the history tail: one launch per call
             h->hist.cur ^= 1;
-            h->last_serial = g_launches.load();
-            h->last_stream = s;
-            h->last_in = ib;
-            h->last_out = ob;
-            h->last_bytes = bytes;
+            h->chain.record(s, in_dev, bytes, out_dev, bytes);
             return count;
         }
-        h->last_serial = -1;
+        h->chain.clear();
     } else {
         // FIR == polyphase bank with I = D = 1 read one sample later (filter.h:65 reads &buffer[i+1]);
         // y[i] = sum_j taps[j] * x[i - (T-1) + j]; the generic kernel's TPP-deep window with lead=1.
@@ -254,7 +270,7 @@ int qdsp_fir_get_history(qdsp_fir* h, void* hist_host) {
     return 0;
 }
 int qdsp_fir_set_history(qdsp_fir* h, const void* hist_host) {
-    h->last_serial = -1;
+    h->chain.clear();
     QDSP_CUDA_OK(cudaDeviceSynchronize());
     if (h->hist.H > 0)
         QDSP_CUDA_OK(cudaMemcpy(h->hist.buf[h->hist.cur], hist_host, (size_t)h->hist.H * h->hist.elem,
@@ -262,11 +278,11 @@ int qdsp_fir_set_history(qdsp_fir* h, const void* hist_host) {
     return 0;
 }
 int qdsp_fir_import_tail(qdsp_fir* h, const void* tail_dev, int src_device, qdsp_stream_t s) {
-    h->last_serial = -1;
+    h->chain.clear();
     return import_tail_impl(h->hist, tail_dev, src_device, as_stream(s));
 }
 int qdsp_fir_reset(qdsp_fir* h) {
-    h->last_serial = -1;
+    h->chain.clear();
     return h->hist.reset(nullptr);
 }
 int qdsp_fir_set_variant(qdsp_fir* h, int variant) {
@@ -289,16 +305,8 @@ struct qdsp_resamp {
     FirDecimPlan* fplan = nullptr;   // small decimation (2..8): dense polyphase kernel
     int variant = 0;
     std::vector<float> taps;         // host copy (kernels that take their taps as launch parameters)
-    // the last single-kernel call (launch_firrow): when the very next library launch is this handle's next call on the same
-    // stream and its buffers do not touch that call's, the two grids may overlap (programmatic dependent launch)
-    long long last_serial = -1;
-    cudaStream_t last_stream = nullptr;
-    const char *last_in = nullptr, *last_out = nullptr;
-    size_t last_in_bytes = 0, last_out_bytes = 0;
+    CallChain chain;                 // the last launch_firrow call (history advance folded in)
 };
-static bool byte_ranges_overlap(const char* a, size_t na, const char* b, size_t nb) {
-    return a < b + nb && b < a + na;
-}
 
 extern "C" {
 
@@ -327,7 +335,7 @@ void qdsp_resamp_destroy(qdsp_resamp* h) {
     delete h;
 }
 int qdsp_resamp_set_taps(qdsp_resamp* h, const float* taps, int tapCount) {
-    h->last_serial = -1;      // state changed from the host: the next call does not overlap its predecessor
+    h->chain.clear();      // state changed from the host: the next call does not overlap its predecessor
     int tpp = 0;
     std::vector<float> ph = build_phases(taps, tapCount, h->interp, &tpp);
     if (upload_floats(&h->phases_dev, ph) != 0) return -1;
@@ -379,22 +387,15 @@ long long qdsp_resamp_process(qdsp_resamp* h, const void* in_dev, void* out_dev,
     if (regular && h->variant != 2 && h->part.total_out > 0 && firrow_supported(h->T, h->decim) &&
         (reinterpret_cast<uintptr_t>(in_dev) & 15) == 0) {
         // config 1b's geometry: row-per-lane kernel (TMA-fed, taps as uniform-register operands)
-        const char* ib = (const char*)in_dev;
-        const char* ob = (const char*)out_dev;
         const size_t ibytes = (size_t)count * 8, obytes = (size_t)h->part.total_out * 8;
-        const bool overlap_prev = h->last_serial == g_launches.load() && h->last_stream == s &&
-                                  !byte_ranges_overlap(ib, ibytes, h->last_out, h->last_out_bytes) &&
-                                  !byte_ranges_overlap(ob, obytes, h->last_in, h->last_in_bytes) &&
-                                  !byte_ranges_overlap(ob, obytes, h->last_out, h->last_out_bytes);
+        const CallChain& prev = h->chain;
+        const bool overlap_prev = prev.follows(s) && !ranges_overlap(in_dev, ibytes, prev.out, prev.out_bytes) &&
+                                  !ranges_overlap(out_dev, obytes, prev.in, prev.in_bytes) &&
+                                  !ranges_overlap(out_dev, obytes, prev.out, prev.out_bytes);
         rc = launch_firrow(h->taps.data(), h->T, h->decim, (const float2*)h->hist.ptr(), (float2*)h->hist.buf[h->hist.cur ^ 1],
                            h->hist.H, (const float2*)in_dev, count, h->part.total_out, (float2*)out_dev, s, overlap_prev);
         if (rc != 0) return -1;
-        h->last_serial = g_launches.load();
-        h->last_stream = s;
-        h->last_in = ib;
-        h->last_in_bytes = ibytes;
-        h->last_out = ob;
-        h->last_out_bytes = obytes;
+        h->chain.record(s, in_dev, ibytes, out_dev, obytes);
         h->hist.cur ^= 1;            // the kernel's first CTA advanced the history tail
         return h->part.total_out;
     } else if (regular) {
@@ -428,14 +429,14 @@ int qdsp_resamp_get_history(qdsp_resamp* h, void* hist_host) {
     return 0;
 }
 int qdsp_resamp_set_history(qdsp_resamp* h, const void* hist_host) {
-    h->last_serial = -1;
+    h->chain.clear();
     QDSP_CUDA_OK(cudaDeviceSynchronize());
     QDSP_CUDA_OK(cudaMemcpy(h->hist.buf[h->hist.cur], hist_host, (size_t)h->hist.H * h->hist.elem,
                             cudaMemcpyHostToDevice));
     return 0;
 }
 int qdsp_resamp_reset(qdsp_resamp* h) {
-    h->last_serial = -1;
+    h->chain.clear();
     return h->hist.reset(nullptr);
 }
 int qdsp_resamp_set_variant(qdsp_resamp* h, int variant) {
@@ -592,12 +593,8 @@ struct qdsp_channelizer {
     unsigned long long* ring = nullptr;                     // [2 * ring_pairs]: first CTA start, last CTA end (ns)
     int ring_pairs = 0;
     long long ring_launches = 0;
-    // the last row-per-lane call (see qdsp_resamp): when the very next library launch is this handle's next call on the same
-    // stream, the two grids may overlap; the kernel orders the carried state and its audio stores itself (k_rowlane.cu)
-    long long last_serial = -1;
-    cudaStream_t last_stream = nullptr;
-    const char* last_out = nullptr;
-    size_t last_out_bytes = 0;
+    // the last row-per-lane call without IQ output; the kernel orders the carried state and its audio stores (k_rowlane.cu)
+    CallChain chain;
     // element type of the input (set_input_format): integer input is converted to cf32 in `conv` (grown to the largest
     // call, so the hot path stays allocation-free) and the kernels read that
     int in_fmt = QDSP_CF32;
@@ -606,14 +603,14 @@ struct qdsp_channelizer {
 
     int set_input_format(int fmt, float scale, float offset, const char* who) {
         if (fmt != QDSP_CF32 && !iq_format_ok(fmt, scale, offset, who)) return -1;
-        last_serial = -1;
+        chain.clear();
         in_fmt = fmt;
         in_conv = fmt == QDSP_CF32 ? IqConv{1.0f, 0.0f} : IqConv{scale, offset};
         return 0;
     }
 
     int upload_nco() {
-        last_serial = -1;
+        chain.clear();
         std::vector<NcoDev> v(nch);
         for (int c = 0; c < nch; c++) v[c] = NcoDev{nco[c].phase, nco[c].step};
         if (!nco_dev) QDSP_CUDA_OK(cudaMalloc(&nco_dev, sizeof(NcoDev) * nch));
@@ -691,21 +688,15 @@ struct qdsp_channelizer {
             const NcoDev nh{nco[0].phase, nco[0].step};
             // overlap needs: no block-table upload between the launches (uniform partition), no IQ output (stored
             // without the wait), and no read of the previous call's audio (the input is staged before the wait)
-            const bool overlap_prev = last_serial == g_launches.load() && last_stream == s && !iq &&
-                                      part.view.table == nullptr &&
-                                      !byte_ranges_overlap((const char*)in_dev, (size_t)count * 8, last_out, last_out_bytes);
+            const bool overlap_prev = chain.follows(s) && !iq && part.view.table == nullptr &&
+                                      !ranges_overlap(in_dev, (size_t)count * 8, chain.out, chain.out_bytes);
             unsigned long long* tslot = ring && ring_launches < ring_pairs ? ring + 2 * ring_launches : nullptr;
             rc = launch_decim_rowlane(plan, taps.data(), (const float2*)hist.ptr(), (float2*)hist.buf[hist.cur ^ 1], hist.H,
                                       (const float2*)in_dev, part, 1, nco_dev, &nh, abs_pos, phasor_speed, din, dout,
                                       (float2*)iq, audio, rpad, s, overlap_prev, tslot);
             if (ring && rc == 0) ring_launches++;
             hist_folded = rc == 0;
-            if (hist_folded && !iq) {
-                last_serial = g_launches.load();
-                last_stream = s;
-                last_out = (const char*)audio;
-                last_out_bytes = (size_t)part.total_out * 4;
-            }
+            if (hist_folded && !iq) chain.record(s, in_dev, (size_t)count * 8, audio, (size_t)part.total_out * 4);
         } else if (plan && variant != 1 && chan_supported(plan) && (reinterpret_cast<uintptr_t>(in_dev) & 15) == 0 &&
                    part.max_out > 0 && (rpad = rowlane_uniform_pad(part, T)) >= 0) {
             // wide rows: channel-per-lane kernel (32 channels share every staged sample), one launch per column slice
@@ -718,7 +709,7 @@ struct qdsp_channelizer {
             rc = launch_generic_vfofm((const float2*)hist.ptr(), hist.H, (const float2*)in_dev, phases_dev, tpp, part,
                                       nco_dev, abs_pos, nch, phasor_speed, din, dout, audio, (float2*)iq, out_stride,
                                       s);
-        if (!hist_folded || iq) last_serial = -1;
+        if (!hist_folded || iq) chain.clear();
         if (rc != 0) return -1;
         if (events) QDSP_CUDA_OK(cudaEventRecord(ev_k1, s));
         if (part.total_out > 0) cur ^= 1;
@@ -838,7 +829,7 @@ long long qdsp_vfofm_process_host(qdsp_vfofm* h, const void* in_host, float* aud
         QDSP_CUDA_OK(cudaStreamWaitEvent(s, ev_h2d[slot], 0));
         const long long m = c.process(c.stage_in[slot], c.stage_out[slot], nullptr, 0, n, nullptr, 0, block_size, nullptr, s);
         if (m < 0) return -1;
-        c.last_serial = -1;   // copies and event waits go between the chunks' kernels: never overlapped
+        c.chain.clear();   // copies and event waits go between the chunks' kernels: never overlapped
         if (m > 0)
             QDSP_CUDA_OK(cudaMemcpyAsync(audio_out_host + produced, c.stage_out[slot], (size_t)m * sizeof(float),
                                          cudaMemcpyDeviceToHost, s));
@@ -925,7 +916,7 @@ long long qdsp_vfofm_process_replay(qdsp_vfofm* h, const void* in_dev, float* au
 }
 int qdsp_vfofm_reset(qdsp_vfofm* h) {
     qdsp_channelizer& c = h->c;
-    c.last_serial = -1;
+    c.chain.clear();
     QDSP_CUDA_OK(cudaDeviceSynchronize());
     if (c.hist.reset(nullptr) != 0) return -1;
     std::vector<float> z(2 * c.nch, 0.0f);
@@ -938,17 +929,17 @@ int qdsp_vfofm_set_input_format(qdsp_vfofm* h, int fmt, float scale, float offse
     return h->c.set_input_format(fmt, scale, offset, "vfofm_set_input_format");
 }
 int qdsp_vfofm_set_variant(qdsp_vfofm* h, int variant) {
-    h->c.last_serial = -1;
+    h->c.chain.clear();
     h->c.variant = variant;
     return 0;
 }
 int qdsp_vfofm_seek(qdsp_vfofm* h, long long start) {
-    h->c.last_serial = -1;
+    h->c.chain.clear();
     h->c.abs_pos = start;
     return 0;
 }
 int qdsp_vfofm_import_tail(qdsp_vfofm* h, const void* tail_dev, int src_device, qdsp_stream_t s) {
-    h->c.last_serial = -1;
+    h->c.chain.clear();
     return import_tail_impl(h->c.hist, tail_dev, src_device, as_stream(s));
 }
 int qdsp_vfofm_history_len(qdsp_vfofm* h) { return h->c.hist.H; }
@@ -1027,7 +1018,7 @@ long long qdsp_channelizer_process(qdsp_channelizer* h, const void* in_dev, floa
                       as_stream(s));
 }
 int qdsp_channelizer_reset(qdsp_channelizer* h) {
-    h->last_serial = -1;
+    h->chain.clear();
     QDSP_CUDA_OK(cudaDeviceSynchronize());
     if (h->hist.reset(nullptr) != 0) return -1;
     std::vector<float> z(2 * h->nch, 0.0f);
@@ -1040,12 +1031,12 @@ int qdsp_channelizer_set_input_format(qdsp_channelizer* h, int fmt, float scale,
     return h->set_input_format(fmt, scale, offset, "channelizer_set_input_format");
 }
 int qdsp_channelizer_set_variant(qdsp_channelizer* h, int variant) {
-    h->last_serial = -1;
+    h->chain.clear();
     h->variant = variant;
     return 0;
 }
 int qdsp_channelizer_seek(qdsp_channelizer* h, long long start) {
-    h->last_serial = -1;
+    h->chain.clear();
     h->abs_pos = start;
     return 0;
 }
@@ -1157,15 +1148,9 @@ qdsp_deemp* qdsp_deemp_create(float sampleRate, float tau) {
 }
 void qdsp_deemp_destroy(qdsp_deemp* h) { delete h; }
 // the chunk-with-warm-up recurrences re-read input that a neighbouring chunk's thread overwrites when out aliases in
-static bool ranges_overlap(const void* a, const void* b, long long count, size_t elem) {
-    const char* pa = (const char*)a;
-    const char* pb = (const char*)b;
-    const size_t bytes = (size_t)count * elem;
-    return pa < pb + bytes && pb < pa + bytes;
-}
 long long qdsp_deemp_process(qdsp_deemp* h, const void* in_dev, void* out_dev, long long count, qdsp_stream_t s) {
     if (count < 0) return -1;
-    if (count > 0 && ranges_overlap(in_dev, out_dev, count, 8)) {
+    if (count > 0 && ranges_overlap(in_dev, (size_t)count * 8, out_dev, (size_t)count * 8)) {
         set_last_error("deemp_process: in and out must not overlap (chunked scan with warm-up re-reads the input)");
         return -1;
     }
@@ -1331,7 +1316,7 @@ void qdsp_costas_destroy(qdsp_costas* h) { delete h; }
 long long qdsp_costas_process(qdsp_costas* h, const void* in_dev, void* out_dev, long long count, qdsp_stream_t s) {
     if (count < 0) return -1;
     if (count == 0) return 0;
-    if (ranges_overlap(in_dev, out_dev, count, 8)) {
+    if (ranges_overlap(in_dev, (size_t)count * 8, out_dev, (size_t)count * 8)) {
         set_last_error("costas_process: in and out must not overlap (chunked scan with warm-up re-reads the input)");
         return -1;
     }

@@ -1,5 +1,6 @@
-// qdsp_b200/csrc/decim_common.cuh — pieces shared by the decimating-FIR kernel families (k_decim.cu: column-pair
-// kernels; k_rowlane.cu: row-per-lane kernel): plan / argument structs, mbarrier + TMA bulk-copy PTX wrappers, and
+// qdsp_b200/csrc/decim_common.cuh — pieces shared by the FIR kernel families (k_decim.cu: column-pair kernels;
+// k_rowlane.cu, k_firrow.cu: row-per-lane kernels; k_fir.cu: dense FIR): plan / argument structs, mbarrier + TMA
+// bulk-copy PTX wrappers, the overlapped-call helpers (programmatic dependent launch, folded history advance), and
 // the brute-force single output used for a block's leading FM-demod angle.
 #pragma once
 #include <stdlib.h>
@@ -95,6 +96,33 @@ __device__ __forceinline__ void tma_bulk_g2s(void* dst_smem, const void* src_gme
                      smem_u32(dst_smem)),
                  "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
+}
+
+// ---- overlapped consecutive calls (DESIGN.md §6.0f) ---------------------------------------------------------------
+// The kernels of k_fir.cu (fir_cplx_kernel, fir_longcplx_kernel), k_firrow.cu (fir_rowcplx_kernel, fir_slide4_kernel)
+// and k_rowlane.cu (decim_rowlane_kernel) fold the history advance into their launch: a CTA writes the advanced tail to
+// `hist_next` (fold_history), the other half of the handle's double buffer, and the next call reads it as `hist`. The
+// next call of the same handle may then be launched with programmatic dependent launch (launch_ex, overlap) and start
+// while this grid drains. Ordering rests on one rule: whatever the previous grid also touches -- `hist`, which it wrote,
+// `hist_next`, which it read as its `hist`, and the fused chain's demodulator phase and audio -- a CTA touches only after
+// pdl_wait(), which returns once the previous grid has completed and its writes are visible. Every other access reads
+// this call's `in` and writes this call's `out`; the launcher overlaps a call only when those do not touch the previous
+// call's buffers (api.cu, CallChain). A grid that has waited completes after its predecessor, so the order holds down
+// a whole chain of calls. pdl_launch_dependents() only lets the next grid be scheduled early; where a kernel calls it does
+// not change what it computes. Without the launch attribute both instructions are no-ops.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;"); }
+
+// folded history advance (filter.h:71 / resampling.h:129): hist_next[j] = (hist ++ in)[count - H + j], the CTA's threads
+// t, t + nt, ... sharing the H elements. The kernels pass fields of their __grid_constant__ parameter; taken by reference,
+// a field is read where the loop reads it. A caller that wants H and count loaded once before the loop passes values
+// (k_fir.cu: +fa.H).
+__device__ __forceinline__ void fold_history(const float2* const& hist, const float2* const& in, const int& H, const long long& count,
+                                             float2* const& hist_next, int t, int nt) {
+    for (int j = t; j < H; j += nt) {
+        const long long v = count - H + j;
+        hist_next[j] = v >= 0 ? in[v] : hist[H + v];
+    }
 }
 
 // single output by brute force (warp-cooperative): used for the one "previous output" a block's first

@@ -26,8 +26,8 @@ inline void count_launch(int n = 1) { g_launches.fetch_add(n, std::memory_order_
 inline cudaStream_t as_stream(qdsp_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
 
 // Launches kern(*arg) (one kernel-parameter struct). overlap: programmatic dependent launch -- the grid may start while
-// the previous grid of the stream drains, the kernel orders what it shares with it by griddepcontrol.wait (a no-op
-// without the attribute). QDSP_PDL=0 never overlaps: the serialized reference of the overlapped-call tests.
+// the previous grid of the stream drains, the kernel orders what it shares with it by pdl_wait() (decim_common.cuh).
+// QDSP_PDL=0 never overlaps: the serialized reference of the overlapped-call tests.
 inline cudaError_t launch_ex(const void* kern, dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool overlap, void* arg) {
     static const bool pdl = getenv("QDSP_PDL") ? atoi(getenv("QDSP_PDL")) != 0 : true;
     cudaLaunchConfig_t cfg = {};

@@ -462,16 +462,6 @@ struct FirCplxArgs {
     float2* hist_next;        // when non-null: CTA 0 writes the advanced history tail here (filter.h:71)
     alignas(16) float g[256];
 };
-// Folded history advance + the ordering of overlapped consecutive calls (see k_firrow.cu / DESIGN.md 6.0c): the CTAs
-// that touch the carried history wait for the previous grid (a no-op without the launch attribute), everything else
-// reads only `in` and writes only `out`.
-__device__ __forceinline__ void fir_fold_history(const float2* hist, const float2* in, int H, long long count, float2* hist_next,
-                                                 int t, int nt) {
-    for (int j = t; j < H; j += nt) {
-        const long long v = count - H + j;
-        hist_next[j] = v >= 0 ? in[v] : hist[H + v];
-    }
-}
 template <int T, int K>
 __global__ void __launch_bounds__(32) fir_cplx_kernel(const __grid_constant__ FirCplxArgs fa) {
     constexpr int R = 9, STEP = 32 * R, NOUT = K * STEP, NS = NOUT + T - 1;
@@ -481,8 +471,10 @@ __global__ void __launch_bounds__(32) fir_cplx_kernel(const __grid_constant__ Fi
     const int lane = threadIdx.x;
     const long long n_t = (long long)blockIdx.x * NOUT;               // first output of the tile
     const long long B = n_t - (T - 1);                                // sample index of win[0]
-    if (blockIdx.x == 0 || B < 0) asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (blockIdx.x == 0 && fa.hist_next != nullptr) fir_fold_history(fa.hist, fa.in, fa.H, fa.count, fa.hist_next, lane, 32);
+    // overlapped consecutive calls (decim_common.cuh): CTA 0 folds the history, a tile whose window starts before sample 0
+    // reads it
+    if (blockIdx.x == 0 || B < 0) pdl_wait();
+    if (blockIdx.x == 0 && fa.hist_next != nullptr) fold_history(fa.hist, fa.in, +fa.H, +fa.count, fa.hist_next, lane, 32);
     if (B >= 0 && B + NS <= fa.count) {
         if (lane == 0) {
             mbar_init(&s_mbar, 1);
@@ -490,11 +482,11 @@ __global__ void __launch_bounds__(32) fir_cplx_kernel(const __grid_constant__ Fi
             mbar_arrive_expect_tx(&s_mbar, (uint32_t)NS * 8u);
             tma_bulk_g2s(win, fa.in + B, (uint32_t)NS * 8u, &s_mbar);
         }
-        asm volatile("griddepcontrol.launch_dependents;");
+        pdl_launch_dependents();
         __syncwarp();
         mbar_wait(&s_mbar, 0);
     } else {   // history before sample 0 / ragged end: guarded fill
-        asm volatile("griddepcontrol.launch_dependents;");
+        pdl_launch_dependents();
         VStream<float2> xs{fa.hist, fa.in, fa.H};
         for (int e = lane; e < NS; e += 32) {
             const long long idx = B + e;
@@ -556,9 +548,10 @@ __global__ void __launch_bounds__(256, 3) fir_longcplx_kernel(const __grid_const
     const int NS = NOUT + Tp - 1;                                         // even: NOUT even, Tp odd
     const long long n_t = (long long)blockIdx.x * NOUT;                   // first output of the tile
     const long long B = n_t - (Tp - 1);                                   // sample index of win[0] (even)
-    if (blockIdx.x == 0 || B < 0) asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (blockIdx.x == 0 && fa.hist_next != nullptr) fir_fold_history(fa.hist, fa.in, fa.H, fa.count, fa.hist_next, t, NT);
-    asm volatile("griddepcontrol.launch_dependents;");
+    // overlapped consecutive calls: as in fir_cplx_kernel (with 4095 taps, tiles after the first may start before sample 0)
+    if (blockIdx.x == 0 || B < 0) pdl_wait();
+    if (blockIdx.x == 0 && fa.hist_next != nullptr) fold_history(fa.hist, fa.in, +fa.H, +fa.count, fa.hist_next, t, NT);
+    pdl_launch_dependents();
     if (B >= 0 && B + NS <= fa.count) {
         if (t == 0) {
             mbar_init(&s_mbar, 1);

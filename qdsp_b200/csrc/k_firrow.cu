@@ -57,18 +57,10 @@ __global__ void __launch_bounds__(32) fir_rowcplx_kernel(const __grid_constant__
     const int rows_per_tile = 32 * fa.nstep - (Q - 1);
     const long long row_t0 = (long long)blockIdx.x * rows_per_tile;
     const long long nrows_total = (fa.n_out + NPH - 1) / NPH;
-    // programmatic dependent launch (launch_firrow, overlap_prev): the next call of the same handle may start while this
-    // grid drains. Its only true dependencies are the history hand-over -- tile 0 reads `hist`, written by the previous
-    // call's CTA 0, and writes `hist_next`, which the previous call's tile 0 read -- so CTA 0 alone waits for the previous
-    // grid to complete; every other CTA reads only `in` and writes only `out` (the launcher has checked that they do not
-    // overlap the previous call's buffers). Without the launch attribute both instructions are no-ops.
-    if (blockIdx.x == 0) asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (fa.hist_next != nullptr && blockIdx.x == 0) {
-        for (int j = lane; j < fa.H; j += 32) {
-            const long long v = fa.count - fa.H + j;
-            fa.hist_next[j] = v >= 0 ? fa.in[v] : fa.hist[fa.H + v];
-        }
-    }
+    // overlapped consecutive calls (decim_common.cuh): CTA 0 alone waits -- it folds the history, and only tile 0's window
+    // starts before sample 0
+    if (blockIdx.x == 0) pdl_wait();
+    if (fa.hist_next != nullptr && blockIdx.x == 0) fold_history(fa.hist, fa.in, fa.H, fa.count, fa.hist_next, lane, 32);
     if (row_t0 >= nrows_total) return;
     const long long left = nrows_total - row_t0;
     const int nrows_emit = left < rows_per_tile ? (int)left : rows_per_tile;
@@ -102,7 +94,7 @@ __global__ void __launch_bounds__(32) fir_rowcplx_kernel(const __grid_constant__
         }
     };
     for (int i = 0; i < NSTG; i++) issue(i);
-    asm volatile("griddepcontrol.launch_dependents;");
+    pdl_launch_dependents();
     float2 old[NPH];
 #pragma unroll
     for (int j = 0; j < NPH; j++) old[j] = make_float2(0.f, 0.f);
@@ -215,14 +207,10 @@ __global__ void __launch_bounds__(32) fir_slide4_kernel(const __grid_constant__ 
     __shared__ __align__(128) float2 win[NS];
     __shared__ uint64_t s_mbar;
     const int lane = threadIdx.x;
-    // overlapped consecutive calls: see fir_rowcplx_kernel
-    if (blockIdx.x == 0) asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (fa.hist_next != nullptr && blockIdx.x == 0) {     // folded history advance: new_hist[j] = virtual[count - H + j]
-        for (int j = lane; j < fa.H; j += 32) {
-            const long long v = fa.count - fa.H + j;
-            fa.hist_next[j] = v >= 0 ? fa.in[v] : fa.hist[fa.H + v];
-        }
-    }
+    // overlapped consecutive calls (decim_common.cuh): CTA 0 alone waits -- it folds the history, and only tile 0's window
+    // starts before sample 0
+    if (blockIdx.x == 0) pdl_wait();
+    if (fa.hist_next != nullptr && blockIdx.x == 0) fold_history(fa.hist, fa.in, fa.H, fa.count, fa.hist_next, lane, 32);
     const long long k_t = (long long)blockIdx.x * NOUT;               // first output of the tile
     if (k_t >= fa.n_out) return;
     const long long B = D * k_t - T - 1;                              // sample index of win[0]
@@ -233,11 +221,11 @@ __global__ void __launch_bounds__(32) fir_slide4_kernel(const __grid_constant__ 
             mbar_arrive_expect_tx(&s_mbar, (uint32_t)NS * 8u);
             tma_bulk_g2s(win, fa.in + B, (uint32_t)NS * 8u, &s_mbar);
         }
-        asm volatile("griddepcontrol.launch_dependents;");
+        pdl_launch_dependents();
         __syncwarp();
         mbar_wait(&s_mbar, 0);
     } else {   // history before sample 0 / ragged end: guarded fill
-        asm volatile("griddepcontrol.launch_dependents;");
+        pdl_launch_dependents();
         VStream<float2> xs{fa.hist, fa.in, fa.H};
         for (int e = lane; e < NS; e += 32) {
             const long long idx = B + e;

@@ -55,21 +55,13 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
     const int k0 = tile * LT;
     if (ra.tstamp != nullptr && tile == 0 && b == 0 && lane == 0) atomicMin(&ra.tstamp[0], globaltimer_ns());
 
-    // Overlapped consecutive calls (programmatic dependent launch, launch_decim_rowlane's overlap_prev): the next call of
-    // the same handle may start while this grid drains. The state carried from call to call -- `hist` and `demod_in`,
-    // written by the previous grid, and `hist_next`, which the previous grid read as `hist` -- is touched only by the
-    // CTAs that wait for the previous grid at their start: CTA (0,0), and a tile whose rows or leading-angle window reach
-    // before sample 0 or which takes its leading angle from `demod_in`. Every other CTA reads only `in` (the launcher
-    // refuses an input that overlaps the previous call's audio) and holds its audio and `demod_out` until its tile is
-    // computed, then waits and stores: write-after-write on `audio` and on the `demod_out` ping-pong stays ordered
-    // whatever buffers the caller passes. Without the launch attribute both instructions are no-ops.
-    // ---- folded history advance: new_hist[j] = virtual[count - H + j] ------------------------------
+    // Overlapped consecutive calls (decim_common.cuh). A CTA waits at its start when it folds the history (CTA (0,0)), when
+    // its rows or its leading-angle window reach before sample 0, or when it takes its leading angle from `demod_in`.
+    // Every fused CTA waits again before it stores its held audio and `demod_out`, so write-after-write on them stays ordered
+    // whatever buffers the caller passes; the launcher only refuses an input that overlaps the previous call's audio.
     if (ra.hist_next != nullptr && tile == 0 && b == 0) {
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-        for (int j = lane; j < a.H; j += 32) {
-            const long long v = a.n_in - a.H + j;
-            ra.hist_next[j] = v >= 0 ? a.in[v] : a.hist[a.H + v];
-        }
+        pdl_wait();
+        fold_history(a.hist, a.in, a.H, a.n_in, ra.hist_next, lane, 32);
     }
     if (k0 >= bi.out_count) return;
 
@@ -108,7 +100,7 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
             ovr_win = pbi.in_start + (long long)(pbi.out_count - 1) * D - a.T;
         }
     }
-    if (row0 < 0 || (use_override && (pb < 0 || ovr_win < 0))) asm volatile("griddepcontrol.wait;" ::: "memory");
+    if (row0 < 0 || (use_override && (pb < 0 || ovr_win < 0))) pdl_wait();
     if (use_override) {
         if (pb < 0) {
             override_ang = a.demod_in[0];
@@ -142,7 +134,7 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
         }
     };
     for (int i = 0; i < NSTG; i++) issue(i);
-    asm volatile("griddepcontrol.launch_dependents;");
+    pdl_launch_dependents();
 
     // ---- per-lane state -------------------------------------------------------------------------------
     float2 Pr = make_float2(1.f, 0.f);        // row phasor of this lane's current row
@@ -241,7 +233,7 @@ __global__ void __launch_bounds__(32) decim_rowlane_kernel(const __grid_constant
         }
     }
     if (DEMOD) {
-        asm volatile("griddepcontrol.wait;" ::: "memory");
+        pdl_wait();
         __syncwarp();
         for (int e = LEAD + lane; e < nout + LEAD; e += 32) a.audio[obase + e] = hold[e];
         if (last_here) a.demod_out[0] = last_ang;

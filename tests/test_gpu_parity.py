@@ -10,6 +10,7 @@ import pytest
 from oracle import loader
 from tests.cases import CASES, make_input
 from tests.runners import rel_l2, run_gpu, run_port
+from tests.test_iq_formats import _bits_equal
 
 pytestmark = pytest.mark.gpu
 
@@ -849,83 +850,61 @@ def test_fir_constant_bank_kernel_tap_counts(ntaps):
     assert rel_l2(y, yo) <= 1e-5, rel_l2(y, yo)
 
 
-def test_resampler_back_to_back_calls_overlapped_launches():
-    # consecutive calls of ONE handle with disjoint buffers are launched so that their grids may overlap (programmatic
-    # dependent launch; only the history hand-over is ordered). 12 back-to-back calls on preloaded device buffers, nothing
-    # in between, against the oracle over the whole stream; then the same stream again with ONE output buffer reused by
-    # every call (overlap refused by the launcher: write-after-write) and with out == the previous call's in
-    from qdsp_b200 import blocks as B, synth
+@pytest.fixture(scope="module")
+def overlap_runs():
+    from tests import overlapped
 
-    P = loader.port()
-    win = B.BlackmanWindow(300e3, 4 * 2.4e6 / 127, 2.4e6)
-    taps = P.blackman_taps(300e3, 4 * 2.4e6 / 127, 2.4e6)
-    ncall, n, blk = 12, 1 << 19, 1 << 17
-    x = synth.uniform_cf32(11, 0, ncall * n)
-    yo, _ = P.resamp_cf32(taps, 1, 4, x, blk)
-    ins = [B.DevBuf.from_numpy(x[i * n:(i + 1) * n]) for i in range(ncall)]
-    outs = [B.DevBuf(n // 4 * 8) for _ in range(ncall)]
-    r = B.PolyphaseResampler(win, 2.4e6, 0.6e6)
-    for i in range(ncall):
-        assert r.process_device(ins[i].ptr, outs[i].ptr, n, blk) == n // 4
-    y = np.concatenate([o.to_numpy(np.complex64, n // 4) for o in outs])
+    return overlapped.runs()
+
+
+def test_resampler_back_to_back_calls_overlapped_launches(overlap_runs):
+    # consecutive calls of ONE handle with disjoint buffers are launched so that their grids may overlap (programmatic
+    # dependent launch; only the history hand-over is ordered). 12 back-to-back calls on preloaded buffers, nothing in
+    # between, against the oracle over the whole stream; then the same stream again with ONE output buffer reused by
+    # every call (overlap refused by the launcher: write-after-write), with and without a read-back between the calls.
+    # Every sequence is bit-identical to serialized launches (tests/overlapped.py)
+    from qdsp_b200 import synth
+    from tests.overlapped import RS_BLK, RS_N, RS_NCALL, _resampler_taps
+
+    ours, serial = overlap_runs
+    for k in ("resamp_distinct", "resamp_one_out", "resamp_one_out_last"):
+        assert _bits_equal(ours[k], serial[k]), k
+    x = synth.uniform_cf32(11, 0, RS_NCALL * RS_N)
+    yo, _ = loader.port().resamp_cf32(_resampler_taps(), 1, 4, x, RS_BLK)
+    y = ours["resamp_distinct"]
     assert rel_l2(y, yo) <= 1e-5, rel_l2(y, yo)
-    # one output buffer for every call: each call's result is read back before the next call
-    r2 = B.PolyphaseResampler(win, 2.4e6, 0.6e6)
-    parts = []
-    for i in range(ncall):
-        r2.process_device(ins[i].ptr, outs[0].ptr, n, blk)
-        parts.append(outs[0].to_numpy(np.complex64, n // 4))
-    assert rel_l2(np.concatenate(parts), yo) <= 1e-5
-    # no read-back between the calls, the same output buffer: the last call's result must be the one that stays
-    r3 = B.PolyphaseResampler(win, 2.4e6, 0.6e6)
-    for i in range(ncall):
-        r3.process_device(ins[i].ptr, outs[1].ptr, n, blk)
-    last = outs[1].to_numpy(np.complex64, n // 4)
-    assert rel_l2(last, yo[(ncall - 1) * (n // 4):]) <= 1e-5
-    for b in ins + outs:
-        b.free()
+    assert rel_l2(ours["resamp_one_out"], yo) <= 1e-5
+    assert rel_l2(ours["resamp_one_out_last"], yo[(RS_NCALL - 1) * (RS_N // 4):]) <= 1e-5
 
 
 @pytest.mark.parametrize("ntaps", [127, 601])
-def test_fir_back_to_back_calls_overlapped_launches(ntaps):
+def test_fir_back_to_back_calls_overlapped_launches(overlap_runs, ntaps):
     # the constant-bank FIR kernels advance the history themselves (one launch per call) and consecutive calls of one
     # handle with disjoint buffers may overlap on the GPU; 10 back-to-back calls incl. one shorter than the filter, then the
-    # refused case (one output buffer for every call) -- against the oracle over the whole stream
-    from qdsp_b200 import blocks as B, synth
+    # refused case (one output buffer for every call) -- against the oracle over the whole stream, and bit-identical to
+    # serialized launches (tests/overlapped.py)
+    from qdsp_b200 import synth
+    from tests.overlapped import FIR_SIZES, _fir_taps
 
-    P = loader.port()
-    rng = np.random.default_rng(ntaps)
-    taps = (rng.standard_normal(ntaps) * np.hanning(ntaps + 2)[1:-1] / np.sqrt(ntaps)).astype(np.float32)
-    sizes = [1 << 18, 1 << 18, 100, 1 << 18, 4 * 288 + 7, 1 << 18, 1 << 18, 2304 * 3, 1 << 18, 1 << 17]
-    x = synth.uniform_cf32(13, 0, sum(sizes))
-    yo = P.fir_cf32(taps, x)
-    offs = np.concatenate([[0], np.cumsum(sizes)])
-    ins = [B.DevBuf.from_numpy(x[offs[i]:offs[i + 1]]) for i in range(len(sizes))]
-    outs = [B.DevBuf(max(s, 2) * 8) for s in sizes]
-    f = B.FIR(B._TapsWindow(taps))
-    for i, s in enumerate(sizes):
-        assert f.process_device(ins[i].ptr, outs[i].ptr, s) == s
-    y = np.concatenate([outs[i].to_numpy(np.complex64, s) for i, s in enumerate(sizes)])
+    ours, serial = overlap_runs
+    for k in ("distinct", "one_out", "history"):
+        assert _bits_equal(ours[f"fir{ntaps}_{k}"], serial[f"fir{ntaps}_{k}"]), k
+    x = synth.uniform_cf32(13, 0, sum(FIR_SIZES))
+    yo = loader.port().fir_cf32(_fir_taps(ntaps), x)
+    y = ours[f"fir{ntaps}_distinct"]
     assert rel_l2(y, yo) <= 1e-5, rel_l2(y, yo)
-    big = B.DevBuf(max(sizes) * 8)
-    f2 = B.FIR(B._TapsWindow(taps))
-    parts = []
-    for i, s in enumerate(sizes):
-        f2.process_device(ins[i].ptr, big.ptr, s)
-        parts.append(big.to_numpy(np.complex64, s))
-    assert rel_l2(np.concatenate(parts), yo) <= 1e-5
+    assert rel_l2(ours[f"fir{ntaps}_one_out"], yo) <= 1e-5
     # history read-back after the folded advance equals the stream's tail
-    assert np.array_equal(f.get_history(), x[-(ntaps - 1):])
-    for b in ins + outs + [big]:
-        b.free()
+    assert np.array_equal(ours[f"fir{ntaps}_history"], x[-(ntaps - 1):])
 
 
-def test_resampler_sliding_window_kernel_long_calls():
+def test_resampler_sliding_window_kernel_long_calls(overlap_runs):
     # calls of >= 2^25 samples take the constant-bank sliding-window decimate-by-4 kernel (fir_slide4_kernel) instead of the
     # row-per-lane one: two consecutive calls with the history carried (the first off the decimation grid, the second cut
-    # into run() blocks with a ragged last one), then back-to-back overlapped calls on distinct device buffers, against
-    # the oracle
+    # into run() blocks with a ragged last one), then back-to-back overlapped calls on distinct device buffers
+    # (tests/overlapped.py, bit-identical to serialized launches), against the oracle
     from qdsp_b200 import blocks as B, synth
+    from tests.overlapped import SL_N, SL_NCALL
 
     P = loader.port()
     win = B.BlackmanWindow(300e3, 4 * 2.4e6 / 127, 2.4e6)
@@ -937,15 +916,9 @@ def test_resampler_sliding_window_kernel_long_calls():
     y = np.concatenate([r.process(x[:n1], n1), r.process(x[n1:], blk)])
     assert y.shape == yo.shape and rel_l2(y, yo) <= 1e-5, rel_l2(y, yo)
     del x, y, yo
-    ncall, m = 3, 1 << 25
-    x2 = synth.uniform_cf32(19, 0, ncall * m)
-    yo2, _ = P.resamp_cf32(taps, 1, 4, x2, m)
-    ins = [B.DevBuf.from_numpy(x2[i * m:(i + 1) * m]) for i in range(ncall)]
-    outs = [B.DevBuf(m // 4 * 8) for _ in range(ncall)]
-    r2 = B.PolyphaseResampler(win, 2.4e6, 0.6e6)
-    for i in range(ncall):
-        assert r2.process_device(ins[i].ptr, outs[i].ptr, m, m) == m // 4
-    y2 = np.concatenate([o.to_numpy(np.complex64, m // 4) for o in outs])
+    ours, serial = overlap_runs
+    assert _bits_equal(ours["slide_distinct"], serial["slide_distinct"])
+    x2 = synth.uniform_cf32(19, 0, SL_NCALL * SL_N)
+    yo2, _ = P.resamp_cf32(taps, 1, 4, x2, SL_N)
+    y2 = ours["slide_distinct"]
     assert rel_l2(y2, yo2) <= 1e-5, rel_l2(y2, yo2)
-    for b in ins + outs:
-        b.free()

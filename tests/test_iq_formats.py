@@ -5,7 +5,6 @@ import ctypes as C
 import math
 import os
 import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -193,48 +192,12 @@ def test_fused_ragged_table_unaligned_calls(fmt):
     assert np.abs(audio[16:] - a64[16:]).max() <= AUDIO_TOL
 
 
-def _overlap_sequences():
-    """The back-to-back call sequences of test_vfofm_overlapped_calls.py on integer input; nothing is read back between
-    the calls of a sequence."""
-    from qdsp_b200 import blocks as B, lib
-
-    L = lib.load()
-    out = {}
-    for fmt in FMTS:
-        q1, _ = _quantized(fmt, 0, N1)
-        xin = B.DevBuf.from_numpy(q1)
-        v = B.VFOFM(*CHAIN)
-        v.set_input_format(fmt)
-        m1 = v.out_count(N1, BLOCK)
-        aud = B.DevBuf((m1 + 64) * 4)
-        for _ in range(K1):
-            assert _process_raw(L, v.h, xin.ptr, aud.ptr, N1) == m1
-        out[fmt + "_same_last"] = aud.to_numpy(np.float32, m1)
-        q2, _ = _quantized(fmt, 0, sum(SIZES2))
-        offs = np.concatenate([[0], np.cumsum(SIZES2)])
-        ins = [B.DevBuf.from_numpy(q2[2 * offs[i]:2 * offs[i + 1]]) for i in range(len(SIZES2))]
-        v2 = B.VFOFM(*CHAIN)
-        v2.set_input_format(fmt)
-        cnt = [v2.out_count(s, BLOCK) for s in SIZES2]
-        auds = [B.DevBuf((c + 64) * 4) for c in cnt]
-        for i, s in enumerate(SIZES2):
-            assert _process_raw(L, v2.h, ins[i].ptr, auds[i].ptr, s) == cnt[i]
-        out[fmt + "_distinct"] = np.concatenate([a.to_numpy(np.float32, c) for a, c in zip(auds, cnt)])
-    return out
-
-
-def _dump(path):
-    np.savez(path, **_overlap_sequences())
-
-
 @pytest.fixture(scope="module")
-def overlap_runs(tmp_path_factory):
-    path = str(tmp_path_factory.mktemp("serial_iq") / "serial.npz")
-    env = dict(os.environ, QDSP_PDL="0", PYTHONPATH=ROOT)
-    code = f"from tests.test_iq_formats import _dump; _dump({path!r}); print('ok')"
-    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stdout + r.stderr
-    return _overlap_sequences(), dict(np.load(path))
+def overlap_runs():
+    # the back-to-back sequences of test_vfofm_overlapped_calls.py on integer input, overlapped and serialized
+    from tests import overlapped
+
+    return overlapped.runs()
 
 
 @pytest.mark.gpu

@@ -228,6 +228,16 @@ int qdsp_channelizer_design(qdsp_channelizer* h, int* tapCount, int* interp, int
 long long qdsp_channelizer_process(qdsp_channelizer* h, const void* in_dev, float* audio_out_dev,
                                    long long out_stride, long long count, const int* blocks, int nblocks,
                                    int block_size, qdsp_stream_t s);
+/* as qdsp_channelizer_process, and also channel c's complex baseband -- the VFO output, resampling.h:99-132 after the
+ * translator, before FloatFMDemod -- at iq_out_dev + c * out_stride (cf32, 8-byte aligned, not NULL): the input of any
+ * complex-baseband block (AM / SSB demodulation, squelch, AGC, Costas, clock recovery, ...), the reference's
+ * Splitter<complex_t> -> N x VFO. audio_out_dev may be NULL: no audio is stored, but the demodulator state advances exactly
+ * as if it had been. Same handle state as qdsp_channelizer_process (history, demodulator phases, position, seek, input
+ * format, variant); calls with and without IQ may be mixed. Returns -1 (qdsp_last_error) for a NULL or misaligned
+ * iq_out_dev and wherever qdsp_channelizer_process would. */
+long long qdsp_channelizer_process_iq(qdsp_channelizer* h, const void* in_dev, void* iq_out_dev, float* audio_out_dev,
+                                      long long out_stride, long long count, const int* blocks, int nblocks,
+                                      int block_size, qdsp_stream_t s);
 int qdsp_channelizer_reset(qdsp_channelizer* h);
 /* as qdsp_vfofm_set_input_format */
 int qdsp_channelizer_set_input_format(qdsp_channelizer* h, int fmt, float scale, float offset);

@@ -638,7 +638,7 @@ class VFOFM(_InputFormat, _Block):
 class Channelizer(_InputFormat, _Block):
     """nch x [VFO -> FloatFMDemod] fed by one Splitter (routing.h:47-57): every channel reads the same
     device-resident wideband buffer; output is [nch, n_out] float32. set_input_format as VFOFM (the channelizer's
-    kernels read the input converted to cf32)."""
+    kernels read the input converted to cf32). process_iq also returns every channel's complex baseband."""
 
     _destroy = "qdsp_channelizer_destroy"
     _set_fmt = "qdsp_channelizer_set_input_format"
@@ -677,6 +677,27 @@ class Channelizer(_InputFormat, _Block):
         m = self.process_device(din.ptr, dout.ptr, n, stride, block)
         y = dout.to_numpy(np.float32, self.nch * stride).reshape(self.nch, stride)[:, :m].copy()
         return y
+
+    def process_device_iq(self, in_ptr, iq_ptr, audio_ptr, n, out_stride, block=None, stream=None) -> int:
+        """As process_device, and also every channel's complex baseband (the VFO output, before the FM demodulator):
+        channel c at iq_ptr + c * out_stride complex64 elements. audio_ptr may be None (no audio stored; the demodulator
+        state advances as if it had been)."""
+        b, nb, bs = _blocks_arg(n, block)
+        return int(check(_L().qdsp_channelizer_process_iq(self.h, in_ptr, iq_ptr, audio_ptr, int(out_stride), int(n), _iptr(b),
+                                                          nb, bs, stream), "qdsp_channelizer_process_iq"))
+
+    def process_iq(self, x, block=None, audio=True):
+        """Complex baseband of every channel, [nch, n_out] complex64 -- the input of any complex-baseband block (AMDemod,
+        SSBDemod, Squelch, ComplexAGC, CostasLoop, ...). With audio=True returns (iq, audio [nch, n_out] float32)."""
+        x, n = _iq_input(x, self._in_fmt)
+        stride = (n * self._interp) // self._decim + 16
+        din, diq = DevBuf.from_numpy(x), DevBuf(self.nch * stride * 8)
+        dout = DevBuf(self.nch * stride * 4) if audio else None
+        m = self.process_device_iq(din.ptr, diq.ptr, dout.ptr if audio else None, n, stride, block)
+        iq = diq.to_numpy(np.complex64, self.nch * stride).reshape(self.nch, stride)[:, :m].copy()
+        if not audio:
+            return iq
+        return iq, dout.to_numpy(np.float32, self.nch * stride).reshape(self.nch, stride)[:, :m].copy()
 
 
 class IQConverter(_Block):

@@ -600,6 +600,9 @@ struct qdsp_channelizer {
     int in_fmt = QDSP_CF32;
     IqConv in_conv{1.0f, 0.0f};
     Scratch conv;
+    // IQ-only calls (qdsp_channelizer_process_iq with no audio buffer): the direct forms store their audio here instead,
+    // so the demodulator state advances as if it had been stored (grown to the largest call: no allocation in steady state)
+    Scratch audio_sink;
 
     int set_input_format(int fmt, float scale, float offset, const char* who) {
         if (fmt != QDSP_CF32 && !iq_format_ok(fmt, scale, offset, who)) return -1;
@@ -675,13 +678,19 @@ struct qdsp_channelizer {
             if (launch_iq_convert(in_fmt, in_conv, in_dev, (float2*)conv.p, count, s) != 0) return -1;
             in_dev = conv.p;
         }
+        const bool fft = fftplan && variant == 0 && chanfft_usable(fftplan, part, in_dev);
+        if (!audio && !fft) {
+            // the FFT form has an IQ-only kernel; the direct forms store their audio to scratch
+            if (audio_sink.reserve(((size_t)(nch - 1) * (size_t)out_stride + (size_t)part.total_out) * sizeof(float)) != 0) return -1;
+            audio = (float*)audio_sink.p;
+        }
         if (events) QDSP_CUDA_OK(cudaEventRecord(ev_k0, s));
         bool hist_folded = false;
         int rpad = -1;
-        if (fftplan && variant == 0 && !iq && chanfft_usable(fftplan, part, in_dev)) {
+        if (fft) {
             // all 256 channels from one pass of column filters + two 256-point FFTs per output row
             rc = launch_chanfft(fftplan, (const float2*)hist.ptr(), hist.H, (const float2*)in_dev, part, nco[0].step, nco[0].phase,
-                                abs_pos, phasor_speed, din, dout, audio, out_stride, s);
+                                abs_pos, phasor_speed, din, dout, audio, (float2*)iq, out_stride, s);
         } else if (plan && variant != 1 && nch == 1 && rowlane_supported(plan) && (reinterpret_cast<uintptr_t>(in_dev) & 15) == 0 &&
             part.max_out > 0 && (rpad = rowlane_uniform_pad(part, T)) >= 0) {
             // row-per-lane kernel; the history advance (resampling.h:129) is folded into its first CTA
@@ -1015,6 +1024,16 @@ long long qdsp_channelizer_process(qdsp_channelizer* h, const void* in_dev, floa
                                    long long out_stride, long long count, const int* blocks, int nblocks,
                                    int block_size, qdsp_stream_t s) {
     return h->process(in_dev, audio_out_dev, nullptr, out_stride, count, blocks, nblocks, block_size, nullptr,
+                      as_stream(s));
+}
+long long qdsp_channelizer_process_iq(qdsp_channelizer* h, const void* in_dev, void* iq_out_dev, float* audio_out_dev,
+                                      long long out_stride, long long count, const int* blocks, int nblocks,
+                                      int block_size, qdsp_stream_t s) {
+    if (!iq_out_dev || (reinterpret_cast<uintptr_t>(iq_out_dev) & 7) != 0) {
+        set_last_error("channelizer_process_iq: iq_out_dev must be a non-NULL, 8-byte aligned cf32 buffer");
+        return -1;
+    }
+    return h->process(in_dev, audio_out_dev, iq_out_dev, out_stride, count, blocks, nblocks, block_size, nullptr,
                       as_stream(s));
 }
 int qdsp_channelizer_reset(qdsp_channelizer* h) {

@@ -22,7 +22,8 @@
 // rows per stage). Writes U, V per (row, column).
 // Kernel B (chanfft_fft_kernel): 15 output rows (+ the predecessor of the first, for the FM difference) per CTA; the two
 // 256-point FFTs of a row as 16 x 16 with both 16-point passes in registers and ONE shared-memory transpose; per-channel
-// phase (64-bit turn arithmetic, MUFU sin/cos), first-order correction, fast_arctan2 + FM step, transposed store.
+// phase (64-bit turn arithmetic, MUFU sin/cos), first-order correction, fast_arctan2 + FM step, transposed store of the
+// audio and / or of the channel samples themselves (the complex baseband, qdsp_channelizer_process_iq).
 #include <math.h>
 #include <new>
 #include <vector>
@@ -241,6 +242,7 @@ struct ChanFftBArgs {
     float* audio;
     long long out_stride;
     float inv_speed;                // 1 / phasorSpeed (demodulator.h:91)
+    float2* iq;                     // [M][out_stride] channel baseband (IQ instantiations)
 };
 
 // The reference's fast_arctan2 (demodulator.h:11-30) with the quotient from the reciprocal unit (<= 2 ulp: 2e-7 rad) and a
@@ -274,12 +276,16 @@ __device__ __forceinline__ float2 phasor_mufu(uint64_t turns) {
 // 256-point FFTs as 16 x 16 (four-step) with both 16-point passes in registers: thread (f, c) = (row of the CTA, column).
 // Pass 1: column n2 = c of row f, over n1 (input index 16 n1 + n2), twiddle W256^{n2 k1}; transpose through shared memory;
 // pass 2: k1 = c, over n2: bins k1 + 16 k2. U and V of a row share the thread (and the twiddles).
+// AUDIO: FM audio into `audio`; IQ: the channel samples y themselves into `iq`, staged in the (by then free) transpose tiles
+// and stored transposed like the audio. Without AUDIO the angle is taken only where the carried state needs it: the last row.
+template <bool AUDIO, bool IQ>
 __global__ void __launch_bounds__(kCfM, 2) chanfft_fft_kernel(const ChanFftBArgs a) {
     extern __shared__ __align__(16) unsigned char smem_b[];
     float2* sU = reinterpret_cast<float2*>(smem_b);
     float2* sV = sU + kCfRB * 16 * kCfLd;
     float2* tw = sV + kCfRB * 16 * kCfLd;
     float* s_ang = reinterpret_cast<float*>(tw + kCfM);            // [kCfRB][M + 1]
+    float2* s_y = sU;                                                // [kCfRB][M + 1] (IQ): over the transpose tiles
     const int t = threadIdx.x, f = t >> 4, c = t & 15;
     const long long m0 = (long long)blockIdx.x * kCfNew;
     const long long m = m0 - 1 + f;
@@ -316,6 +322,7 @@ __global__ void __launch_bounds__(kCfM, 2) chanfft_fft_kernel(const ChanFftBArgs
     }
     fft16(u);
     fft16(v);
+    if (IQ) __syncthreads();               // every row is done with the transpose tiles: s_y overwrites them
     // epilogue: bins c + 16 k2 of row m
     const long long Ns = a.abs0 + m * (long long)a.D - a.T;
     const unsigned A9 = (unsigned)((Ns - a.pad) & (2 * kCfM - 1));
@@ -334,22 +341,29 @@ __global__ void __launch_bounds__(kCfM, 2) chanfft_fft_kernel(const ChanFftBArgs
         const unsigned long long turns = a.ph0 + (unsigned long long)__ldg(a.dturn + k) * (unsigned long long)Ns +
                                          (unsigned long long)__ldg(a.dt0 + k) + ((unsigned long long)(hb * A9) << 55);
         const float2 y = cmul(Y, phasor_mufu(turns));
-        ang_row[k] = fast_arctan2_rcp(y.y, y.x);
+        if (AUDIO) ang_row[k] = fast_arctan2_rcp(y.y, y.x);
+        if (IQ) s_y[f * (kCfM + 1) + k] = y;
     }
     if (carried || last) {
 #pragma unroll 1
         for (int k2 = 0; k2 < 16; k2++) {
             const int k = (c + 16 * k2 + (a.twob >> 1)) & (kCfM - 1);
-            if (carried) ang_row[k] = a.demod_in[k];
+            if (!AUDIO) {
+                // the thread's own s_y entries: the last row's angle is the carried state
+                if (last) a.demod_out[k] = fast_arctan2_rcp(s_y[f * (kCfM + 1) + k].y, s_y[f * (kCfM + 1) + k].x);
+            } else if (carried) ang_row[k] = a.demod_in[k];
             else a.demod_out[k] = ang_row[k];
         }
     }
     __syncthreads();
-    // transposed store: consecutive threads write consecutive rows of one channel
+    // transposed store: consecutive threads write consecutive rows of one channel (nothing for the carried row)
     for (int idx = t; idx < kCfNew * kCfM; idx += kCfM) {
         const int k = idx / kCfNew, mr = idx - k * kCfNew;
-        if (m0 + mr < a.total_out)
-            a.audio[(size_t)k * a.out_stride + m0 + mr] = fm_step_mul(s_ang[(mr + 1) * (kCfM + 1) + k], s_ang[mr * (kCfM + 1) + k], a.inv_speed);
+        if (m0 + mr < a.total_out) {
+            if (AUDIO)
+                a.audio[(size_t)k * a.out_stride + m0 + mr] = fm_step_mul(s_ang[(mr + 1) * (kCfM + 1) + k], s_ang[mr * (kCfM + 1) + k], a.inv_speed);
+            if (IQ) a.iq[(size_t)k * a.out_stride + m0 + mr] = s_y[(mr + 1) * (kCfM + 1) + k];
+        }
     }
 }
 
@@ -455,7 +469,7 @@ static int chanfft_pick_seg(const Partition& part) {
 
 int launch_chanfft(ChanFftPlan* plan, const float2* hist, int H, const float2* in, const Partition& part, uint64_t beta_step,
                    uint64_t beta_ph0, long long abs0, float phasor_speed, const float* demod_in, float* demod_out, float* audio,
-                   long long out_stride, cudaStream_t s) {
+                   float2* iq, long long out_stride, cudaStream_t s) {
     const long long rows = part.total_out;
     const size_t need = (size_t)2 * rows * kCfM;
     if (need > plan->uv_cap) {
@@ -490,7 +504,9 @@ int launch_chanfft(ChanFftPlan* plan, const float2* hist, int H, const float2* i
     if (!attr) {
         QDSP_CUDA_OK(cudaFuncSetAttribute(chanfft_poly_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         QDSP_CUDA_OK(cudaFuncSetAttribute(chanfft_poly_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        QDSP_CUDA_OK(cudaFuncSetAttribute(chanfft_fft_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        QDSP_CUDA_OK(cudaFuncSetAttribute(chanfft_fft_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        QDSP_CUDA_OK(cudaFuncSetAttribute(chanfft_fft_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        QDSP_CUDA_OK(cudaFuncSetAttribute(chanfft_fft_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
         attr = true;
     }
     dim3 grid((part.max_out + a.seg_rows - 1) / a.seg_rows, part.view.nblocks);
@@ -517,7 +533,14 @@ int launch_chanfft(ChanFftPlan* plan, const float2* hist, int H, const float2* i
     bb.audio = audio;
     bb.out_stride = out_stride;
     bb.inv_speed = (float)(1.0 / (double)phasor_speed);
-    chanfft_fft_kernel<<<(unsigned)((rows + kCfNew - 1) / kCfNew), kCfM, smem_b, s>>>(bb);
+    bb.iq = iq;
+    const unsigned nb = (unsigned)((rows + kCfNew - 1) / kCfNew);
+    if (!iq)
+        chanfft_fft_kernel<true, false><<<nb, kCfM, smem_b, s>>>(bb);
+    else if (audio)
+        chanfft_fft_kernel<true, true><<<nb, kCfM, smem_b, s>>>(bb);
+    else
+        chanfft_fft_kernel<false, true><<<nb, kCfM, smem_b, s>>>(bb);
     QDSP_LAUNCH_OK();
     return 0;
 }

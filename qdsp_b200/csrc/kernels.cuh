@@ -75,7 +75,7 @@ void chanfft_plan_destroy(ChanFftPlan* p);
 bool chanfft_usable(const ChanFftPlan* p, const Partition& part, const void* in);
 int launch_chanfft(ChanFftPlan* plan, const float2* hist, int H, const float2* in, const Partition& part, uint64_t beta_step,
                    uint64_t beta_ph0, long long abs0, float phasor_speed, const float* demod_in, float* demod_out, float* audio,
-                   long long out_stride, cudaStream_t s);
+                   float2* iq, long long out_stride, cudaStream_t s);
 
 // ---- k_spectrum.cu: Welch power spectrum (windowed N-point FFT frames, |X|^2 averaged per row, FFT-shifted) --------------
 struct SpectrumPlan;

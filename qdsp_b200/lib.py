@@ -123,6 +123,7 @@ SIGNATURES = {
     "qdsp_channelizer_destroy": (None, [_vp]),
     "qdsp_channelizer_design": (_i, [_vp, _ip, _ip, _ip]),
     "qdsp_channelizer_process": (_ll, [_vp, _vp, _vp, _ll, _ll, _ip, _i, _i, _vp]),
+    "qdsp_channelizer_process_iq": (_ll, [_vp, _vp, _vp, _vp, _ll, _ll, _ip, _i, _i, _vp]),
     "qdsp_channelizer_reset": (_i, [_vp]),
     "qdsp_channelizer_set_variant": (_i, [_vp, _i]),
     "qdsp_channelizer_set_input_format": (_i, [_vp, _i, _f, _f]),

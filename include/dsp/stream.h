@@ -42,18 +42,10 @@ namespace dsp {
         };
 
     public:
-        stream() {
-            for (Side& s : side) {
-                s.host = (T*)qdsp_malloc_pinned(STREAM_BUFFER_SIZE * sizeof(T));
-                s.dev = (T*)qdsp_malloc_device(STREAM_BUFFER_SIZE * sizeof(T));
-                s.produced = qdsp_event_create();
-                s.consumed = qdsp_event_create();
-            }
-            wr = 0;
-            rd = 1;
-            writeBuf = side[wr].host;
-            readBuf = side[rd].host;
-        }
+        stream() { allocate(STREAM_BUFFER_SIZE); }
+        // an addition: buffers of `capacity` elements instead of STREAM_BUFFER_SIZE, for streams that never carry more
+        // (a decimating block's outputs: dsp::ChannelizerT owns one per channel)
+        explicit stream(int capacity) { allocate(capacity > 0 ? capacity : 1); }
         ~stream() {
             for (Side& s : side) {
                 qdsp_free_pinned(s.host);
@@ -111,7 +103,23 @@ namespace dsp {
         T* writeBuf;
         T* readBuf;
 
+        // elements each of the two buffers holds
+        int capacity() const { return cap; }
+
     private:
+        void allocate(int n) {
+            cap = n;
+            for (Side& s : side) {
+                s.host = (T*)qdsp_malloc_pinned((size_t)n * sizeof(T));
+                s.dev = (T*)qdsp_malloc_device((size_t)n * sizeof(T));
+                s.produced = qdsp_event_create();
+                s.consumed = qdsp_event_create();
+            }
+            wr = 0;
+            rd = 1;
+            writeBuf = side[wr].host;
+            readBuf = side[rd].host;
+        }
         bool publish(int size, Residency where, qdsp_stream_t cuStream) {
             std::unique_lock<std::mutex> lk(mtx);
             cv.wait(lk, [this] { return !full || writerStop; });
@@ -161,5 +169,6 @@ namespace dsp {
         bool full = false;
         bool readerStop = false, writerStop = false;
         int count = 0;
+        int cap = 0;
     };
 }

@@ -1,10 +1,10 @@
 /* include/qdsp_b200.h — C ABI of libqdsp_b200.so (B200 / sm_100a).
  *
  * This is the drop-in boundary underneath the reference's header-only `dsp::` block API
- * (AlexandreRouma/qdsp, src/dsp/*.h). The reference has no FFI seam of its own: every block is a
+ * (AlexandreRouma/qdsp, src/dsp/ headers). The reference has no FFI seam of its own: every block is a
  * C++ class whose `run()` does the arithmetic on the CPU (mostly through VOLK). Each entry point
  * below replaces the body of one `run()` (cited per function) and is what the new
- * `include/dsp/*.h` mirror headers, the ctypes binding (`qdsp_b200/lib.py`) and `bench.py` call.
+ * `include/dsp/` mirror headers, the ctypes binding (`qdsp_b200/lib.py`) and `bench.py` call.
  *
  * Conventions
  *   - plain C types only; all `*_dev` pointers are CUDA device pointers owned by the caller;
@@ -249,6 +249,23 @@ int qdsp_channelizer_set_variant(qdsp_channelizer* h, int variant);
  * A shard that starts mid-stream is fed max(history, decimation) extra samples ahead of its first wanted output and drops
  * the outputs those produce (bench.py config 4 at N > 1). Extension: the reference's state is implicit in its run() order. */
 int qdsp_channelizer_seek(qdsp_channelizer* h, long long start);
+/* VFO::setOffset (vfo.h:87-90) for every channel at once: offsets[nch], from the next process call on. Channel c's NCO
+ * phase is continuous at the current stream position (as qdsp_vfofm_set_offset); a channel whose offset did not change
+ * keeps its NCO bit for bit, so retuning one channel is the same array with one entry changed. The history (kept
+ * untranslated), the demodulator phases, the position, the input format and the variant carry on: outputs whose filter
+ * window reaches back before the retune see those samples at the new frequency. The FFT polyphase form is planned again:
+ * kept while the offsets form the comb (moved by any amount), otherwise the direct form until a later retune restores it.
+ * Not a hot-path call: it synchronises the device. Returns -1 (qdsp_last_error) for a NULL handle or array, a non-finite
+ * offset, or a device allocation failure while planning the FFT form, and then leaves the handle as it was. */
+int qdsp_channelizer_set_offsets(qdsp_channelizer* h, const float* offsets);
+/* 1 if the next call with a suitable partition can take the FFT polyphase form (the offsets form the uniform comb and the
+ * variant is 0), else 0 */
+int qdsp_channelizer_fft_form(qdsp_channelizer* h);
+/* Per-channel delivery of the planar [nrows][src_stride] outputs above: row r's first `count` elements (elem_bytes 4:
+ * float, 8: cf32) go to dst_table_dev[r], a DEVICE array of nrows device pointers. One launch whatever nrows (<= 65535);
+ * returns count, or -1. Used by dsp::ChannelizerT (include/dsp/channelizer.h) to fill one stream buffer per channel. */
+long long qdsp_scatter_rows(const void* src_dev, long long src_stride, void* const* dst_table_dev, int nrows, long long count,
+                            int elem_bytes, qdsp_stream_t s);
 
 /* ---- power spectrum: Welch-averaged FFT rows of a cf32 stream (an addition: the reference computes no spectrum) ---- *
  * Frame f covers stream samples [f hop, f hop + N) (sample 0 = the first after create or reset; samples in a gap between *

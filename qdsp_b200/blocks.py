@@ -665,6 +665,22 @@ class Channelizer(_InputFormat, _Block):
     def reset(self):
         check(_L().qdsp_channelizer_reset(self.h))
 
+    def set_offsets(self, offsets):
+        """VFO::setOffset for every channel, from the next call on: each NCO's phase is continuous at the current stream
+        position, a channel whose offset is unchanged keeps its NCO bit for bit, and every other piece of state carries
+        on. Synchronises the device. Raises QdspError (handle unchanged) for a wrong length or a non-finite offset."""
+        offs = np.ascontiguousarray(offsets, np.float32)
+        if offs.shape != (self.nch,):
+            raise ValueError(f"set_offsets takes {self.nch} offsets, got shape {offs.shape}")
+        check(_L().qdsp_channelizer_set_offsets(self.h, _fptr(offs)), "qdsp_channelizer_set_offsets")
+        self.offsets = offs
+
+    @property
+    def fft_form(self) -> bool:
+        """True if the next call with a suitable partition takes the FFT polyphase form (the offsets form the uniform
+        256-channel comb and the variant is 0)."""
+        return bool(_L().qdsp_channelizer_fft_form(self.h))
+
     def process_device(self, in_ptr, out_ptr, n, out_stride, block=None, stream=None) -> int:
         b, nb, bs = _blocks_arg(n, block)
         return int(check(_L().qdsp_channelizer_process(self.h, in_ptr, out_ptr, int(out_stride), int(n), _iptr(b), nb,

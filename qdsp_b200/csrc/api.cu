@@ -621,6 +621,39 @@ struct qdsp_channelizer {
         QDSP_CUDA_OK(cudaMemcpy(nco_dev, v.data(), sizeof(NcoDev) * nch, cudaMemcpyHostToDevice));
         return 0;
     }
+    // VFO::setOffset (vfo.h:87-90) for every channel, from the next call on: each NCO keeps its phase at the current
+    // position abs_pos, so a channel whose offset did not change keeps its Nco bit for bit. The history stays untranslated:
+    // outputs whose window reaches back before abs_pos see those samples at the new frequency. The FFT form is planned
+    // again on the new steps and phases (nullptr when they no longer form the comb: the direct form until a later retune
+    // restores it). Synchronises the device before the old plan and the NCO table are replaced. -1 if the new plan cannot be
+    // allocated: nothing changes.
+    int set_offsets(const float* offsets) {
+        std::vector<Nco> next = nco;
+        std::vector<uint64_t> steps(nch), phases(nch);
+        for (int c = 0; c < nch; c++) {
+            Nco& n = next[c];
+            const uint64_t cur_phase = n.phase + n.step * (uint64_t)abs_pos;
+            n.set_freq(in_sr, -offsets[c]);
+            n.phase = cur_phase - n.step * (uint64_t)abs_pos;
+            steps[c] = n.step;
+            phases[c] = n.phase;
+        }
+        bool plan_failed = false;
+        ChanFftPlan* next_plan = chanfft_plan_create(taps.data(), T, interp, decim, nch, steps.data(), phases.data(), &plan_failed);
+        if (plan_failed) return -1;   // a comb whose plan could not be built: refused, the handle unchanged (not demoted)
+        nco.swap(next);
+        if (upload_nco() != 0) {
+            nco.swap(next);
+            if (next_plan) chanfft_plan_destroy(next_plan);
+            return -1;
+        }
+        if (fftplan) {
+            chanfft_plan_take_scratch(next_plan, fftplan);
+            chanfft_plan_destroy(fftplan);
+        }
+        fftplan = next_plan;
+        return 0;
+    }
     int setup(int nch_, const float* offsets, float inSR, float outSR, float bandWidth, float deviation) {
         nch = nch_;
         in_sr = inSR;
@@ -771,11 +804,7 @@ int qdsp_vfofm_design(qdsp_vfofm* h, int* tapCount, int* interp, int* decim) {
 }
 int qdsp_vfofm_set_offset(qdsp_vfofm* h, float offset) {
     // keep the phase continuous at the current position: phase(abs_pos) is preserved
-    Nco& n = h->c.nco[0];
-    const uint64_t cur_phase = n.phase + n.step * (uint64_t)h->c.abs_pos;
-    n.set_freq(h->c.in_sr, -offset);
-    n.phase = cur_phase - n.step * (uint64_t)h->c.abs_pos;
-    return h->c.upload_nco();
+    return h->c.set_offsets(&offset);
 }
 void qdsp_vfofm_get_phase(qdsp_vfofm* h, float* re, float* im) {
     Nco n = h->c.nco[0];
@@ -1058,6 +1087,30 @@ int qdsp_channelizer_seek(qdsp_channelizer* h, long long start) {
     h->chain.clear();
     h->abs_pos = start;
     return 0;
+}
+int qdsp_channelizer_set_offsets(qdsp_channelizer* h, const float* offsets) {
+    if (!h || !offsets) {
+        set_last_error("channelizer_set_offsets: NULL %s", h ? "offsets" : "handle");
+        return -1;
+    }
+    for (int c = 0; c < h->nch; c++)
+        if (!isfinite(offsets[c])) {
+            set_last_error("channelizer_set_offsets: offset %d is not finite (%g)", c, (double)offsets[c]);
+            return -1;
+        }
+    return h->set_offsets(offsets);
+}
+int qdsp_channelizer_fft_form(qdsp_channelizer* h) { return h && h->fftplan && h->variant == 0 ? 1 : 0; }
+// Per-channel delivery: one launch copies row r of the planar [nrows][src_stride] source to dst_table[r].
+long long qdsp_scatter_rows(const void* src_dev, long long src_stride, void* const* dst_table_dev, int nrows, long long count,
+                            int elem_bytes, qdsp_stream_t s) {
+    if (nrows < 0 || count < 0 || src_stride < count || (elem_bytes != 4 && elem_bytes != 8) ||
+        (nrows > 0 && count > 0 && (!src_dev || !dst_table_dev)) || (reinterpret_cast<uintptr_t>(src_dev) % elem_bytes) != 0) {
+        set_last_error("scatter_rows: bad arguments (elem_bytes 4 or 8, src aligned to it, src_stride >= count)");
+        return -1;
+    }
+    if (launch_scatter_rows(src_dev, src_stride, dst_table_dev, nrows, count, elem_bytes, as_stream(s)) != 0) return -1;
+    return count;
 }
 
 }  // extern "C"

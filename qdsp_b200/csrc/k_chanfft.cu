@@ -47,7 +47,7 @@ struct ChanFftPlan {
     bool rotate = false;                // pre-rotate the stream by channel 0's NCO (comb neither on the bin nor the half-bin grid)
     float2* gpair_dev = nullptr;        // [J * M] (g, (t' - pad - T/2) g), g[t'] = h[t' - pad]
     long long* dturn_dev = nullptr;     // [M] delta_k in turns * 2^64 (signed)
-    long long* dt0_dev = nullptr;       // [M] round(delta_k * T / 2) in the same unit
+    long long* dt0_dev = nullptr;       // [M] round(delta_k * T / 2) + (phase_k - phase_0) in the same unit
     float* delta_dev = nullptr;         // [M] delta_k in rad / sample
     float2* uv = nullptr;               // [2][rows][M] scratch: U then V
     size_t uv_cap = 0;
@@ -233,7 +233,7 @@ struct ChanFftBArgs {
     long long total_out;
     long long abs0;                 // absolute index of this call's first input sample
     int T, pad, D, twob;            // twob: channel 0 sits on half-bin twob of the raw stream (0 when pre-rotated)
-    uint64_t ph0;                   // the channels' common NCO phase constant when the stream is not pre-rotated
+    uint64_t ph0;                   // channel 0's NCO phase constant when the stream is not pre-rotated (the rest: dt0)
     const long long* dturn;         // [M]
     const long long* dt0;           // [M]
     const float* delta;             // [M]
@@ -368,7 +368,9 @@ __global__ void __launch_bounds__(kCfM, 2) chanfft_fft_kernel(const ChanFftBArgs
 }
 
 // ---- host side -------------------------------------------------------------------------------------
-ChanFftPlan* chanfft_plan_create(const float* taps, int T, int interp, int decim, int nch, const uint64_t* nco_steps) {
+ChanFftPlan* chanfft_plan_create(const float* taps, int T, int interp, int decim, int nch, const uint64_t* nco_steps,
+                                 const uint64_t* nco_phases, bool* failed) {
+    if (failed) *failed = false;
     if (interp != 1 || nch != kCfM || decim != kCfDR * kCfM || T + 1 > kCfJ * kCfM) return nullptr;
     const double to_rad = 6.283185307179586476925286766559 / 18446744073709551616.0;
     // is channel 0 on the half-bin grid of the M-point FFT (theta_0 = 2 pi hb / (2 M) within rounding)? then no pre-rotation
@@ -389,12 +391,19 @@ ChanFftPlan* chanfft_plan_create(const float* taps, int T, int interp, int decim
         const double rad = (double)d * to_rad;
         if (fabs(rad) > 2e-6) return nullptr;                            // not a uniform comb: direct form
         dturn[k] = d;
-        dt0[k] = llrint((double)d * 0.5 * (double)T);
+        // channel k's phase constant enters its epilogue turn count as a difference to channel 0's: launch_chanfft adds
+        // channel 0's (the common ph0, or the pre-rotation's beta_ph0), and y_k carries e^{j phase_k} as a whole-row factor
+        const uint64_t dph = nco_phases ? nco_phases[k] - nco_phases[0] : 0ull;
+        dt0[k] = (long long)((uint64_t)llrint((double)d * 0.5 * (double)T) + dph);
         delta[k] = (float)rad;
         if (fabs(rad) > maxd) maxd = fabs(rad);
     }
     ChanFftPlan* p = new (std::nothrow) ChanFftPlan();
-    if (!p) return nullptr;
+    if (!p) {
+        set_last_error("chanfft_plan_create: out of host memory");
+        if (failed) *failed = true;
+        return nullptr;
+    }
     p->T = T;
     p->D = decim;
     p->nch = nch;
@@ -419,6 +428,7 @@ ChanFftPlan* chanfft_plan_create(const float* taps, int T, int interp, int decim
         cudaMalloc(&p->delta_dev, kCfM * sizeof(float)) != cudaSuccess ||
         cudaMemcpy(p->delta_dev, delta.data(), kCfM * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess) {
         set_last_error("chanfft_plan_create: device allocation failed");
+        if (failed) *failed = true;
         chanfft_plan_destroy(p);
         return nullptr;
     }
@@ -432,6 +442,13 @@ void chanfft_plan_destroy(ChanFftPlan* p) {
     if (p->delta_dev) cudaFree(p->delta_dev);
     if (p->uv) cudaFree(p->uv);
     delete p;
+}
+void chanfft_plan_take_scratch(ChanFftPlan* to, ChanFftPlan* from) {
+    if (!to || !from || to->uv) return;
+    to->uv = from->uv;
+    to->uv_cap = from->uv_cap;
+    from->uv = nullptr;
+    from->uv_cap = 0;
 }
 // usable for this batch? uniform run() partition on the decimation grid, 16-byte aligned input
 bool chanfft_usable(const ChanFftPlan* p, const Partition& part, const void* in) {

@@ -70,8 +70,14 @@ int launch_decim_finish(const float2* ypart, long long ypart_stride, int nslices
 
 // ---- k_chanfft.cu: FFT polyphase channelizer (256 channels on a uniform fs/256 comb, decimation 1280) ---------------
 struct ChanFftPlan;
-ChanFftPlan* chanfft_plan_create(const float* taps, int T, int interp, int decim, int nch, const uint64_t* nco_steps);
+// nco_phases: the channels' closed-form phase constants (NULL: all equal); channel k's difference to channel 0's goes into
+// its epilogue constant, so the kernels take only channel 0's phase. nullptr when the steps do not form the comb, or when
+// a device allocation failed: then *failed (if given) is set, and qdsp_last_error says why
+ChanFftPlan* chanfft_plan_create(const float* taps, int T, int interp, int decim, int nch, const uint64_t* nco_steps,
+                                 const uint64_t* nco_phases = nullptr, bool* failed = nullptr);
 void chanfft_plan_destroy(ChanFftPlan* p);
+// hand `from`'s U / V scratch (grown to the largest call) to `to`, which has none yet: a retune keeps it
+void chanfft_plan_take_scratch(ChanFftPlan* to, ChanFftPlan* from);
 bool chanfft_usable(const ChanFftPlan* p, const Partition& part, const void* in);
 int launch_chanfft(ChanFftPlan* plan, const float2* hist, int H, const float2* in, const Partition& part, uint64_t beta_step,
                    uint64_t beta_ph0, long long abs0, float phasor_speed, const float* demod_in, float* demod_out, float* audio,
@@ -140,6 +146,10 @@ int launch_ssb(const float2* in, float* out, long long count, uint64_t phase0, u
                float2 inc3, cudaStream_t s);
 // integer IQ (fmt QDSP_CS16 / QDSP_CS8 / QDSP_CU8, `in` aligned to its pair) -> cf32 (`out` 8-byte aligned)
 int launch_iq_convert(int fmt, IqConv c, const void* in, float2* out, long long count, cudaStream_t s);
+
+// ---- k_route.cu: row r of a planar [nrows][src_stride] buffer -> dst_table[r] (device table), elem_bytes 4 or 8 ----------
+int launch_scatter_rows(const void* src, long long src_stride, void* const* dst_table, int nrows, long long count, int elem_bytes,
+                        cudaStream_t s);
 
 // ---- k_clock.cu: MMClockRecovery (sequential-exact, one warp per stream) --------------------------
 int launch_mm(int cplx, const void* in, const Partition& part, const float* taps_dev, float omega, float gainOmega,

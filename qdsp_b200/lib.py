@@ -128,6 +128,9 @@ SIGNATURES = {
     "qdsp_channelizer_set_variant": (_i, [_vp, _i]),
     "qdsp_channelizer_set_input_format": (_i, [_vp, _i, _f, _f]),
     "qdsp_channelizer_seek": (_i, [_vp, _ll]),
+    "qdsp_channelizer_set_offsets": (_i, [_vp, _fp]),
+    "qdsp_channelizer_fft_form": (_i, [_vp]),
+    "qdsp_scatter_rows": (_ll, [_vp, _ll, _vp, _i, _ll, _i, _vp]),
     "qdsp_spectrum_create": (_vp, [_i, _fp, _i, _i]),
     "qdsp_spectrum_destroy": (None, [_vp]),
     "qdsp_spectrum_out_rows": (_ll, [_vp, _ll]),

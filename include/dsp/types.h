@@ -50,7 +50,8 @@ namespace dsp {
 
     // integer IQ as radio front ends deliver it (interleaved re, im): USRP / BladeRF / LimeSDR / SDRplay / Airspy HF+
     // (int16), HackRF (int8), RTL-SDR (uint8). Read as complex_t by IQToComplex<T> (convertion.h) and directly by
-    // FusedVFOFloatFMDemodT<T> (vfo.h), both converting on the GPU: y = (float(x) + offset) * scale per component.
+    // FusedVFOFloatFMDemodT<T> (vfo.h), ChannelizerT<T> (channelizer.h) and SpectrumT<T> (spectrum.h), all converting on
+    // the GPU: y = (float(x) + offset) * scale per component.
     struct complex_s16_t { int16_t re; int16_t im; };
     struct complex_s8_t { int8_t re; int8_t im; };
     struct complex_u8_t { uint8_t re; uint8_t im; };

@@ -33,7 +33,8 @@ typedef void* qdsp_stream_t;
 enum { QDSP_F32 = 0, QDSP_CF32 = 1 }; /* element type of a stream: float or {float re,im} (== stereo_t) */
 /* integer IQ as radio front ends deliver it: interleaved (re, im) pairs of int16 (USRP, BladeRF sc16q11, LimeSDR,
  * SDRplay, Airspy HF+), int8 (HackRF) or uint8 (RTL-SDR). Accepted by qdsp_iq_convert_process and, after
- * *_set_input_format, by the fused VFO -> FM chain and the channelizer; every `dtype` argument rejects them. */
+ * *_set_input_format, by the fused VFO -> FM chain, the channelizer and the power spectrum; every `dtype` argument
+ * rejects them. */
 enum { QDSP_CS16 = 2, QDSP_CS8 = 3, QDSP_CU8 = 4 };
 
 /* ---- runtime plumbing (replaces volk_malloc/volk_free in src/dsp/stream.h:25-31) ------------- */
@@ -267,20 +268,28 @@ int qdsp_channelizer_fft_form(qdsp_channelizer* h);
 long long qdsp_scatter_rows(const void* src_dev, long long src_stride, void* const* dst_table_dev, int nrows, long long count,
                             int elem_bytes, qdsp_stream_t s);
 
-/* ---- power spectrum: Welch-averaged FFT rows of a cf32 stream (an addition: the reference computes no spectrum) ---- *
+/* ---- power spectrum: Welch-averaged FFT rows of an IQ stream (an addition: the reference computes no spectrum) ----- *
  * Frame f covers stream samples [f hop, f hop + N) (sample 0 = the first after create or reset; samples in a gap between *
  * frames are never read); P_f[k] = |sum_n w[n] x[f hop + n] e^{-2 pi i k n / N}|^2. Row r is the mean of P over frames   *
  * r A .. r A + A - 1, FFT-shifted (out[j] = mean P[(j + N / 2) mod N]: bin 0 of a row is -fs / 2), linear power, float32. *
  * A row is a pure function of the stream: any split into calls gives the same bits. N a power of two in [64, 16384],     *
  * window N floats (NULL = rectangular), hop >= 1, average >= 1; create returns NULL on anything else. process writes the  *
- * rows it completes contiguously (N floats each) and returns their number, -1 for a negative count or in_dev not 8-byte  *
- * aligned; samples of rows not yet complete stay in the handle. out_rows: rows the next call of `count` samples returns.*/
+ * rows it completes contiguously (N floats each) and returns their number, -1 for a negative count or in_dev not aligned *
+ * to its pair (8 bytes for cf32, 4 for cs16, 2 for cs8 / cu8); samples of rows not yet complete stay in the handle.      *
+ * out_rows: rows the next call of `count` samples returns.                                                              *
+ * set_input_format: the element type of in_dev from the next process call on, as qdsp_vfofm_set_input_format (QDSP_CF32, *
+ * the default, or QDSP_CS16 / QDSP_CS8 / QDSP_CU8 with the conversion of qdsp_iq_convert_process; -1 and no change for a *
+ * bad format, scale or offset; reset keeps the format). The rows equal, bit for bit, those of a cf32 handle fed the      *
+ * converted samples. The carried samples are kept as cf32, so formats may change from call to call. The frames kernel    *
+ * reads the integer pairs itself, so samples in the gaps between frames are never converted; only at N = 16384 with      *
+ * hop <= N is a call converted to cf32 first, into a buffer of the handle grown to the largest call.                     */
 typedef struct qdsp_spectrum qdsp_spectrum;
 qdsp_spectrum* qdsp_spectrum_create(int fftSize, const float* window, int hop, int average);
 void qdsp_spectrum_destroy(qdsp_spectrum* h);
 long long qdsp_spectrum_out_rows(qdsp_spectrum* h, long long count);
 long long qdsp_spectrum_process(qdsp_spectrum* h, const void* in_dev, float* rows_out_dev, long long count, qdsp_stream_t s);
 int qdsp_spectrum_reset(qdsp_spectrum* h);
+int qdsp_spectrum_set_input_format(qdsp_spectrum* h, int fmt, float scale, float offset);
 
 /* ---- recurrent blocks (chunked block-parallel scans) ----------------------------------------- */
 /* BFMDeemp::run, src/dsp/filter.h:129-158 (stereo_t in/out, state lastOutL/R) */

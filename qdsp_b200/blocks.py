@@ -738,13 +738,16 @@ class IQConverter(_Block):
         return dout.to_numpy(np.complex64, m)
 
 
-class Spectrum(_Block):
+class Spectrum(_InputFormat, _Block):
     """Welch power spectrum of a complex64 stream (qdsp_spectrum_*; an addition, the reference has none). Row r is the
     mean of |FFT(window * frame)|^2 over frames r*average .. r*average + average - 1, frame f = samples
     [f*hop, f*hop + fftSize), FFT-shifted (column 0 is -fs/2), linear float32 power. hop defaults to fftSize, window to
-    rectangular. Rows are a pure function of the stream: samples of rows not yet complete stay in the handle."""
+    rectangular. Rows are a pure function of the stream: samples of rows not yet complete stay in the handle.
+    After set_input_format('cs16' | 'cs8' | 'cu8'), process takes interleaved integer pairs (read and converted by the
+    frames kernel itself) and process_device a pointer to them."""
 
     _destroy = "qdsp_spectrum_destroy"
+    _set_fmt = "qdsp_spectrum_set_input_format"
     out_dtype = np.float32
 
     def __init__(self, fftSize, window=None, hop=None, average=1):
@@ -766,14 +769,15 @@ class Spectrum(_Block):
         return int(check(_L().qdsp_spectrum_out_rows(self.h, int(n)), "qdsp_spectrum_out_rows"))
 
     def process_device(self, in_ptr, out_ptr, n, stream=None) -> int:
-        """in_ptr: n complex64 samples (8-byte aligned); out_ptr: room for out_rows(n) rows of fftSize floats."""
+        """in_ptr: n complex64 samples (8-byte aligned), or n integer pairs after set_input_format (aligned to the pair);
+        out_ptr: room for out_rows(n) rows of fftSize floats."""
         return int(check(_L().qdsp_spectrum_process(self.h, in_ptr, out_ptr, int(n), stream), "qdsp_spectrum_process"))
 
     def process(self, x) -> np.ndarray:
-        x = np.ascontiguousarray(x, np.complex64)
-        rows = self.out_rows(len(x))
+        x, n = _iq_input(x, self._in_fmt)
+        rows = self.out_rows(n)
         din, dout = DevBuf.from_numpy(x), DevBuf(max(rows, 1) * self.fftSize * 4)
-        m = self.process_device(din.ptr, dout.ptr, len(x))
+        m = self.process_device(din.ptr, dout.ptr, n)
         return dout.to_numpy(np.float32, m * self.fftSize).reshape(m, self.fftSize)
 
     def reset(self):

@@ -1120,6 +1120,12 @@ long long qdsp_scatter_rows(const void* src_dev, long long src_stride, void* con
 // =================================================================================================
 struct qdsp_spectrum {
     SpectrumPlan* plan = nullptr;
+    // element type of the input (set_input_format): integer pairs are read and converted by the frames kernel itself,
+    // except at N = 16384 with hop <= N (spectrum_native_integer), where they are converted into `conv` first (grown to the
+    // largest call, so the hot path stays allocation-free)
+    int in_fmt = QDSP_CF32;
+    IqConv in_conv{1.0f, 0.0f};
+    Scratch conv;
 };
 
 extern "C" {
@@ -1152,8 +1158,9 @@ void qdsp_spectrum_destroy(qdsp_spectrum* h) {
 }
 long long qdsp_spectrum_out_rows(qdsp_spectrum* h, long long count) { return spectrum_out_rows(h->plan, count); }
 long long qdsp_spectrum_process(qdsp_spectrum* h, const void* in_dev, float* rows_out_dev, long long count, qdsp_stream_t s) {
-    if (count < 0 || (reinterpret_cast<uintptr_t>(in_dev) & 7) != 0) {
-        set_last_error("spectrum_process: negative count or input not aligned to 8 bytes");
+    const int E = iq_pair_bytes(h->in_fmt);   // the input is aligned to its pair: 8 bytes for cf32, 4 for cs16, 2 for 8-bit
+    if (count < 0 || (reinterpret_cast<uintptr_t>(in_dev) % E) != 0) {
+        set_last_error("spectrum_process: negative count or input not aligned to %d bytes", E);
         return -1;
     }
     if (count == 0) return 0;
@@ -1161,10 +1168,21 @@ long long qdsp_spectrum_process(qdsp_spectrum* h, const void* in_dev, float* row
         set_last_error("spectrum_process: NULL input or output");
         return -1;
     }
-    return launch_spectrum(h->plan, (const float2*)in_dev, rows_out_dev, count, as_stream(s));
+    if (h->in_fmt != QDSP_CF32 && !spectrum_native_integer(h->plan)) {
+        if (h->conv.reserve((size_t)count * sizeof(float2)) != 0) return -1;
+        if (launch_iq_convert(h->in_fmt, h->in_conv, in_dev, (float2*)h->conv.p, count, as_stream(s)) != 0) return -1;
+        return launch_spectrum(h->plan, h->conv.p, QDSP_CF32, IqConv{1.0f, 0.0f}, rows_out_dev, count, as_stream(s));
+    }
+    return launch_spectrum(h->plan, in_dev, h->in_fmt, h->in_conv, rows_out_dev, count, as_stream(s));
 }
 int qdsp_spectrum_reset(qdsp_spectrum* h) {
     spectrum_plan_reset(h->plan);
+    return 0;
+}
+int qdsp_spectrum_set_input_format(qdsp_spectrum* h, int fmt, float scale, float offset) {
+    if (fmt != QDSP_CF32 && !iq_format_ok(fmt, scale, offset, "spectrum_set_input_format")) return -1;
+    h->in_fmt = fmt;
+    h->in_conv = fmt == QDSP_CF32 ? IqConv{1.0f, 0.0f} : IqConv{scale, offset};
     return 0;
 }
 

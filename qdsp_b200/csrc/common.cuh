@@ -99,5 +99,16 @@ __device__ __forceinline__ float2 ldg_stream64(const float2* p) {
     asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0,%1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
     return v;
 }
+// the same for one integer IQ pair: a 32-bit (cs16) or 16-bit (cs8 / cu8) word, zero-extended
+__device__ __forceinline__ uint32_t ldg_stream32(const uint32_t* p) {
+    uint32_t v;
+    asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(v) : "l"(p));
+    return v;
+}
+__device__ __forceinline__ uint32_t ldg_stream16(const uint16_t* p) {
+    uint16_t v;
+    asm volatile("ld.global.nc.L1::no_allocate.u16 %0, [%1];" : "=h"(v) : "l"(p));
+    return v;
+}
 
 }  // namespace qdsp

@@ -9,7 +9,8 @@
 // the open row's finished slices, and the next call continues them to the same bits.
 //
 // spectrum_frames_kernel: one CTA per slice (or the part of it this call completes). Thread (lane g, column j) loads
-// samples j + r N / 16 (r < 16) of its frame straight from global memory (coalesced across j), windows them and runs the first
+// samples j + r N / 16 (r < 16) of its frame straight from global memory (coalesced across j), in the input format FMT
+// (cf32, or cs16 / cs8 / cu8 words converted by the rule of iq_common.cuh), windows them and runs the first
 // radix-16 pass in registers; the remaining passes are Stockham radix-16 passes (and one radix-2/4/8 pass for log2 N
 // mod 4) through a padded shared-memory frame, twiddles from a float64-designed table. The last pass leaves 16 bins per
 // thread, always the same ones, so the frame-order power sums stay in registers across the frames. Up to 512 threads a
@@ -19,6 +20,7 @@
 #include <new>
 #include <vector>
 #include "fft_common.cuh"
+#include "iq_common.cuh"
 #include "kernels.cuh"
 
 namespace qdsp {
@@ -30,7 +32,8 @@ struct SpectrumPlan {
     float2* tw = nullptr;               // [N] e^{-j 2 pi k / N}
     float* open[2] = {nullptr, nullptr};    // [G][N] lane sums of the open slice (ping-pong)
     float* rowp[2] = {nullptr, nullptr};    // [N] running sum of the open row's finished slices (ping-pong)
-    float2* tail[2] = {nullptr, nullptr};   // [N] samples from the first incomplete frame on (ping-pong)
+    float2* tail[2] = {nullptr, nullptr};   // [2N] samples from the first incomplete frame on, as cf32 (ping-pong; the
+                                            // second N: the head of an integer call, launch_spectrum)
     float* slices = nullptr;            // [umax][N] finished slice sums of one launch
     int cur = 0, tcur = 0;
     long long pos = 0;                  // samples seen
@@ -39,7 +42,7 @@ struct SpectrumPlan {
 };
 
 struct SpecArgs {
-    const float2* in;
+    const void* in;                     // cf32, or integer pairs (the frames kernel's FMT)
     const float2* tail;
     long long pos, tail0;               // stream positions of in[0] and tail[0]
     long long fa, fb;                   // frames [fa, fb) of this launch
@@ -50,6 +53,7 @@ struct SpecArgs {
     const float* open_in;
     float* open_out;
     float* slices;
+    IqConv conv;                        // integer input
 };
 
 template <int LOGN>
@@ -72,6 +76,26 @@ __host__ __device__ inline long long sp_slice_end(long long s, int A, int S, int
 }
 __host__ __device__ inline long long sp_slice_of(long long f, int A, int S, int spr) { return (f / A) * spr + (f % A) / S; }
 
+// integer pair i of this call's input as its raw word (FMT QDSP_CS16: 32 bits; QDSP_CS8 / QDSP_CU8: 16), and a raw word
+// converted by the rule of iq_common.cuh
+template <int FMT>
+__device__ __forceinline__ uint32_t sp_word(const void* in, long long i) {
+    if (FMT == QDSP_CS16) return ldg_stream32(reinterpret_cast<const uint32_t*>(in) + i);
+    return ldg_stream16(reinterpret_cast<const uint16_t*>(in) + i);
+}
+template <int FMT>
+__device__ __forceinline__ float2 sp_convert(uint32_t w, IqConv c) {
+    if (FMT == QDSP_CS16) return iq_cs16(w, c);
+    const float4 v = iq_b8x2<FMT>(w, c);
+    return make_float2(v.x, v.y);
+}
+// sample i of this call's input, as cf32: FMT is QDSP_CF32, QDSP_CS16, QDSP_CS8 or QDSP_CU8
+template <int FMT>
+__device__ __forceinline__ float2 sp_sample(const void* in, long long i, IqConv c) {
+    if (FMT == QDSP_CF32) return ldg_stream64(reinterpret_cast<const float2*>(in) + i);
+    return sp_convert<FMT>(sp_word<FMT>(in, i), c);
+}
+
 // the bin of accumulator e of column j after the last pass
 template <int LOGN>
 __device__ __forceinline__ int sp_bin(int j, int e) {
@@ -80,7 +104,7 @@ __device__ __forceinline__ int sp_bin(int j, int e) {
     return j + (e / RL) * Gm::TPF + (e % RL) * (Gm::N / RL);
 }
 
-template <int LOGN>
+template <int LOGN, int FMT>
 __global__ void __launch_bounds__(SpGeom<LOGN>::THREADS, SpGeom<LOGN>::MINB) spectrum_frames_kernel(const SpecArgs a) {
     using Gm = SpGeom<LOGN>;
     constexpr int N = Gm::N, TPF = Gm::TPF, G = Gm::G, RL = Gm::RL;
@@ -108,20 +132,40 @@ __global__ void __launch_bounds__(SpGeom<LOGN>::THREADS, SpGeom<LOGN>::MINB) spe
         for (int r = 0; r < 16; r++) {
             const long long q = q0 + r * TPF;
             x[r] = make_float2(0.f, 0.f);
-            if (live) x[r] = q >= a.pos ? ldg_stream64(a.in + (q - a.pos)) : __ldg(a.tail + (q - a.tail0));
+            if (live) x[r] = q >= a.pos ? sp_sample<FMT>(a.in, q - a.pos, a.conv) : __ldg(a.tail + (q - a.tail0));
         }
     };
     // up to 512 threads a CTA: the next wave's samples are loaded while this wave's passes run (32 more registers; at
     // 1024 threads, 64 registers a thread, there is no room for them)
     constexpr bool PF = Gm::THREADS <= 512;
-    float2 nx[16];
-    if (PF) fetch(w0, nx);
+    // Integer input: the prefetch holds the raw words (16 registers instead of 32), converted when the wave is taken, so
+    // the loads are in flight during the previous wave's passes (converted as they arrive, they would be waited for
+    // before those passes). The integer kernels never take a frame that starts in the carried tail (launch_spectrum).
+    constexpr bool RAW = PF && FMT != QDSP_CF32;
+    auto fetch_raw = [&](long long wv, uint32_t (&w)[16]) {
+        const long long f = base + wv * G + g;
+        const bool live = f >= ua && f < ub;
+        const long long i0 = f * a.hop + j - a.pos;
+#pragma unroll
+        for (int r = 0; r < 16; r++) {
+            w[r] = 0;
+            if (live) w[r] = sp_word<FMT>(a.in, i0 + r * TPF);
+        }
+    };
+    float2 nx[RAW ? 1 : 16];
+    uint32_t nw[RAW ? 16 : 1];
+    if constexpr (RAW) fetch_raw(w0, nw);
+    else if (PF) fetch(w0, nx);
 #pragma unroll 1
     for (long long wv = w0; wv <= w1; wv++) {
         const long long f = base + wv * G + g;
         const bool live = f >= ua && f < ub;
         float2 v[16];
-        if (PF) {
+        if constexpr (RAW) {
+#pragma unroll
+            for (int r = 0; r < 16; r++) v[r] = sp_convert<FMT>(nw[r], a.conv);
+            if (wv < w1) fetch_raw(wv + 1, nw);
+        } else if (PF) {
 #pragma unroll
             for (int r = 0; r < 16; r++) v[r] = nx[r];
             if (wv < w1) fetch(wv + 1, nx);
@@ -246,6 +290,12 @@ static int spectrum_slice_len(int N, int A) {
     return A < s ? A : s;
 }
 
+// Integer input is read by the frames kernel itself, except where that kernel has no prefetch (N = 16384: 1024 threads at
+// 64 registers, where even 16 raw words spill) and reads every sample (hop <= N). There the kernel is bound by its
+// instructions, the conversion's instructions take as long as a conversion pass over the whole call, and the native read
+// measured 0.2-0.3 % slower than that pass on cs8 / cu8 (DESIGN.md §6.0e): the handle converts first.
+bool spectrum_native_integer(const SpectrumPlan* p) { return p->N / 16 <= 512 || p->hop > p->N; }
+
 static long long sp_frames_complete(const SpectrumPlan* p, long long P) { return P >= p->N ? (P - p->N) / p->hop + 1 : 0; }
 
 long long spectrum_out_rows(const SpectrumPlan* p, long long count) {
@@ -292,7 +342,7 @@ SpectrumPlan* spectrum_plan_create(int N, const float* window, int hop, int A) {
               cudaMalloc(&p->slices, (size_t)p->umax * N * sizeof(float)) == cudaSuccess;
     for (int i = 0; ok && i < 2; i++)
         ok = cudaMalloc(&p->open[i], (size_t)p->G * N * sizeof(float)) == cudaSuccess &&
-             cudaMalloc(&p->rowp[i], N * sizeof(float)) == cudaSuccess && cudaMalloc(&p->tail[i], N * sizeof(float2)) == cudaSuccess;
+             cudaMalloc(&p->rowp[i], N * sizeof(float)) == cudaSuccess && cudaMalloc(&p->tail[i], 2 * N * sizeof(float2)) == cudaSuccess;
     if (!ok) {
         set_last_error("spectrum_create: device allocation failed");
         spectrum_plan_destroy(p);
@@ -306,7 +356,7 @@ void spectrum_plan_reset(SpectrumPlan* p) {
     p->pos = p->frames_done = p->tail0 = 0;
 }
 
-template <int LOGN>
+template <int LOGN, int FMT>
 static int sp_launch_frames(const SpecArgs& a, long long units, cudaStream_t s) {
     using Gm = SpGeom<LOGN>;
     const size_t smem = (size_t)Gm::G * Gm::PADN * sizeof(float2) + (Gm::THREADS > 512 ? (size_t)Gm::THREADS * 16 * sizeof(float) : 0);
@@ -314,27 +364,56 @@ static int sp_launch_frames(const SpecArgs& a, long long units, cudaStream_t s) 
     int dev = 0;
     cudaGetDevice(&dev);
     if (!attr_dev[dev & 63]) {
-        QDSP_CUDA_OK(cudaFuncSetAttribute(spectrum_frames_kernel<LOGN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        QDSP_CUDA_OK(cudaFuncSetAttribute(spectrum_frames_kernel<LOGN, FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_dev[dev & 63] = true;
     }
-    spectrum_frames_kernel<LOGN><<<(unsigned)units, Gm::THREADS, smem, s>>>(a);
+    spectrum_frames_kernel<LOGN, FMT><<<(unsigned)units, Gm::THREADS, smem, s>>>(a);
     QDSP_LAUNCH_OK();
     return 0;
 }
 
-long long launch_spectrum(SpectrumPlan* p, const float2* in, float* rows_out, long long count, cudaStream_t s) {
+template <int LOGN>
+static int sp_launch_frames(int fmt, const SpecArgs& a, long long units, cudaStream_t s) {
+    switch (fmt) {
+        case QDSP_CF32: return sp_launch_frames<LOGN, QDSP_CF32>(a, units, s);
+        case QDSP_CS16: return sp_launch_frames<LOGN, QDSP_CS16>(a, units, s);
+        case QDSP_CS8: return sp_launch_frames<LOGN, QDSP_CS8>(a, units, s);
+        case QDSP_CU8: return sp_launch_frames<LOGN, QDSP_CU8>(a, units, s);
+    }
+    return -1;
+}
+
+long long launch_spectrum(SpectrumPlan* p, const void* in, int fmt, IqConv conv, float* rows_out, long long count,
+                          cudaStream_t s) {
     const int N = p->N;
     const long long pos_end = p->pos + count;
     const long long f_end = sp_frames_complete(p, pos_end);
     const long long r_out0 = p->frames_done / p->A;
+    // Integer input: the frames [frames_done, f1) start in the carried tail (before this call's first sample) and end
+    // before sample pos + min(count, N). They are taken by the cf32 kernel from the tail followed by this call's first
+    // min(count, N) samples converted to cf32, the same cut as a call boundary; the integer kernels read this call's
+    // input only, and need no registers for the tail.
+    long long f1 = p->frames_done;
+    const float2* head = nullptr;
+    if (fmt != QDSP_CF32) {
+        f1 = (p->pos + p->hop - 1) / p->hop;
+        if (f1 > f_end) f1 = f_end;
+        if (f1 > p->frames_done) {
+            float2* h = p->tail[p->tcur] + (p->pos - p->tail0);   // pos - tail0 < N: the tail holds an incomplete frame
+            if (launch_iq_convert(fmt, conv, in, h, count < N ? count : N, s) != 0) return -1;
+            head = h;
+        }
+    }
     for (long long fa = p->frames_done; fa < f_end;) {
         const long long s_a = sp_slice_of(fa, p->A, p->S, p->spr);
         long long fb = sp_slice_start(s_a + p->umax, p->A, p->S, p->spr);
         if (fb > f_end) fb = f_end;
+        const bool in_head = fa < f1;
+        if (in_head && fb > f1) fb = f1;
         const long long s_b = sp_slice_of(fb - 1, p->A, p->S, p->spr);
         const long long s_done = sp_slice_end(s_b, p->A, p->S, p->spr) == fb ? s_b + 1 : s_b;
         SpecArgs a{};
-        a.in = in;
+        a.in = in_head ? head : in;
         a.tail = p->tail[p->tcur];
         a.pos = p->pos;
         a.tail0 = p->tail0;
@@ -350,18 +429,20 @@ long long launch_spectrum(SpectrumPlan* p, const float2* in, float* rows_out, lo
         a.open_in = p->open[p->cur];
         a.open_out = p->open[p->cur ^ 1];
         a.slices = p->slices;
+        a.conv = conv;
         const long long units = s_b - s_a + 1;
+        const int kfmt = in_head ? QDSP_CF32 : fmt;
         int rc = -1;
         switch (p->logN) {
-            case 6: rc = sp_launch_frames<6>(a, units, s); break;
-            case 7: rc = sp_launch_frames<7>(a, units, s); break;
-            case 8: rc = sp_launch_frames<8>(a, units, s); break;
-            case 9: rc = sp_launch_frames<9>(a, units, s); break;
-            case 10: rc = sp_launch_frames<10>(a, units, s); break;
-            case 11: rc = sp_launch_frames<11>(a, units, s); break;
-            case 12: rc = sp_launch_frames<12>(a, units, s); break;
-            case 13: rc = sp_launch_frames<13>(a, units, s); break;
-            case 14: rc = sp_launch_frames<14>(a, units, s); break;
+            case 6: rc = sp_launch_frames<6>(kfmt, a, units, s); break;
+            case 7: rc = sp_launch_frames<7>(kfmt, a, units, s); break;
+            case 8: rc = sp_launch_frames<8>(kfmt, a, units, s); break;
+            case 9: rc = sp_launch_frames<9>(kfmt, a, units, s); break;
+            case 10: rc = sp_launch_frames<10>(kfmt, a, units, s); break;
+            case 11: rc = sp_launch_frames<11>(kfmt, a, units, s); break;
+            case 12: rc = sp_launch_frames<12>(kfmt, a, units, s); break;
+            case 13: rc = sp_launch_frames<13>(kfmt, a, units, s); break;
+            case 14: rc = sp_launch_frames<14>(kfmt, a, units, s); break;
         }
         if (rc != 0) return -1;
         SpecRowArgs ra{};
@@ -382,7 +463,8 @@ long long launch_spectrum(SpectrumPlan* p, const float2* in, float* rows_out, lo
         p->cur ^= 1;
         fa = fb;
     }
-    // carry the samples from the first incomplete frame on (fewer than N)
+    // carry the samples from the first incomplete frame on (fewer than N), converted to cf32: the format may change with
+    // the next call
     const long long t0 = f_end * p->hop;
     if (t0 < pos_end) {
         float2* dst = p->tail[p->tcur ^ 1];
@@ -392,7 +474,13 @@ long long launch_spectrum(SpectrumPlan* p, const float2* in, float* rows_out, lo
             QDSP_CUDA_OK(cudaMemcpyAsync(dst, p->tail[p->tcur] + (t0 - p->tail0), off * sizeof(float2), cudaMemcpyDeviceToDevice, s));
         }
         const long long from = t0 > p->pos ? t0 - p->pos : 0;
-        QDSP_CUDA_OK(cudaMemcpyAsync(dst + off, in + from, (count - from) * sizeof(float2), cudaMemcpyDeviceToDevice, s));
+        if (fmt == QDSP_CF32) {
+            QDSP_CUDA_OK(cudaMemcpyAsync(dst + off, static_cast<const float2*>(in) + from, (count - from) * sizeof(float2),
+                                         cudaMemcpyDeviceToDevice, s));
+        } else if (launch_iq_convert(fmt, conv, static_cast<const char*>(in) + from * iq_pair_bytes(fmt), dst + off,
+                                     count - from, s) != 0) {
+            return -1;
+        }
         p->tcur ^= 1;
     }
     p->tail0 = t0;

@@ -89,8 +89,13 @@ SpectrumPlan* spectrum_plan_create(int N, const float* window, int hop, int aver
 void spectrum_plan_destroy(SpectrumPlan* p);
 void spectrum_plan_reset(SpectrumPlan* p);
 long long spectrum_out_rows(const SpectrumPlan* p, long long count);
-// `in` 8-byte aligned; returns the rows written to rows_out ([rows][N]) or -1
-long long launch_spectrum(SpectrumPlan* p, const float2* in, float* rows_out, long long count, cudaStream_t s);
+// false where integer input is converted to cf32 by launch_iq_convert before launch_spectrum instead of being read by the
+// frames kernel (N = 16384 with hop <= N)
+bool spectrum_native_integer(const SpectrumPlan* p);
+// `in`: cf32 (fmt QDSP_CF32, 8-byte aligned) or integer pairs (QDSP_CS16 / QDSP_CS8 / QDSP_CU8, converted by `conv`,
+// aligned to the pair); returns the rows written to rows_out ([rows][N]) or -1
+long long launch_spectrum(SpectrumPlan* p, const void* in, int fmt, IqConv conv, float* rows_out, long long count,
+                          cudaStream_t s);
 
 // ---- k_fir.cu: register-blocked dense FIR (cf32, D = 1) -----------------------------------------
 struct FirPlan;

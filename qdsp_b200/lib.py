@@ -136,6 +136,7 @@ SIGNATURES = {
     "qdsp_spectrum_out_rows": (_ll, [_vp, _ll]),
     "qdsp_spectrum_process": (_ll, [_vp, _vp, _vp, _ll, _vp]),
     "qdsp_spectrum_reset": (_i, [_vp]),
+    "qdsp_spectrum_set_input_format": (_i, [_vp, _i, _f, _f]),
     "qdsp_deemp_create": (_vp, [_f, _f]),
     "qdsp_deemp_destroy": (None, [_vp]),
     "qdsp_deemp_process": (_ll, [_vp, _vp, _vp, _ll, _vp]),
